@@ -120,10 +120,36 @@ def measured_peak_gbs():
 
 
 def cpu_impl():
-    """the CPU arm: the reference's OWN sources (oracle/_ref/libmlmap_ref.so, built from /root/reference by
-    oracle/ref_build/Makefile; the prebuilt file travels to the GPU box) when available, else the restatement"""
+    """the CPU arm: the reference's OWN sources (oracle/_ref/libmlmap_ref.so, built from $MLMAPPING_REFERENCE by
+    oracle/ref_build/Makefile) when available, else the restatement"""
     from oracle_binding import reference_available
     return "reference" if reference_available() else "port"
+
+
+def dump_outputs(out_dir, m, st, exported, budget=64 << 20):
+    """what the timed path computed in its last step, as float32 / float64 .npy files under out_dir: the frame's FrameStats
+    (field order of mlmapping_b200.capi.FrameStats), its hit cells (rho, phi, z in the reference's iteration order) with
+    their probabilities, its miss cells (flat indices, sorted) and the whole map sorted by subbox index (occupancy and
+    inflate as the byte codes 'u' / 'f' / 'o').  A map larger than the budget is cut to a fixed, seeded sample of
+    subboxes."""
+    keys, p = m.last_frame_hits()
+    arrays = {"frame_stats": np.array([getattr(st, f) for f, _ in st._fields_], dtype=np.float64),
+              "hit_keys": keys.astype(np.float64), "hit_p": p.astype(np.float32),
+              "miss_cells": np.sort(m.last_frame_misses()).astype(np.float64)}
+    cells = exported["log_odds"].shape[1]
+    rows = exported["glb"].shape[0]
+    left = budget - sum(a.nbytes for a in arrays.values())
+    keep = max(0, min(rows, left // (3 * 8 + 4 + 3 * 4 * cells)))
+    sel = np.arange(rows) if keep == rows else np.sort(np.random.default_rng(0).choice(rows, keep, replace=False))
+    arrays.update({"map_glb": exported["glb"][sel].astype(np.float64),
+                   "map_collapsed": exported["collapsed"][sel].astype(np.float32),
+                   "map_occupancy": exported["occupancy"][sel].view(np.uint8).astype(np.float32),
+                   "map_inflate": exported["inflate"][sel].view(np.uint8).astype(np.float32),
+                   "map_log_odds": exported["log_odds"][sel].astype(np.float32)})
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", a)
 
 
 def run_cpu_sample(cfg, frames, poses, n_frames):
@@ -587,7 +613,11 @@ def main():
     ap.add_argument("--agents-only", action="store_true", help="run only the CFG-D agents section and print its JSON (tooling)")
     ap.add_argument("--no-agents", action="store_true")
     ap.add_argument("--queries", type=int, default=10_000_000, help="planner queries per step (4:4:2 odd/occupancy/grad)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed to DIR/<name>.npy "
+                    "(frame stats, hit and miss cells, the map) for comparing two builds on the same inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -647,22 +677,26 @@ def main():
     launches0 = m.kernel_launch_count()
     barrier()
     sampler.start()
-    wall0 = time.perf_counter()
-    dev_ms, rays, alg_bytes, slow_frames = 0.0, 0, 0, 0
-    for k in range(args.warmup, total):
-        m.flush_l2()
-        m.timer_start()
-        st = m.integrate_depth_device(d_frames[k], ROWS, COLS, poses[k])
-        dev_ms += m.timer_stop_ms()
-        rays += st.n_points
-        alg_bytes += algorithmic_bytes(st)
-        slow_frames += st.ordering_slow_path
-    barrier()
-    wall1 = time.perf_counter()
-    clocks = sampler.stop()
+    try:
+        wall0 = time.perf_counter()
+        dev_ms, rays, alg_bytes, slow_frames = 0.0, 0, 0, 0
+        for k in range(args.warmup, total):
+            m.flush_l2()
+            m.timer_start()
+            st = m.integrate_depth_device(d_frames[k], ROWS, COLS, poses[k])
+            dev_ms += m.timer_stop_ms()
+            rays += st.n_points
+            alg_bytes += algorithmic_bytes(st)
+            slow_frames += st.ordering_slow_path
+        barrier()
+        wall1 = time.perf_counter()
+    finally:  # the sampler's nvidia-smi child must not outlive a failed run
+        clocks = sampler.stop()
     launches = m.kernel_launch_count() - launches0  # the library counts its map kernels only (the L2 flush is not one)
     exported = m.export_map()
     submaps = exported["glb"].shape[0]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, m, st, exported)
 
     # ---------------- batched planner queries against the map just built (BASELINE config 5 mix) ----------------
     queries = None

@@ -114,9 +114,9 @@ CASES = ["cfg_a_config1_single_frame", "cfg_a_config2_first_8_frames_stride_25",
          "cfg_a_exploration_6_frames_rolled_poses"]
 
 if __name__ == "__main__":
-    from oracle_binding import _REFERENCE
-    if not _REFERENCE.exists():
-        raise SystemExit("the golden vectors are generated from the reference's own sources: /root/reference is needed")
+    from oracle_binding import reference_available
+    if not reference_available():
+        raise SystemExit("the golden vectors are generated from the reference's own build: oracle/_ref or its sources are needed")
     out = {"generator": "tests/golden/make_golden.py",
            "provenance": "outputs of the UNMODIFIED reference sources (/root/reference src/map_awareness.cpp, src/map_local.cpp, "
                          "src/mlmap.cpp, src/rviz_vis.cpp, include/*.h, 3rdPartLib/Sophus/sophus/{so3,se3}.cpp) built by "

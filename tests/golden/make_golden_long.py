@@ -16,7 +16,7 @@ sys.path.insert(0, str(HERE.parent.parent))
 sys.path.insert(0, str(HERE.parent))
 
 from mlmapping_b200 import config_cfg_a, config_cfg_b, config_cfg_c, scenes  # noqa: E402
-from oracle_binding import Oracle, _REFERENCE  # noqa: E402
+from oracle_binding import Oracle, reference_available  # noqa: E402
 
 COUNTERS = ("n_points", "n_inside", "n_cast", "n_hit_cells", "n_miss_cells", "n_touched_voxels", "hit_bucket_count",
             "ram_expand_cnt", "obs_cnt")
@@ -79,8 +79,8 @@ def run(name, impl):
 
 
 if __name__ == "__main__":
-    if not _REFERENCE.exists():
-        raise SystemExit("generated from the reference's own sources: /root/reference is needed")
+    if not reference_available():
+        raise SystemExit("generated from the reference's own build: oracle/_ref or its sources are needed")
     res = {"generator": "tests/golden/make_golden_long.py", "counters": list(COUNTERS),
            "provenance": "outputs of the UNMODIFIED reference sources built into oracle/_ref/libmlmap_ref.so (see golden.json)",
            "series": {n: run(n, "reference") for n in SERIES}}

@@ -4,6 +4,7 @@ product package."""
 from __future__ import annotations
 
 import ctypes as C
+import os
 import subprocess
 import sys
 from pathlib import Path
@@ -17,7 +18,9 @@ from mlmapping_b200.capi import FrameStats, MlmConfig  # noqa: E402  (struct lay
 _ORACLE_DIR = ROOT / "oracle"
 _LIB = _ORACLE_DIR / "liboracle.so"
 _REF_LIB = _ORACLE_DIR / "_ref" / "libmlmap_ref.so"  # the UNMODIFIED reference sources (oracle/ref_build/Makefile)
-_REFERENCE = Path("/root/reference")
+# a checkout of the original MLMapping sources (the repository does not ship them): MLMAPPING_REFERENCE, else the
+# documented place
+_REFERENCE = Path(os.environ.get("MLMAPPING_REFERENCE") or "/root/reference")
 _lib = None
 _ref_lib = None
 
@@ -30,26 +33,32 @@ def build_oracle():
 
 
 def build_reference():
-    """compile the reference's own mapping sources into oracle/_ref (only possible where /root/reference exists)"""
-    res = subprocess.run(["make", "-C", str(_ORACLE_DIR / "ref_build"), "-j8"], capture_output=True, text=True)
+    """compile the reference's own mapping sources (_REFERENCE) into oracle/_ref"""
+    res = subprocess.run(["make", "-C", str(_ORACLE_DIR / "ref_build"), "-j8", f"REF={_REFERENCE}"], capture_output=True,
+                         text=True)
     if res.returncode != 0:
         raise RuntimeError("oracle/_ref build failed:\n" + res.stdout[-3000:] + res.stderr[-3000:])
     return _REF_LIB
 
 
+def reference_sources() -> bool:
+    """the original sources are there and readable (os.path.isdir is False, not an error, where a user may not look)"""
+    return os.path.isdir(_REFERENCE)
+
+
 def reference_available() -> bool:
-    """the prebuilt library travels to the GPU box; the sources do not"""
-    return _REF_LIB.exists() or _REFERENCE.exists()
+    """a library built earlier, or the sources to build it from"""
+    return _REF_LIB.exists() or reference_sources()
 
 
 def load_reference():
     global _ref_lib
     if _ref_lib is not None:
         return _ref_lib
-    if _REFERENCE.exists():
+    if reference_sources():
         build_reference()  # make: a no-op when up to date
     if not _REF_LIB.exists():
-        raise FileNotFoundError(f"{_REF_LIB} missing and /root/reference absent: build it where the reference exists")
+        raise FileNotFoundError(f"{_REF_LIB} missing and no original sources at {_REFERENCE} (MLMAPPING_REFERENCE)")
     _ref_lib = _prototypes(C.CDLL(str(_REF_LIB)))
     _ref_lib.orc_get_odd_at.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]
     return _ref_lib
@@ -113,7 +122,7 @@ def _prototypes(lib):
 
 def best_oracle(cfg, **kw):
     """the checker the GPU parity tests use: the reference's own sources (oracle/_ref) when that library is available
-    (built here from /root/reference; the prebuilt file travels to the GPU box), else the restatement"""
+    (built from _REFERENCE), else the restatement"""
     return Oracle(cfg, impl="reference" if reference_available() else "port", **kw)
 
 

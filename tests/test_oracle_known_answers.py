@@ -16,7 +16,7 @@ from order_model import BUCKET_CHAIN, iteration_order, vector_hash
 @pytest.fixture(scope="module", params=["port", "reference"])
 def impl(request):
     if request.param == "reference" and not reference_available():
-        pytest.skip("oracle/_ref/libmlmap_ref.so not built and /root/reference absent")
+        pytest.skip("needs the reference build: oracle/_ref, or the original sources (MLMAPPING_REFERENCE)")
     return request.param
 
 

@@ -4,8 +4,10 @@ src/mlmap.cpp, src/rviz_vis.cpp, include/*.h, vendored Sophus, built where they 
 Same seeded inputs into both; everything the reference exposes must be identical bit for bit: the hit map in its
 iteration order with its probabilities, the miss set in ITS iteration order, the counters, the whole local map, the
 queries, box fill, inflation, frontiers, collapsed subboxes, the published clouds and the forwarded pose.
-Where /root/reference does not exist (the GPU box) the prebuilt library is used; with neither, these tests skip and
-tests/golden/golden.json (generated from the same library) keeps the restatement pinned."""
+Every test first holds the restatement (and the reference build, where it is available) to the stored outputs in
+tests/golden/reference_pin.json (make_golden_pin.py: counters and digests of everything compared below, same inputs), so
+the comparisons hold where the reference's own build is not available; the live comparisons follow where it is
+(oracle/_ref prebuilt, or the sources at MLMAPPING_REFERENCE, else /root/reference)."""
 import ctypes as C
 import json
 from pathlib import Path
@@ -16,7 +18,18 @@ import pytest
 from mlmapping_b200 import config_cfg_a, config_cfg_b, config_cfg_c, scenes
 from oracle_binding import Oracle, _d7, load_oracle, load_reference, reference_available
 
-pytestmark = pytest.mark.skipif(not reference_available(), reason="oracle/_ref not built and /root/reference absent")
+PIN = json.loads((Path(__file__).parent / "golden" / "reference_pin.json").read_text())["cases"]
+
+
+def _pinned(name):
+    """the restatement, and the reference build where it is available, against the stored outputs; True where the live
+    comparison can follow"""
+    from golden.make_golden_pin import run_case
+    assert run_case(name) == PIN[name], ("restatement differs from the stored reference outputs", name)
+    if not reference_available():
+        return False
+    assert run_case(name, impl="reference") == PIN[name], ("reference build differs from the stored outputs", name)
+    return True
 
 
 def _bits(a):
@@ -43,11 +56,6 @@ def assert_same_map(p, r, tag):
     return mp
 
 
-def _rolled(pose, k):
-    a, b = 0.05 * np.sin(0.7 * k), 0.04 * np.cos(0.9 * k)
-    from golden.make_golden import _quat_mul
-    q = _quat_mul(pose[3:7], _quat_mul([np.cos(a / 2), np.sin(a / 2), 0, 0], [np.cos(b / 2), 0, np.sin(b / 2), 0]))
-    return np.r_[pose[:3], q]
 
 
 def test_golden_vectors_come_from_the_reference_and_the_restatement_reproduces_them():
@@ -56,11 +64,15 @@ def test_golden_vectors_come_from_the_reference_and_the_restatement_reproduces_t
     assert "UNMODIFIED reference sources" in meta["provenance"]
     for name in CASES:
         want = meta["cases"][name]
-        assert run_case(name, impl="reference") == want, ("reference build no longer reproduces its golden vectors", name)
+        if reference_available():
+            assert run_case(name, impl="reference") == want, ("reference build no longer reproduces its golden vectors", name)
         assert run_case(name, impl="port") == want, ("restatement differs from the reference", name)
 
 
 def test_depth_trajectory_with_rolled_poses_queries_and_clouds():
+    if not _pinned("depth_trajectory"):
+        return
+    from golden.make_golden_pin import rolled as _rolled
     cfg = config_cfg_a()
     cfg.inflate_n, cfg.inflate_global_n = 2, 2
     p, r = Oracle(cfg), Oracle(cfg, impl="reference")
@@ -91,6 +103,8 @@ def test_depth_trajectory_with_rolled_poses_queries_and_clouds():
 
 
 def test_exploration_mode_frontiers_and_release():
+    if not _pinned("exploration"):
+        return
     cfg = config_cfg_a()
     cfg.use_exploration_frontiers = 1
     p, r = Oracle(cfg), Oracle(cfg, impl="reference")
@@ -109,6 +123,8 @@ def test_exploration_mode_frontiers_and_release():
 
 
 def test_lidar_points_and_the_large_configs():
+    if not _pinned("lidar_and_cfg_b"):
+        return
     cfg = config_cfg_c()
     cfg.am_n_rho, cfg.am_n_z_below, cfg.am_n_z_over = 120, 30, 30
     p, r = Oracle(cfg), Oracle(cfg, impl="reference")
@@ -129,6 +145,8 @@ def test_lidar_points_and_the_large_configs():
 
 def test_sampled_projection_is_the_references_own_project_depth():
     """mlmapping_sample_cnt > 0: here the reference's own mlmap::project_depth (src/mlmap.cpp:311-349) runs on its cv::Mat"""
+    if not _pinned("sampled_projection"):
+        return
     cfg = config_cfg_a()
     cfg.sample_cnt = 400
     libc = C.CDLL("libc.so.6")
@@ -150,6 +168,11 @@ def test_prologue_transform_and_pose_forwarding_bit_for_bit():
     """T_ls = T_wa^-1 * (T_wb * T_bs), T_ls * p and the callback's pose forwarding: restatement == reference build ==
     the product's host code (mlm_compensate_pose), on general (rolled, pitched, unnormalised) quaternions"""
     from mlmapping_b200 import compensate_pose
+    from golden.make_golden_pin import d, prologue_inputs
+    _, fwd = prologue_inputs()
+    assert d(np.array([compensate_pose(*f) for f in fwd])) == PIN["prologue"]["compensate_pose"]
+    if not _pinned("prologue"):
+        return
     a, b = load_oracle(), load_reference()
     rng = np.random.default_rng(0)
     for i in range(1500):
@@ -181,6 +204,8 @@ def test_prologue_transform_and_pose_forwarding_bit_for_bit():
 
 def test_get_odd_by_index_overload():
     """getOdd(const Vec3I&, size_t) (mlmap.h:128,227-235) of the reference on lattice indices"""
+    if not _pinned("odd_by_index"):
+        return
     cfg = config_cfg_a()
     r = Oracle(cfg, impl="reference")
     pose = scenes.corridor_trajectory_pose(0)
