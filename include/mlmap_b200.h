@@ -191,6 +191,42 @@ int mlm_get_occupancy_device(mlm_handle h, const double *d_pos, size_t n, int32_
 int mlm_get_odd_device(mlm_handle h, const double *d_pos, size_t n, float *d_out);
 int mlm_get_odd_grad_device(mlm_handle h, const double *d_pos, size_t n, size_t max_iter, double *d_out3n);
 
+/* Batched ray casting (no reference counterpart; the query octomap::OcTree::castRay users know): for each segment
+ * from[i] -> to[i] (n x 3 doubles, world frame) the cells it crosses, up to the first blocking one.
+ *  1. Cell of a point: c_k = (int)floor(p_k / d_sub) per axis, d_sub = subbox_d_xyz, IEEE division (get_subbox_id's
+ *     floor(pt / d_sub), reference include/map_local.h:167-173).  This is the canonical cell: the id-0 quirk that
+ *     getOccupancy inherits from unordered_map::operator[] applies to point queries only.
+ *  2. Traversal, a 6-connected DDA bounded by integer steps: c = cell(from), e = cell(to), rem_k = |e_k - c_k|,
+ *     s_k = sign(e_k - c_k), v_k = to_k - from_k.  For each axis with rem_k > 0, inv_k = 1.0 / v_k once, and the next
+ *     boundary t_k = ((double)(c_k + (s_k > 0)) * d_sub - from_k) * inv_k, recomputed from the integer cell after every
+ *     step.  A step takes, among the axes with rem_k > 0, the one with the smallest t_k (ties: x, then y, then z; an
+ *     axis replaces an earlier one only when its t_k compares strictly smaller), sets c_k += s_k, rem_k -= 1 and
+ *     t_enter = t_k.  The walk visits |e - c|_1 + 1 cells and ends in e; rounding can only reorder axis steps.  All
+ *     arithmetic is IEEE double without fused multiply-add.
+ *  3. State of a cell: what getOccupancy returns for it: subbox absent -> UNKNOWN, collapsed -> its element 0, else
+ *     occupancy[cell].  A cell blocks when its state is OCCUPIED; with MLM_RAY_INFLATED also when getInflateOccupancy
+ *     of it is OCCUPIED (inflate_occupancy[cell] == 'o'; a collapsed subbox never blocks by inflation, reference
+ *     include/mlmap.h:195-211).
+ *  4. Output: one record per segment.  The walk stops at the first blocking cell, which may be the start cell;
+ *     from == to is one cell.
+ * mlm_cast_rays stages through the handle's stream and returns when the records are in `out`; mlm_cast_rays_device
+ * takes device pointers and only enqueues.  flags is 0 or MLM_RAY_INFLATED.  A rank of a sharded map with world > 1
+ * returns MLM_ERR_UNSUPPORTED: a segment crosses subboxes of several owners (replica handles and world-1 shards hold
+ * the whole map and answer). */
+#define MLM_RAY_INFLATED 1
+#define MLM_RAY_INVALID (-2)
+typedef struct mlm_ray_hit {
+  int32_t status;    /* MLM_OCCUPIED: stopped at a blocking cell; MLM_FREE: reached cell(to) without one;
+                        MLM_RAY_INVALID: a non-finite endpoint, |p / d_sub| >= 2^30, or |e - c|_1 > 2^20 cells */
+  int32_t cell[3];   /* the stop cell: the first blocking cell, or cell(to); {0,0,0} when INVALID */
+  int32_t n_free;    /* non-blocking cells visited whose state is FREE (the end cell included when status is FREE) */
+  int32_t n_unknown; /* non-blocking cells visited whose state is UNKNOWN */
+  double t;          /* t_enter of the stop cell clamped to [0, 1] (NaN -> 0); 0 for the start cell */
+} mlm_ray_hit;
+int mlm_cast_rays(mlm_handle h, const double *from, const double *to, size_t n, int flags, mlm_ray_hit *out);
+int mlm_cast_rays_device(mlm_handle h, const double *d_from, const double *d_to, size_t n, int flags, mlm_ray_hit *d_out);
+size_t mlm_sizeof_ray_hit(void);
+
 /* ---- stream control / timing (CUDA events on the handle's own stream) ------------------------- */
 
 int mlm_sync(mlm_handle h);

@@ -109,6 +109,19 @@ class ShardExchange(C.Structure):
         return {k: getattr(self, k) for k, _ in self._fields_}
 
 
+RAY_INFLATED, RAY_INVALID = 1, -2  # MLM_RAY_INFLATED, MLM_RAY_INVALID
+
+
+class RayHit(C.Structure):
+    """mirror of mlm_ray_hit (include/mlmap_b200.h): one record of mlm_cast_rays"""
+    _fields_ = [("status", C.c_int32), ("cell", C.c_int32 * 3), ("n_free", C.c_int32), ("n_unknown", C.c_int32),
+                ("t", C.c_double)]
+
+
+# the same record as a numpy dtype: MLMap.cast_rays returns arrays of it
+RAY_HIT_DTYPE = np.dtype([("status", "<i4"), ("cell", "<i4", (3,)), ("n_free", "<i4"), ("n_unknown", "<i4"), ("t", "<f8")])
+
+
 # every symbol include/mlmap_b200.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
     "mlm_default_config", "mlm_create", "mlm_destroy", "mlm_last_error", "mlm_abi_version",
@@ -129,6 +142,7 @@ ABI_SYMBOLS = [
     "mlm_export_cloud", "mlm_export_cloud_device", "mlm_export_odds_slice",
     "mlm_checkpoint_size", "mlm_checkpoint_save", "mlm_checkpoint_restore", "mlm_compensate_pose",
     "mlm_export_cloud", "mlm_export_cloud_device", "mlm_export_odds_slice",
+    "mlm_cast_rays", "mlm_cast_rays_device", "mlm_sizeof_ray_hit",
 ]
 FRAME_KERNELS = ["k_project", "k_column", "k_fuse"]
 
@@ -183,6 +197,9 @@ def load_library() -> C.CDLL:
         "mlm_get_occupancy_device": ([vp, vp, sz, vp], C.c_int),
         "mlm_get_odd_device": ([vp, vp, sz, vp], C.c_int),
         "mlm_get_odd_grad_device": ([vp, vp, sz, sz, vp], C.c_int),
+        "mlm_cast_rays": ([vp, vp, vp, sz, C.c_int, vp], C.c_int),
+        "mlm_cast_rays_device": ([vp, vp, vp, sz, C.c_int, vp], C.c_int),
+        "mlm_sizeof_ray_hit": ([], C.c_size_t),
         "mlm_sync": ([vp], C.c_int),
         "mlm_timer_start": ([vp], C.c_int),
         "mlm_timer_stop_ms": ([vp, fp], C.c_int),
@@ -244,7 +261,8 @@ def load_library() -> C.CDLL:
         fn = getattr(lib, name)
         fn.argtypes = args
         fn.restype = ret
-    if lib.mlm_sizeof_config() != C.sizeof(MlmConfig) or lib.mlm_sizeof_frame_stats() != C.sizeof(FrameStats):
+    if (lib.mlm_sizeof_config() != C.sizeof(MlmConfig) or lib.mlm_sizeof_frame_stats() != C.sizeof(FrameStats)
+            or not lib.mlm_sizeof_ray_hit() == C.sizeof(RayHit) == RAY_HIT_DTYPE.itemsize):
         raise MlmError(1, "ctypes struct layout does not match include/mlmap_b200.h")
     _lib = lib
     return lib
@@ -496,6 +514,23 @@ class MLMap:
         out = np.empty((p.shape[0], 3), dtype=np.float64)
         self._check(self._lib.mlm_get_odd_grad(self._h, p.ctypes.data, p.shape[0], max_iter, out.ctypes.data))
         return out
+
+    # ---- batched ray casting (no reference counterpart; spec in include/mlmap_b200.h) ----------------
+    def cast_rays(self, from_, to, inflated: bool = False) -> np.ndarray:
+        """segments from_[i] -> to[i] ((n,3) world coordinates) walked cell by cell up to the first blocking cell:
+        a structured array of RAY_HIT_DTYPE (status OCCUPIED / FREE / RAY_INVALID, stop cell, free and unknown cells
+        crossed, t of the stop cell).  inflated: cells of the inflation layer block too."""
+        a, b = self._pos(from_), self._pos(to)
+        if a.shape != b.shape:
+            raise ValueError(f"from_ and to differ in shape: {a.shape} vs {b.shape}")
+        out = np.empty(a.shape[0], dtype=RAY_HIT_DTYPE)
+        self._check(self._lib.mlm_cast_rays(self._h, a.ctypes.data, b.ctypes.data, a.shape[0],
+                                            RAY_INFLATED if inflated else 0, out.ctypes.data))
+        return out
+
+    def cast_rays_device(self, d_from: int, d_to: int, n: int, d_out: int, inflated: bool = False):
+        """the same on device memory (n x 3 doubles each, n 32-byte records); only enqueues on the handle's stream"""
+        self._check(self._lib.mlm_cast_rays_device(self._h, d_from, d_to, n, RAY_INFLATED if inflated else 0, d_out))
 
     # ---- stream / timing -------------------------------------------------------------------------
     def sync(self):

@@ -23,6 +23,7 @@
 #include "explore_kernels.cuh"
 #include "query_kernels.cuh"
 #include "shard_kernels.cuh"
+#include "ray_kernels.cuh"
 
 using namespace mlm;
 
@@ -1820,6 +1821,57 @@ int mlm_get_odd_grad_device(mlm_handle h, const double *d_pos, size_t n, size_t 
   if (n == 0) return MLM_OK;
   k_get_odd_grad<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, (int)max_iter, d_out3n);
   h->launches++;
+  return MLM_OK;
+}
+
+// ---- batched ray casting (ray_kernels.cuh) --------------------------------------------------------------------
+size_t mlm_sizeof_ray_hit(void) { return sizeof(mlm_ray_hit); }
+static_assert(sizeof(mlm_ray_hit) == sizeof(RayHit), "mlm_ray_hit / RayHit layouts differ");
+
+static int cast_rays_check(mlm_handle h, const void *from, const void *to, size_t n, int flags, const void *out) {
+  if (!h || ((!from || !to || !out) && n) || (flags != 0 && flags != MLM_RAY_INFLATED)) return MLM_ERR_INVALID_ARG;
+  if (h->shard_world > 1) {
+    g_last_error = "mlm_cast_rays: a rank of a sharded map holds only the subboxes it owns";
+    return MLM_ERR_UNSUPPORTED;
+  }
+  return MLM_OK;
+}
+static void cast_rays_launch(mlm_handle h, const double *d_from, const double *d_to, size_t n, int flags, mlm_ray_hit *d_out) {
+  RayHit *o = reinterpret_cast<RayHit *>(d_out);
+  if (flags & MLM_RAY_INFLATED) k_cast_rays<true><<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_from, d_to, n, o);
+  else k_cast_rays<false><<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_from, d_to, n, o);
+  h->launches++;
+}
+int mlm_cast_rays_device(mlm_handle h, const double *d_from, const double *d_to, size_t n, int flags, mlm_ray_hit *d_out) {
+  const int rc = cast_rays_check(h, d_from, d_to, n, flags, d_out);
+  if (rc != MLM_OK) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (n == 0) return MLM_OK;
+  cast_rays_launch(h, d_from, d_to, n, flags, d_out);
+  return MLM_OK;
+}
+// the host variant stages both endpoint arrays and the records through the handle's stream (like host_query)
+int mlm_cast_rays(mlm_handle h, const double *from, const double *to, size_t n, int flags, mlm_ray_hit *out) {
+  const int rc = cast_rays_check(h, from, to, n, flags, out);
+  if (rc != MLM_OK) return rc;
+  if (n == 0) return MLM_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  double *d_ft = nullptr;
+  mlm_ray_hit *d_o = nullptr;
+  CUDA_TRY(cudaMallocAsync((void **)&d_ft, n * 48, s));
+  CUDA_TRY(cudaMallocAsync((void **)&d_o, n * sizeof(mlm_ray_hit), s));
+  cudaError_t e = cudaMemcpyAsync(d_ft, from, n * 24, cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) e = cudaMemcpyAsync(d_ft + 3 * n, to, n * 24, cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) {
+    cast_rays_launch(h, d_ft, d_ft + 3 * n, n, flags, d_o);
+    e = cudaMemcpyAsync(out, d_o, n * sizeof(mlm_ray_hit), cudaMemcpyDeviceToHost, s);
+  }
+  cudaFreeAsync(d_ft, s);
+  cudaFreeAsync(d_o, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  CUDA_TRY(e);
+  CUDA_TRY(cudaGetLastError());
   return MLM_OK;
 }
 

@@ -179,6 +179,17 @@ class mlmap {
   void getOddGrad(const Vec3 *pos_w, size_t n, Vec3 *out, size_t max_iter = 5) {
     check(mlm_get_odd_grad(h_, pos_w->v, n, max_iter, out->v), "mlm_get_odd_grad");
   }
+  // segment traversal up to the first blocking cell (no reference counterpart; spec at mlm_cast_rays): status
+  // OCCUPIED / FREE / MLM_RAY_INVALID, stop cell, free and unknown cells crossed, t of the stop cell
+  mlm_ray_hit castRay(const Vec3 &from, const Vec3 &to, bool inflated = false) {
+    mlm_ray_hit r;
+    check(mlm_cast_rays(h_, from.v, to.v, 1, inflated ? MLM_RAY_INFLATED : 0, &r), "mlm_cast_rays");
+    return r;
+  }
+  void castRays(const Vec3 *from, const Vec3 *to, size_t n, mlm_ray_hit *out, bool inflated = false) {
+    check(mlm_cast_rays(h_, n ? from->v : nullptr, n ? to->v : nullptr, n, inflated ? MLM_RAY_INFLATED : 0, out),
+          "mlm_cast_rays");
+  }
 
   // map clouds for consumers: what rviz_vis::pub_global_local_map / pub_frontier put on the wire
   // (src/rviz_vis.cpp:267-327) and mlmap::visualize_odds' slice (src/mlmap.cpp:200-284), compacted on the device.
