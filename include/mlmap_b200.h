@@ -227,6 +227,48 @@ int mlm_cast_rays(mlm_handle h, const double *from, const double *to, size_t n, 
 int mlm_cast_rays_device(mlm_handle h, const double *d_from, const double *d_to, size_t n, int flags, mlm_ray_hit *d_out);
 size_t mlm_sizeof_ray_hit(void);
 
+/* Signed distance field over a box of the map (no reference counterpart; the ESDF gradient-based planners expect):
+ * an exact Euclidean distance transform of the box's blocking cells, queried with trilinear interpolation.
+ *  1. Box: lo_k = cell(box_min_k), hi_k = cell(box_max_k) with the ray spec's rule 1 (which fails for a non-finite value
+ *     or |p / d_sub| >= 2^30), N_k = hi_k - lo_k + 1.  The grid holds the cells lo <= c <= hi.
+ *  2. Blocking set B: the cells of the box that block under the ray spec's rule 3, MLM_ESDF_INFLATED playing the part of
+ *     MLM_RAY_INFLATED (absent subbox: UNKNOWN, not blocking; collapsed: its element 0, never blocking by inflation;
+ *     else occupancy[cell] == 'o', or inflate_occupancy[cell] == 'o' with the flag).  With max_dist >= d_sub a cell
+ *     blocks a ray exactly when its value below is <= 0.  Unknown cells do not block.
+ *  3. Squared distances in cell units, exact integers over the cells of the box only:
+ *     D+(c) = min over b in B of |c - b|^2, D-(c) = min over f in box \ B of |c - f|^2; an empty set gives +inf.
+ *     Obstacles outside the box are not seen: pad the box by max_dist where they matter.
+ *  4. Cell value (double, metres): c not in B: v = min(sqrt((double)D+) * d_sub, max_dist); c in B:
+ *     v = d_sub - min(sqrt((double)D-) * d_sub, max_dist), where sqrt(+inf) * d_sub counts as above max_dist.  Free
+ *     cells are >= d_sub, surface obstacle cells 0, interior cells negative; an empty B gives max_dist everywhere, a
+ *     box without a free cell d_sub - max_dist.  IEEE sqrt, multiply and subtract, each correctly rounded.
+ *  5. Query at p (IEEE double, no fused multiply-add, in this order).  If cell(p) fails or lies outside the box:
+ *     dist = NaN (the quiet NaN 0x7ff8000000000000), grad = {0, 0, 0}.  Otherwise per axis q_k = p_k / d_sub - 0.5,
+ *     i_k = (int)floor(q_k), w_k = q_k - (double)i_k, u_k = 1.0 - w_k, and the corner indices
+ *     clamp(i_k - lo_k, 0, N_k - 1) and clamp(i_k - lo_k + 1, 0, N_k - 1) (the clamp acts in the box's outer half
+ *     cell only).  With v_xyz the corner values (x, y, z in {0, 1}) and g_yz = v_1yz - v_0yz:
+ *       e_yz = v_0yz * u_x + v_1yz * w_x;  f_z = e_0z * u_y + e_1z * w_y;  dist = f_0 * u_z + f_1 * w_z;
+ *       grad_z = (f_1 - f_0) / d_sub;  grad_y = ((e_10 - e_00) * u_z + (e_11 - e_01) * w_z) / d_sub;
+ *       grad_x = ((((g_00 * u_y) * u_z + (g_01 * u_y) * w_z) + (g_10 * w_y) * u_z) + (g_11 * w_y) * w_z) / d_sub.
+ *  6. Lifetime: the field is a snapshot of the map at mlm_esdf_build, in stream order; later frames, inflate_map,
+ *     set_free_in_bound or a checkpoint restore leave it as it is until the next build.  Querying or exporting before
+ *     any build returns MLM_ERR_INVALID_ARG.
+ * mlm_esdf_build and the _device calls only enqueue on the handle's stream; the host variants stage through it and
+ * return when the data is in place.  MLM_ERR_INVALID_ARG: null handle, null pointer with n > 0, flags other than 0 /
+ * MLM_ESDF_INFLATED, max_dist not finite or <= 0, a box corner that fails rule 1, box_min > box_max on an axis.
+ * MLM_ERR_CAPACITY: N_k > 4096 on an axis or N_x * N_y * N_z > 2^28 (keeps D+- below 2^26).  A rank of a sharded map
+ * with world > 1 returns MLM_ERR_UNSUPPORTED like mlm_cast_rays.  The grid buffers belong to the handle: allocated by
+ * the first build, grown for a larger box, freed by mlm_destroy.
+ * mlm_esdf_export writes the grid as float32 (float)v(c), x fastest: index (z * N_y + y) * N_x + x, x = c_x - lo_x...;
+ * lo3 and dims3 are always filled; out may be NULL with cap 0 to ask for the size; cap < N_x * N_y * N_z returns
+ * MLM_ERR_CAPACITY. */
+#define MLM_ESDF_INFLATED 1
+int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3], double max_dist, int flags);
+int mlm_esdf_distance(mlm_handle h, const double *pos, size_t n, double *dist, double *grad3n /* may be NULL */);
+int mlm_esdf_distance_device(mlm_handle h, const double *d_pos, size_t n, double *d_dist, double *d_grad3n /* may be NULL */);
+int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
+int mlm_esdf_export_device(mlm_handle h, float *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
+
 /* ---- stream control / timing (CUDA events on the handle's own stream) ------------------------- */
 
 int mlm_sync(mlm_handle h);

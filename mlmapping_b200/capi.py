@@ -121,6 +121,8 @@ class RayHit(C.Structure):
 # the same record as a numpy dtype: MLMap.cast_rays returns arrays of it
 RAY_HIT_DTYPE = np.dtype([("status", "<i4"), ("cell", "<i4", (3,)), ("n_free", "<i4"), ("n_unknown", "<i4"), ("t", "<f8")])
 
+ESDF_INFLATED = 1  # MLM_ESDF_INFLATED
+
 
 # every symbol include/mlmap_b200.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
@@ -143,6 +145,7 @@ ABI_SYMBOLS = [
     "mlm_checkpoint_size", "mlm_checkpoint_save", "mlm_checkpoint_restore", "mlm_compensate_pose",
     "mlm_export_cloud", "mlm_export_cloud_device", "mlm_export_odds_slice",
     "mlm_cast_rays", "mlm_cast_rays_device", "mlm_sizeof_ray_hit",
+    "mlm_esdf_build", "mlm_esdf_distance", "mlm_esdf_distance_device", "mlm_esdf_export", "mlm_esdf_export_device",
 ]
 FRAME_KERNELS = ["k_project", "k_column", "k_fuse"]
 
@@ -200,6 +203,11 @@ def load_library() -> C.CDLL:
         "mlm_cast_rays": ([vp, vp, vp, sz, C.c_int, vp], C.c_int),
         "mlm_cast_rays_device": ([vp, vp, vp, sz, C.c_int, vp], C.c_int),
         "mlm_sizeof_ray_hit": ([], C.c_size_t),
+        "mlm_esdf_build": ([vp, dp, dp, C.c_double, C.c_int], C.c_int),
+        "mlm_esdf_distance": ([vp, vp, sz, vp, vp], C.c_int),
+        "mlm_esdf_distance_device": ([vp, vp, sz, vp, vp], C.c_int),
+        "mlm_esdf_export": ([vp, vp, sz, ip, ip], C.c_int),
+        "mlm_esdf_export_device": ([vp, vp, sz, ip, ip], C.c_int),
         "mlm_sync": ([vp], C.c_int),
         "mlm_timer_start": ([vp], C.c_int),
         "mlm_timer_stop_ms": ([vp, fp], C.c_int),
@@ -531,6 +539,41 @@ class MLMap:
     def cast_rays_device(self, d_from: int, d_to: int, n: int, d_out: int, inflated: bool = False):
         """the same on device memory (n x 3 doubles each, n 32-byte records); only enqueues on the handle's stream"""
         self._check(self._lib.mlm_cast_rays_device(self._h, d_from, d_to, n, RAY_INFLATED if inflated else 0, d_out))
+
+    # ---- signed distance field over a box (no reference counterpart; spec in include/mlmap_b200.h) ------
+    def build_esdf(self, box_min, box_max, max_dist: float, inflated: bool = False):
+        """exact Euclidean distance transform of the box's blocking cells (occupied; with inflated also the inflation
+        layer), clamped to max_dist; a snapshot of the map until the next build.  Only enqueues."""
+        a = (C.c_double * 3)(*[float(v) for v in np.asarray(box_min, dtype=np.float64).reshape(3)])
+        b = (C.c_double * 3)(*[float(v) for v in np.asarray(box_max, dtype=np.float64).reshape(3)])
+        self._check(self._lib.mlm_esdf_build(self._h, a, b, float(max_dist), ESDF_INFLATED if inflated else 0))
+
+    def esdf_distance(self, pos_w):
+        """(dist[n], grad[n, 3]): trilinear distance and its gradient at (n,3) world points; NaN and a zero gradient
+        outside the box"""
+        p = self._pos(pos_w)
+        dist = np.empty(p.shape[0], dtype=np.float64)
+        grad = np.empty((p.shape[0], 3), dtype=np.float64)
+        self._check(self._lib.mlm_esdf_distance(self._h, p.ctypes.data, p.shape[0], dist.ctypes.data, grad.ctypes.data))
+        return dist, grad
+
+    def esdf_distance_device(self, d_pos: int, n: int, d_dist: int, d_grad: int = 0):
+        """the same on device memory (n x 3 doubles in, n doubles and optionally n x 3 doubles out); only enqueues"""
+        self._check(self._lib.mlm_esdf_distance_device(self._h, d_pos, n, d_dist, d_grad or None))
+
+    def export_esdf(self):
+        """(grid[N_z, N_y, N_x] float32, lo[3] int32): the cell values of the last build"""
+        lo, dims = (C.c_int32 * 3)(), (C.c_int32 * 3)()
+        self._check(self._lib.mlm_esdf_export(self._h, None, 0, lo, dims))
+        out = np.empty((dims[2], dims[1], dims[0]), dtype=np.float32)
+        self._check(self._lib.mlm_esdf_export(self._h, out.ctypes.data, out.size, lo, dims))
+        return out, np.array(lo[:], dtype=np.int32)
+
+    def export_esdf_device(self, d_out: int, cap: int):
+        """the grid into device memory of cap floats (only enqueues): (lo[3], dims[3] = N_x, N_y, N_z)"""
+        lo, dims = (C.c_int32 * 3)(), (C.c_int32 * 3)()
+        self._check(self._lib.mlm_esdf_export_device(self._h, d_out or None, cap, lo, dims))
+        return np.array(lo[:], dtype=np.int32), np.array(dims[:], dtype=np.int32)
 
     # ---- stream / timing -------------------------------------------------------------------------
     def sync(self):

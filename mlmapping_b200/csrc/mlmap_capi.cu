@@ -24,6 +24,7 @@
 #include "query_kernels.cuh"
 #include "shard_kernels.cuh"
 #include "ray_kernels.cuh"
+#include "esdf_kernels.cuh"
 
 using namespace mlm;
 
@@ -267,6 +268,13 @@ struct mlm_map {
   int profiling = 0;
   cudaEvent_t kev[MLM_NUM_FRAME_KERNELS + 1] = {};
   float kms[MLM_NUM_FRAME_KERNELS] = {};
+  // signed distance field (mlm_esdf_*): buffers of esdf_cap cells, grown by a larger box; esdf_a holds the cell values
+  // (double) after a build, esdf_grid the box of the last one
+  uint8_t *esdf_blk = nullptr;
+  int2 *esdf_a = nullptr, *esdf_b = nullptr, *esdf_stk = nullptr;
+  size_t esdf_cap = 0;
+  bool esdf_built = false;
+  EsdfGrid esdf_grid = {};
 };
 
 namespace {
@@ -1441,6 +1449,8 @@ int mlm_destroy(mlm_handle h) {
   mlm_shard_close(h);
   if (h->h_shard_state) cudaFreeHost(h->h_shard_state);
   for (void *p : h->allocs) cudaFree(p);
+  for (void *p : {(void *)h->esdf_blk, (void *)h->esdf_a, (void *)h->esdf_b, (void *)h->esdf_stk})
+    if (p) cudaFree(p);
   if (h->d_input) cudaFree(h->d_input);
   if (h->h_stage) cudaFreeHost(h->h_stage);
   if (h->l2_buf) cudaFree(h->l2_buf);
@@ -1869,6 +1879,184 @@ int mlm_cast_rays(mlm_handle h, const double *from, const double *to, size_t n, 
   }
   cudaFreeAsync(d_ft, s);
   cudaFreeAsync(d_o, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  CUDA_TRY(e);
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+// ---- signed distance field (esdf_kernels.cuh) ------------------------------------------------------------------
+static int esdf_refuse_sharded(mlm_handle h, const char *fn) {
+  if (h->shard_world <= 1) return MLM_OK;
+  g_last_error = std::string(fn) + ": a rank of a sharded map holds only the subboxes it owns";
+  return MLM_ERR_UNSUPPORTED;
+}
+// a field is there to query / export
+static int esdf_ready(mlm_handle h, const char *fn) {
+  const int rc = esdf_refuse_sharded(h, fn);
+  if (rc != MLM_OK) return rc;
+  if (!h->esdf_built) {
+    g_last_error = std::string(fn) + ": no signed distance field has been built (mlm_esdf_build first)";
+    return MLM_ERR_INVALID_ARG;
+  }
+  return MLM_OK;
+}
+static void esdf_free(mlm_handle h) {
+  for (void *p : {(void *)h->esdf_blk, (void *)h->esdf_a, (void *)h->esdf_b, (void *)h->esdf_stk})
+    if (p) cudaFree(p);
+  h->esdf_blk = nullptr;
+  h->esdf_a = h->esdf_b = h->esdf_stk = nullptr;
+  h->esdf_cap = 0;
+  h->esdf_built = false;
+}
+
+int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3], double max_dist, int flags) {
+  if (!h) return MLM_ERR_INVALID_ARG;
+  if (!box_min || !box_max || (flags != 0 && flags != MLM_ESDF_INFLATED) || !std::isfinite(max_dist) || !(max_dist > 0)) {
+    g_last_error = "mlm_esdf_build: null box, flags other than 0 / MLM_ESDF_INFLATED, or max_dist not finite and > 0";
+    return MLM_ERR_INVALID_ARG;
+  }
+  int rc = esdf_refuse_sharded(h, "mlm_esdf_build");
+  if (rc != MLM_OK) return rc;
+  EsdfGrid G = {};
+  const double d = h->P.d_sub;
+  const int n = h->P.n;
+  long long cells = 1;
+  for (int k = 0; k < 3; k++) {
+    // rule 1 of the ray spec: floor of the IEEE quotient, |p / d_sub| < 2^30
+    const double qa = box_min[k] / d, qb = box_max[k] / d;
+    if (!(std::fabs(qa) < 1073741824.0) || !(std::fabs(qb) < 1073741824.0) || !(box_min[k] <= box_max[k])) {
+      g_last_error = "mlm_esdf_build: a box corner is not finite, |p / d_sub| >= 2^30, or box_min > box_max";
+      return MLM_ERR_INVALID_ARG;
+    }
+    const int lo = (int)std::floor(qa), hi = (int)std::floor(qb);
+    const long long nk = (long long)hi - lo + 1;
+    if (nk > kEsdfMaxAxis) {
+      g_last_error = "mlm_esdf_build: more than 4096 cells along an axis";
+      return MLM_ERR_CAPACITY;
+    }
+    cells *= nk;
+    G.lo[k] = lo;
+    G.dims[k] = (int)nk;
+    G.glo[k] = host_floor_div(lo, n);
+    G.gdims[k] = host_floor_div(hi, n) - G.glo[k] + 1;
+  }
+  if (cells > kEsdfMaxCells) {
+    g_last_error = "mlm_esdf_build: more than 2^28 cells in the box";
+    return MLM_ERR_CAPACITY;
+  }
+  G.d = d;
+  G.max_dist = max_dist;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if ((size_t)cells > h->esdf_cap) {  // grow: blocking bytes, two int2 grids (the first ends as the values), two stacks
+    esdf_free(h);
+    const size_t c = (size_t)cells;
+    cudaError_t e = cudaMalloc((void **)&h->esdf_blk, c);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&h->esdf_a, c * sizeof(int2));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&h->esdf_b, c * sizeof(int2));
+    if (e == cudaSuccess) e = cudaMalloc((void **)&h->esdf_stk, 2 * c * sizeof(int2));
+    if (e != cudaSuccess) {
+      esdf_free(h);
+      cudaGetLastError();
+      g_last_error = std::string("mlm_esdf_build: grid buffers: ") + cudaGetErrorString(e);
+      return MLM_ERR_CUDA;
+    }
+    h->esdf_cap = c;
+  }
+  cudaStream_t s = h->stream;
+  const int subs = G.gdims[0] * G.gdims[1] * G.gdims[2];
+  if (flags & MLM_ESDF_INFLATED) k_esdf_gather<true><<<subs, 256, 0, s>>>(h->P, h->D, G, h->esdf_blk);
+  else k_esdf_gather<false><<<subs, 256, 0, s>>>(h->P, h->D, G, h->esdf_blk);
+  k_esdf_x<<<G.dims[1] * G.dims[2], 256, 0, s>>>(G, h->esdf_blk, h->esdf_a);
+  const int gx = (G.dims[0] + kEsdfLineThreads - 1) / kEsdfLineThreads;
+  k_esdf_y<<<dim3(gx, G.dims[2]), kEsdfLineThreads, 0, s>>>(G, h->esdf_a, h->esdf_b, h->esdf_stk);
+  k_esdf_z<<<dim3(gx, G.dims[1]), kEsdfLineThreads, 0, s>>>(G, h->esdf_b, reinterpret_cast<double *>(h->esdf_a),
+                                                            h->esdf_stk);
+  h->launches += 4;
+  CUDA_TRY(cudaGetLastError());
+  h->esdf_grid = G;
+  h->esdf_built = true;
+  return MLM_OK;
+}
+
+int mlm_esdf_distance_device(mlm_handle h, const double *d_pos, size_t n, double *d_dist, double *d_grad3n) {
+  if (!h || ((!d_pos || !d_dist) && n)) return MLM_ERR_INVALID_ARG;
+  const int rc = esdf_ready(h, "mlm_esdf_distance");
+  if (rc != MLM_OK) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (n == 0) return MLM_OK;
+  k_esdf_query<<<grid_for(n, 256), 256, 0, h->stream>>>(h->esdf_grid, reinterpret_cast<const double *>(h->esdf_a),
+                                                        d_pos, n, d_dist, d_grad3n);
+  h->launches++;
+  return MLM_OK;
+}
+// the host variant stages the points, distances and gradients through the handle's stream (like mlm_cast_rays)
+int mlm_esdf_distance(mlm_handle h, const double *pos, size_t n, double *dist, double *grad3n) {
+  if (!h || ((!pos || !dist) && n)) return MLM_ERR_INVALID_ARG;
+  const int rc = esdf_ready(h, "mlm_esdf_distance");
+  if (rc != MLM_OK) return rc;
+  if (n == 0) return MLM_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  double *d_buf = nullptr;  // points, distances, gradients
+  const size_t words = n * (grad3n ? 7 : 4);
+  CUDA_TRY(cudaMallocAsync((void **)&d_buf, words * sizeof(double), s));
+  double *d_pos = d_buf, *d_dist = d_buf + 3 * n, *d_grad = grad3n ? d_buf + 4 * n : nullptr;
+  cudaError_t e = cudaMemcpyAsync(d_pos, pos, n * 24, cudaMemcpyHostToDevice, s);
+  if (e == cudaSuccess) {
+    k_esdf_query<<<grid_for(n, 256), 256, 0, s>>>(h->esdf_grid, reinterpret_cast<const double *>(h->esdf_a), d_pos, n,
+                                                  d_dist, d_grad);
+    h->launches++;
+    e = cudaMemcpyAsync(dist, d_dist, n * 8, cudaMemcpyDeviceToHost, s);
+  }
+  if (e == cudaSuccess && grad3n) e = cudaMemcpyAsync(grad3n, d_grad, n * 24, cudaMemcpyDeviceToHost, s);
+  cudaFreeAsync(d_buf, s);
+  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+  CUDA_TRY(e);
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+// lo3 / dims3 always; the grid when out has room for it (out == NULL with cap 0 asks for the size only)
+static int esdf_export_check(mlm_handle h, const float *out, size_t cap, int32_t lo3[3], int32_t dims3[3], size_t &cells) {
+  if (!h || !lo3 || !dims3) return MLM_ERR_INVALID_ARG;
+  const int rc = esdf_ready(h, "mlm_esdf_export");
+  if (rc != MLM_OK) return rc;
+  const EsdfGrid &G = h->esdf_grid;
+  for (int k = 0; k < 3; k++) {
+    lo3[k] = G.lo[k];
+    dims3[k] = G.dims[k];
+  }
+  cells = (size_t)G.dims[0] * G.dims[1] * G.dims[2];
+  if (!out && cap == 0) return MLM_OK;
+  if (!out) return MLM_ERR_INVALID_ARG;
+  if (cap < cells) {
+    g_last_error = "mlm_esdf_export: cap is smaller than N_x * N_y * N_z";
+    return MLM_ERR_CAPACITY;
+  }
+  return MLM_OK;
+}
+int mlm_esdf_export_device(mlm_handle h, float *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]) {
+  size_t cells = 0;
+  const int rc = esdf_export_check(h, d_out, cap, lo3, dims3, cells);
+  if (rc != MLM_OK || !d_out) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  k_esdf_export<<<grid_for(cells, 256), 256, 0, h->stream>>>(reinterpret_cast<const double *>(h->esdf_a), cells, d_out);
+  h->launches++;
+  return MLM_OK;
+}
+int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_t dims3[3]) {
+  size_t cells = 0;
+  const int rc = esdf_export_check(h, out, cap, lo3, dims3, cells);
+  if (rc != MLM_OK || !out) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  float *d_out = nullptr;
+  CUDA_TRY(cudaMallocAsync((void **)&d_out, cells * sizeof(float), s));
+  k_esdf_export<<<grid_for(cells, 256), 256, 0, s>>>(reinterpret_cast<const double *>(h->esdf_a), cells, d_out);
+  h->launches++;
+  cudaError_t e = cudaMemcpyAsync(out, d_out, cells * sizeof(float), cudaMemcpyDeviceToHost, s);
+  cudaFreeAsync(d_out, s);
   if (e == cudaSuccess) e = cudaStreamSynchronize(s);
   CUDA_TRY(e);
   CUDA_TRY(cudaGetLastError());

@@ -34,6 +34,33 @@ __device__ __forceinline__ bool ray_cell(double p, double d, int &c) {
   return true;
 }
 
+// A subbox as a byte pointer per layer and an index mask: pool block (mask ~0: cell `sub`), collapsed (occupancy: its
+// element 0; inflation: an unknown byte, so it never blocks by inflation) or absent (both read an unknown byte).  The ray
+// walk and the ESDF gather (esdf_kernels.cuh) read cells through it, so the two agree on the blocking rule.
+struct SubboxView {
+  const char *occ, *inf;
+  int mask;
+};
+__device__ __forceinline__ SubboxView subbox_view(const MapParams &P, const DeviceBuffers &D, const int g[3]) {
+  uint32_t slot;
+  const int blk = ht_find_slot(P, D, g, slot);
+  SubboxView v = {&g_ray_unknown_cell, &g_ray_unknown_cell, 0};
+  if (blk >= 0) {
+    v.occ = D.pool_occ + (size_t)blk * P.cell_stride;
+    v.inf = D.pool_inf + (size_t)blk * P.cell_stride;
+    v.mask = ~0;
+  } else if (blk == kBlockCollapsed) {
+    v.occ = D.col_occ + slot;
+  }
+  return v;
+}
+// the spec's rule 3: `st` is the cell's state byte; with kInflated the inflation layer blocks too
+template <bool kInflated>
+__device__ __forceinline__ bool view_blocks(const SubboxView &v, int sub, char &st) {
+  st = __ldg(v.occ + (sub & v.mask));
+  return st == 'o' || (kInflated && __ldg(v.inf + (sub & v.mask)) == 'o');
+}
+
 // t of the next cell boundary on one axis, recomputed from the integer cell (no accumulation)
 __device__ __forceinline__ double ray_next_t(int c, int s, double d, double from, double inv) {
   return ((double)(c + (s > 0 ? 1 : 0)) * d - from) * inv;
@@ -76,32 +103,14 @@ __device__ __forceinline__ RayHit cast_ray(const MapParams &P, const DeviceBuffe
     loc[k] = c[k] - g[k] * n;
     sub += loc[k] * stride[k];
   }
-  // The current subbox as a byte pointer per layer and an index mask: pool block (mask ~0: cell `sub`), collapsed
-  // (occupancy: its element 0, inflation: never blocks) or absent (both read an unknown byte).  Every step then does the
-  // same one or two loads whatever kind of subbox it is in.
-  const char *occ = &g_ray_unknown_cell, *inf = &g_ray_unknown_cell;
-  int mask = 0;
-  auto enter = [&]() {
-    uint32_t slot;
-    const int blk = ht_find_slot(P, D, g, slot);
-    occ = inf = &g_ray_unknown_cell;
-    mask = 0;
-    if (blk >= 0) {
-      occ = D.pool_occ + (size_t)blk * P.cell_stride;
-      inf = D.pool_inf + (size_t)blk * P.cell_stride;
-      mask = ~0;
-    } else if (blk == kBlockCollapsed) {
-      occ = D.col_occ + slot;
-    }
-  };
-  enter();
+  // The current subbox (SubboxView): every step does the same one or two loads whatever kind of subbox it is in.
+  SubboxView view = subbox_view(P, D, g);
   int left = (int)total, n_free = 0, n_unknown = 0;
   double t_enter = 0.0;
   int status;
   for (;;) {
-    const char st = __ldg(occ + (sub & mask));
-    const bool blocking = st == 'o' || (kInflated && __ldg(inf + (sub & mask)) == 'o');
-    if (blocking) {
+    char st;
+    if (view_blocks<kInflated>(view, sub, st)) {
       status = 0;  // MLM_OCCUPIED
       break;
     }
@@ -151,7 +160,7 @@ __device__ __forceinline__ RayHit cast_ray(const MapParams &P, const DeviceBuffe
           g[k] += sa;
         }
       sub -= sa * n * stra;
-      enter();
+      view = subbox_view(P, D, g);
     }
   }
   r.status = status;

@@ -190,6 +190,19 @@ class mlmap {
     check(mlm_cast_rays(h_, n ? from->v : nullptr, n ? to->v : nullptr, n, inflated ? MLM_RAY_INFLATED : 0, out),
           "mlm_cast_rays");
   }
+  // signed distance field over a box (no reference counterpart; spec at mlm_esdf_build): a snapshot of the map until
+  // the next build; getEsdf is NaN with a zero gradient outside the box
+  void buildEsdf(const Vec3 &min, const Vec3 &max, double max_dist, bool inflated = false) {
+    check(mlm_esdf_build(h_, min.v, max.v, max_dist, inflated ? MLM_ESDF_INFLATED : 0), "mlm_esdf_build");
+  }
+  double getEsdf(const Vec3 &pos, Vec3 *grad = nullptr) {
+    double d;
+    check(mlm_esdf_distance(h_, pos.v, 1, &d, grad ? grad->v : nullptr), "mlm_esdf_distance");
+    return d;
+  }
+  void getEsdfs(const Vec3 *pos, size_t n, double *dist, Vec3 *grad = nullptr) {
+    check(mlm_esdf_distance(h_, n ? pos->v : nullptr, n, dist, grad ? grad->v : nullptr), "mlm_esdf_distance");
+  }
 
   // map clouds for consumers: what rviz_vis::pub_global_local_map / pub_frontier put on the wire
   // (src/rviz_vis.cpp:267-327) and mlmap::visualize_odds' slice (src/mlmap.cpp:200-284), compacted on the device.
