@@ -269,6 +269,49 @@ int mlm_esdf_distance_device(mlm_handle h, const double *d_pos, size_t n, double
 int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
 int mlm_esdf_export_device(mlm_handle h, float *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
 
+/* Frontier clustering (no reference counterpart; the first step of a frontier-based explorer's planning cycle):
+ * connected components of the exploration frontier sets, one record per cluster.
+ *  1. Frontier set F: a cell c = glb * subbox_n + local is in F when its bit is set in its subbox's frontier bitmask
+ *     (bit c of the little-endian words, cell ids < subbox_n^3 only): the cells mlm_export_frontier and
+ *     MLM_CLOUD_FRONTIER report.  Cell state is not looked at (a cell that mlm_set_free_in_bound made free keeps its
+ *     bit, as in the reference).  Absent and collapsed subboxes hold no frontier cells.  With a box, F is intersected
+ *     with cell(box_min) <= c <= cell(box_max) per axis, cell() being the ray spec's rule 1.
+ *  2. Clusters are the connected components of F.  Two cells a, b are adjacent when max_k |a_k - b_k| == 1
+ *     (26-connectivity, the default) or, with MLM_FRONTIER_CONN6, when sum_k |a_k - b_k| == 1.  Cells outside the box
+ *     connect nothing: a cluster the box cuts is split.
+ *  3. Record of a cluster: n_cells; key = its member smallest in (z, y, x) lexicographic order; lo / hi = the per-axis
+ *     minimum / maximum of its members; centroid_k = (((double)S_k / (double)n_cells) + 0.5) * d_sub with S_k the exact
+ *     int64 sum of the members' c_k, each operation IEEE double, correctly rounded, without fused multiply-add.
+ *  4. Output: the clusters with n_cells >= min_cells, sorted by key in (z, y, x) order; the cluster index is the position
+ *     in that list.  *n_out = the number of clusters kept, which may exceed cap (then only the first cap records are
+ *     written), as for mlm_export_cloud.
+ *  5. Per-cell labels (optional): every cell of a kept cluster as cells3[3 i .. 3 i + 2] with its cluster index in
+ *     cluster_of[i]; at most cell_cap of them are written, in unspecified (but repeatable) order; *n_cells_out (may be
+ *     NULL) = their total.
+ *  6. MLM_ERR_INVALID_ARG: null handle or n_out; only one of box_min / box_max given; a box corner that fails rule 1;
+ *     box_min > box_max on an axis; min_cells < 1; flags other than 0 / MLM_FRONTIER_CONN6; a null output pointer with a
+ *     non-zero cap (cells3 and cluster_of both for cell_cap).  MLM_ERR_UNSUPPORTED: a handle created without
+ *     use_exploration_frontiers, or a rank of a sharded map with world > 1 (a cluster crosses owners; as mlm_cast_rays).
+ *  7. The call is a snapshot of the map in stream order.  mlm_frontier_clusters returns once the records are in `out`;
+ *     mlm_frontier_clusters_device takes device pointers for out / cells3 / cluster_of.  Both synchronise the handle's
+ *     stream twice: for the number of frontier cells (which sizes the handle's scratch) and for the counts.  The scratch
+ *     buffers belong to the handle: allocated by the first call, grown for a larger frontier, freed by mlm_destroy. */
+#define MLM_FRONTIER_CONN6 1
+typedef struct mlm_frontier_cluster {
+  int32_t n_cells;
+  int32_t key[3];       /* smallest member cell in (z, y, x) lexicographic order */
+  int32_t lo[3], hi[3]; /* inclusive cell AABB of the members */
+  double centroid[3];   /* metres */
+} mlm_frontier_cluster; /* 64 bytes */
+size_t mlm_sizeof_frontier_cluster(void);
+int mlm_frontier_clusters(mlm_handle h, const double box_min[3], const double box_max[3] /* both NULL: whole map */,
+                          int32_t min_cells, int flags, mlm_frontier_cluster *out, size_t cap, size_t *n_out,
+                          int32_t *cells3 /* may be NULL */, int32_t *cluster_of /* may be NULL */, size_t cell_cap,
+                          size_t *n_cells_out /* may be NULL */);
+int mlm_frontier_clusters_device(mlm_handle h, const double box_min[3], const double box_max[3], int32_t min_cells,
+                                 int flags, mlm_frontier_cluster *d_out, size_t cap, size_t *n_out, int32_t *d_cells3,
+                                 int32_t *d_cluster_of, size_t cell_cap, size_t *n_cells_out);
+
 /* ---- stream control / timing (CUDA events on the handle's own stream) ------------------------- */
 
 int mlm_sync(mlm_handle h);

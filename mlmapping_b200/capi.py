@@ -122,6 +122,10 @@ class RayHit(C.Structure):
 RAY_HIT_DTYPE = np.dtype([("status", "<i4"), ("cell", "<i4", (3,)), ("n_free", "<i4"), ("n_unknown", "<i4"), ("t", "<f8")])
 
 ESDF_INFLATED = 1  # MLM_ESDF_INFLATED
+FRONTIER_CONN6 = 1  # MLM_FRONTIER_CONN6
+# mlm_frontier_cluster (include/mlmap_b200.h): one record of mlm_frontier_clusters, 64 bytes
+FRONTIER_CLUSTER_DTYPE = np.dtype([("n_cells", "<i4"), ("key", "<i4", (3,)), ("lo", "<i4", (3,)), ("hi", "<i4", (3,)),
+                                   ("centroid", "<f8", (3,))])
 
 
 # every symbol include/mlmap_b200.h declares (checked by tests/test_abi.py)
@@ -146,6 +150,7 @@ ABI_SYMBOLS = [
     "mlm_export_cloud", "mlm_export_cloud_device", "mlm_export_odds_slice",
     "mlm_cast_rays", "mlm_cast_rays_device", "mlm_sizeof_ray_hit",
     "mlm_esdf_build", "mlm_esdf_distance", "mlm_esdf_distance_device", "mlm_esdf_export", "mlm_esdf_export_device",
+    "mlm_frontier_clusters", "mlm_frontier_clusters_device", "mlm_sizeof_frontier_cluster",
 ]
 FRAME_KERNELS = ["k_project", "k_column", "k_fuse"]
 
@@ -208,6 +213,10 @@ def load_library() -> C.CDLL:
         "mlm_esdf_distance_device": ([vp, vp, sz, vp, vp], C.c_int),
         "mlm_esdf_export": ([vp, vp, sz, ip, ip], C.c_int),
         "mlm_esdf_export_device": ([vp, vp, sz, ip, ip], C.c_int),
+        "mlm_frontier_clusters": ([vp, dp, dp, C.c_int32, C.c_int, vp, sz, C.POINTER(sz), vp, vp, sz, C.POINTER(sz)], C.c_int),
+        "mlm_frontier_clusters_device": ([vp, dp, dp, C.c_int32, C.c_int, vp, sz, C.POINTER(sz), vp, vp, sz, C.POINTER(sz)],
+                                         C.c_int),
+        "mlm_sizeof_frontier_cluster": ([], C.c_size_t),
         "mlm_sync": ([vp], C.c_int),
         "mlm_timer_start": ([vp], C.c_int),
         "mlm_timer_stop_ms": ([vp, fp], C.c_int),
@@ -270,7 +279,8 @@ def load_library() -> C.CDLL:
         fn.argtypes = args
         fn.restype = ret
     if (lib.mlm_sizeof_config() != C.sizeof(MlmConfig) or lib.mlm_sizeof_frame_stats() != C.sizeof(FrameStats)
-            or not lib.mlm_sizeof_ray_hit() == C.sizeof(RayHit) == RAY_HIT_DTYPE.itemsize):
+            or not lib.mlm_sizeof_ray_hit() == C.sizeof(RayHit) == RAY_HIT_DTYPE.itemsize
+            or lib.mlm_sizeof_frontier_cluster() != FRONTIER_CLUSTER_DTYPE.itemsize):
         raise MlmError(1, "ctypes struct layout does not match include/mlmap_b200.h")
     _lib = lib
     return lib
@@ -574,6 +584,49 @@ class MLMap:
         lo, dims = (C.c_int32 * 3)(), (C.c_int32 * 3)()
         self._check(self._lib.mlm_esdf_export_device(self._h, d_out or None, cap, lo, dims))
         return np.array(lo[:], dtype=np.int32), np.array(dims[:], dtype=np.int32)
+
+    # ---- frontier clustering (no reference counterpart; spec in include/mlmap_b200.h) -------------------------
+    @staticmethod
+    def _frontier_box(box_min, box_max):
+        if (box_min is None) != (box_max is None):
+            raise ValueError("box_min and box_max go together")
+        if box_min is None:
+            return None, None
+        return tuple((C.c_double * 3)(*[float(v) for v in np.asarray(b, dtype=np.float64).reshape(3)]) for b in (box_min, box_max))
+
+    def frontier_clusters(self, box_min=None, box_max=None, min_cells: int = 1, conn6: bool = False, labels: bool = False):
+        """connected components of the frontier sets (26-connected, or 6 with conn6), optionally inside a box: the
+        clusters with >= min_cells cells as FRONTIER_CLUSTER_DTYPE records sorted by key (z, y, x); with labels also
+        (cells[m, 3] int32, cluster_of[m] int32), every cell of a kept cluster with its cluster index"""
+        a, b = self._frontier_box(box_min, box_max)
+        flags = FRONTIER_CONN6 if conn6 else 0
+        cap, cell_cap = self.__dict__.get("_fc_cap", 256), (self.__dict__.get("_fc_cell_cap", 4096) if labels else 0)
+        n, m = C.c_size_t(), C.c_size_t()
+        while True:
+            out = np.empty(cap, dtype=FRONTIER_CLUSTER_DTYPE)
+            cells = np.empty((cell_cap, 3), dtype=np.int32)
+            of = np.empty(cell_cap, dtype=np.int32)
+            self._check(self._lib.mlm_frontier_clusters(self._h, a, b, int(min_cells), flags, out.ctypes.data, cap,
+                                                        C.byref(n), cells.ctypes.data if labels else None,
+                                                        of.ctypes.data if labels else None, cell_cap, C.byref(m)))
+            if n.value <= cap and (not labels or m.value <= cell_cap):
+                break
+            cap, cell_cap = max(cap, n.value), (max(cell_cap, m.value) if labels else 0)  # too small: size and retry
+        self._fc_cap = cap
+        if labels:
+            self._fc_cell_cap = cell_cap
+            return out[:n.value].copy(), cells[:m.value].copy(), of[:m.value].copy()
+        return out[:n.value].copy()
+
+    def frontier_clusters_device(self, d_out: int, cap: int, d_cells3: int = 0, d_cluster_of: int = 0, cell_cap: int = 0,
+                                 box_min=None, box_max=None, min_cells: int = 1, conn6: bool = False):
+        """the same into device memory (cap 64-byte records; cell_cap cells and labels): (clusters, labelled cells)"""
+        a, b = self._frontier_box(box_min, box_max)
+        n, m = C.c_size_t(), C.c_size_t()
+        self._check(self._lib.mlm_frontier_clusters_device(self._h, a, b, int(min_cells), FRONTIER_CONN6 if conn6 else 0,
+                                                           d_out or None, cap, C.byref(n), d_cells3 or None,
+                                                           d_cluster_of or None, cell_cap, C.byref(m)))
+        return n.value, m.value
 
     # ---- stream / timing -------------------------------------------------------------------------
     def sync(self):

@@ -25,6 +25,7 @@
 #include "shard_kernels.cuh"
 #include "ray_kernels.cuh"
 #include "esdf_kernels.cuh"
+#include "frontier_kernels.cuh"
 
 using namespace mlm;
 
@@ -275,6 +276,10 @@ struct mlm_map {
   size_t esdf_cap = 0;
   bool esdf_built = false;
   EsdfGrid esdf_grid = {};
+  // frontier clustering (mlm_frontier_clusters*): per-word buffers allocated by the first call, per-cell buffers of
+  // fc_cap_cells entries grown by a larger frontier
+  FcScratch fc = {};
+  size_t fc_cap_cells = 0;
 };
 
 namespace {
@@ -1436,6 +1441,8 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   return MLM_OK;
 }
 
+static void frontier_free(mlm_handle h, bool all);
+
 int mlm_destroy(mlm_handle h) {
   if (!h) return MLM_ERR_INVALID_ARG;
   cudaSetDevice(h->device);
@@ -1451,6 +1458,7 @@ int mlm_destroy(mlm_handle h) {
   for (void *p : h->allocs) cudaFree(p);
   for (void *p : {(void *)h->esdf_blk, (void *)h->esdf_a, (void *)h->esdf_b, (void *)h->esdf_stk})
     if (p) cudaFree(p);
+  frontier_free(h, true);
   if (h->d_input) cudaFree(h->d_input);
   if (h->h_stage) cudaFreeHost(h->h_stage);
   if (h->l2_buf) cudaFree(h->l2_buf);
@@ -2061,6 +2069,171 @@ int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_
   CUDA_TRY(e);
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
+}
+
+// ---- frontier clustering (frontier_kernels.cuh) ------------------------------------------------------------------
+size_t mlm_sizeof_frontier_cluster(void) { return sizeof(mlm_frontier_cluster); }
+static_assert(sizeof(mlm_frontier_cluster) == sizeof(FrontierCluster), "mlm_frontier_cluster / FrontierCluster layouts differ");
+
+// all: the per-word buffers too (mlm_destroy); else the per-cell buffers only (before they grow)
+static void frontier_free(mlm_handle h, bool all) {
+  FcScratch &S = h->fc;
+  for (void *p : {(void *)S.parent, (void *)S.acc_n, (void *)S.acc_s, (void *)S.acc_lo, (void *)S.acc_hi,
+                  (void *)S.acc_key, (void *)S.map, (void *)S.sk[0], (void *)S.sk[1], (void *)S.sv[0], (void *)S.sv[1]})
+    if (p) cudaFree(p);
+  S.parent = S.acc_n = S.acc_lo = S.acc_hi = S.map = S.sv[0] = S.sv[1] = nullptr;
+  S.acc_s = S.acc_key = S.sk[0] = S.sk[1] = nullptr;
+  h->fc_cap_cells = 0;
+  if (!all) return;
+  for (void *p : {(void *)S.mword, (void *)S.wbase, (void *)S.slot_cnt, (void *)S.counters})
+    if (p) cudaFree(p);
+  S.mword = nullptr;
+  S.wbase = S.slot_cnt = S.counters = nullptr;
+}
+
+static int frontier_clusters(mlm_handle h, const double box_min[3], const double box_max[3], int32_t min_cells, int flags,
+                             mlm_frontier_cluster *out, size_t cap, size_t *n_out, int32_t *cells3, int32_t *cluster_of,
+                             size_t cell_cap, size_t *n_cells_out, bool device_out) {
+  if (!h || !n_out) return MLM_ERR_INVALID_ARG;
+  if ((!box_min) != (!box_max) || min_cells < 1 || (flags & ~MLM_FRONTIER_CONN6) || (!out && cap) ||
+      ((!cells3 || !cluster_of) && cell_cap)) {
+    g_last_error = "mlm_frontier_clusters: one box pointer without the other, min_cells < 1, unknown flags, or a null "
+                   "output with a non-zero cap";
+    return MLM_ERR_INVALID_ARG;
+  }
+  FcBox B = {{INT_MIN, INT_MIN, INT_MIN}, {INT_MAX, INT_MAX, INT_MAX}, 1};
+  if (box_min) {
+    B.whole = 0;
+    const double d = h->P.d_sub;
+    for (int k = 0; k < 3; k++) {
+      const double qa = box_min[k] / d, qb = box_max[k] / d;  // rule 1 of the ray spec
+      if (!(std::fabs(qa) < 1073741824.0) || !(std::fabs(qb) < 1073741824.0) || !(box_min[k] <= box_max[k])) {
+        g_last_error = "mlm_frontier_clusters: a box corner is not finite, |p / d_sub| >= 2^30, or box_min > box_max";
+        return MLM_ERR_INVALID_ARG;
+      }
+      B.lo[k] = (int)std::floor(qa);
+      B.hi[k] = (int)std::floor(qb);
+    }
+  }
+  if (!h->P.explore) {
+    g_last_error = "mlm_frontier_clusters: the handle was created without use_exploration_frontiers";
+    return MLM_ERR_UNSUPPORTED;
+  }
+  if (h->shard_world > 1) {
+    g_last_error = "mlm_frontier_clusters: a rank of a sharded map holds only the subboxes it owns";
+    return MLM_ERR_UNSUPPORTED;
+  }
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  const MapParams &P = h->P;
+  FcScratch &S = h->fc;
+  const int slots = (int)P.ht_mask + 1;
+  if (!S.mword) {
+    const size_t words = (size_t)P.pool_blocks * P.front_words;
+    cudaError_t e = cudaMalloc((void **)&S.mword, words * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&S.wbase, words * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&S.slot_cnt, ((size_t)slots + 1) * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&S.counters, 16 * 4);
+    if (e != cudaSuccess) {
+      frontier_free(h, true);
+      cudaGetLastError();
+      g_last_error = std::string("mlm_frontier_clusters: scratch: ") + cudaGetErrorString(e);
+      return MLM_ERR_CUDA;
+    }
+  }
+  const int wgrid = h->sm_count * 8;  // warp-per-slot kernels: one full wave of 256-thread CTAs, grid-stride over the slots
+  k_fc_count<<<wgrid, 256, 0, s>>>(P, h->D, B, S);
+  k_fc_scan<<<1, kFcScanThreads, 0, s>>>(S.slot_cnt, slots);
+  h->launches += 2;
+  int total = 0;
+  CUDA_TRY(cudaMemcpyAsync(&total, S.slot_cnt + slots, sizeof(int), cudaMemcpyDeviceToHost, s));
+  CUDA_TRY(cudaStreamSynchronize(s));  // the number of frontier cells sizes the per-cell buffers
+  if ((size_t)total > h->fc_cap_cells) {
+    frontier_free(h, false);
+    const size_t c = (size_t)total;
+    cudaError_t e = cudaSuccess;
+    for (int **p : {&S.parent, &S.acc_n, &S.map, &S.sv[0], &S.sv[1]})
+      if (e == cudaSuccess) e = cudaMalloc((void **)p, c * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&S.acc_lo, 3 * c * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&S.acc_hi, 3 * c * 4);
+    if (e == cudaSuccess) e = cudaMalloc((void **)&S.acc_s, 3 * c * 8);
+    for (unsigned long long **p : {&S.acc_key, &S.sk[0], &S.sk[1]})
+      if (e == cudaSuccess) e = cudaMalloc((void **)p, c * 8);
+    if (e != cudaSuccess) {
+      frontier_free(h, false);
+      cudaGetLastError();
+      g_last_error = std::string("mlm_frontier_clusters: per-cell buffers: ") + cudaGetErrorString(e);
+      return MLM_ERR_CUDA;
+    }
+    h->fc_cap_cells = c;
+  }
+  int counts[2] = {0, 0};  // clusters kept, cells of kept clusters
+  if (total > 0) {
+    const int cgrid = std::min(grid_for((size_t)total, 256), wgrid);
+    const int init[9] = {0, 0, INT_MAX, INT_MAX, INT_MAX, INT_MIN, INT_MIN, INT_MIN, 0};
+    k_fc_index<<<wgrid, 256, 0, s>>>(P, h->D, S);
+    if (flags & MLM_FRONTIER_CONN6) k_fc_hook<true><<<wgrid, 256, 0, s>>>(P, h->D, B, S);
+    else k_fc_hook<false><<<wgrid, 256, 0, s>>>(P, h->D, B, S);
+    k_fc_compress<<<cgrid, 256, 0, s>>>(S, total);
+    k_fc_reduce<0><<<wgrid, 256, 0, s>>>(P, h->D, S);
+    k_fc_reduce<1><<<wgrid, 256, 0, s>>>(P, h->D, S);
+    CUDA_TRY(cudaMemcpyAsync(S.counters, init, sizeof(init), cudaMemcpyHostToDevice, s));
+    k_fc_select<<<cgrid, 256, 0, s>>>(S, total, min_cells);
+    k_fc_sort<<<1, kFcSortThreads, 0, s>>>(S);
+    h->launches += 7;
+    FrontierCluster *d_out = reinterpret_cast<FrontierCluster *>(out);
+    int32_t *d_cells = cells3, *d_of = cluster_of;
+    const size_t rec_n = std::min(cap, (size_t)total), lab_n = std::min(cell_cap, (size_t)total);
+    cudaError_t e = cudaSuccess;
+    if (!device_out) {
+      d_out = nullptr;
+      d_cells = d_of = nullptr;
+      if (rec_n) e = cudaMallocAsync((void **)&d_out, rec_n * sizeof(FrontierCluster), s);
+      if (e == cudaSuccess && lab_n) e = cudaMallocAsync((void **)&d_cells, lab_n * 16, s);
+      d_of = d_cells ? d_cells + 3 * lab_n : nullptr;
+    }
+    if (e == cudaSuccess) {
+      k_fc_records<<<cgrid, 256, 0, s>>>(S, P.d_sub, d_out, rec_n);
+      h->launches++;
+      if (lab_n) {
+        k_fc_labels<false><<<wgrid, 256, 0, s>>>(P, h->D, S, nullptr, nullptr, 0);
+        k_fc_scan<<<1, kFcScanThreads, 0, s>>>(S.slot_cnt, slots);
+        k_fc_labels<true><<<wgrid, 256, 0, s>>>(P, h->D, S, d_cells, d_of, lab_n);
+        h->launches += 3;
+      }
+      e = cudaMemcpyAsync(counts, S.counters, sizeof(counts), cudaMemcpyDeviceToHost, s);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(s);  // the counts
+    }
+    if (!device_out && e == cudaSuccess) {
+      const size_t nr = std::min(rec_n, (size_t)counts[0]), nl = std::min(lab_n, (size_t)counts[1]);
+      if (nr) e = cudaMemcpyAsync(out, d_out, nr * sizeof(FrontierCluster), cudaMemcpyDeviceToHost, s);
+      if (e == cudaSuccess && nl) e = cudaMemcpyAsync(cells3, d_cells, nl * 12, cudaMemcpyDeviceToHost, s);
+      if (e == cudaSuccess && nl) e = cudaMemcpyAsync(cluster_of, d_of, nl * 4, cudaMemcpyDeviceToHost, s);
+    }
+    if (!device_out) {
+      if (d_out) cudaFreeAsync(d_out, s);
+      if (d_cells) cudaFreeAsync(d_cells, s);
+      if (e == cudaSuccess) e = cudaStreamSynchronize(s);
+    }
+    CUDA_TRY(e);
+  }
+  CUDA_TRY(cudaGetLastError());
+  *n_out = (size_t)counts[0];
+  if (n_cells_out) *n_cells_out = (size_t)counts[1];
+  return MLM_OK;
+}
+
+int mlm_frontier_clusters(mlm_handle h, const double box_min[3], const double box_max[3], int32_t min_cells, int flags,
+                          mlm_frontier_cluster *out, size_t cap, size_t *n_out, int32_t *cells3, int32_t *cluster_of,
+                          size_t cell_cap, size_t *n_cells_out) {
+  return frontier_clusters(h, box_min, box_max, min_cells, flags, out, cap, n_out, cells3, cluster_of, cell_cap,
+                           n_cells_out, false);
+}
+int mlm_frontier_clusters_device(mlm_handle h, const double box_min[3], const double box_max[3], int32_t min_cells,
+                                 int flags, mlm_frontier_cluster *d_out, size_t cap, size_t *n_out, int32_t *d_cells3,
+                                 int32_t *d_cluster_of, size_t cell_cap, size_t *n_cells_out) {
+  return frontier_clusters(h, box_min, box_max, min_cells, flags, d_out, cap, n_out, d_cells3, d_cluster_of, cell_cap,
+                           n_cells_out, true);
 }
 
 // ---- stream control ----------------------------------------------------------------------------------

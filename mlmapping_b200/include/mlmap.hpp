@@ -204,6 +204,30 @@ class mlmap {
     check(mlm_esdf_distance(h_, n ? pos->v : nullptr, n, dist, grad ? grad->v : nullptr), "mlm_esdf_distance");
   }
 
+  // frontier clustering (no reference counterpart; spec at mlm_frontier_clusters): the clusters with >= min_cells cells
+  // sorted by key (z, y, x); box_min / box_max both null for the whole map; cells3 / cluster_of (optional) receive every
+  // cell of a kept cluster with its cluster index
+  std::vector<mlm_frontier_cluster> frontierClusters(const Vec3 *box_min = nullptr, const Vec3 *box_max = nullptr,
+                                                     int min_cells = 1, bool conn6 = false,
+                                                     std::vector<int32_t> *cells3 = nullptr,
+                                                     std::vector<int32_t> *cluster_of = nullptr) {
+    const double *a = box_min ? box_min->v : nullptr, *b = box_max ? box_max->v : nullptr;
+    const int flags = conn6 ? MLM_FRONTIER_CONN6 : 0;
+    size_t n = 0, m = 0;
+    check(mlm_frontier_clusters(h_, a, b, min_cells, flags, nullptr, 0, &n, nullptr, nullptr, 0, &m),
+          "mlm_frontier_clusters");
+    std::vector<mlm_frontier_cluster> out(n);
+    const bool lab = cells3 && cluster_of;
+    if (lab) {
+      cells3->resize(3 * m);
+      cluster_of->resize(m);
+    }
+    check(mlm_frontier_clusters(h_, a, b, min_cells, flags, out.data(), n, &n, lab ? cells3->data() : nullptr,
+                                lab ? cluster_of->data() : nullptr, lab ? m : 0, &m),
+          "mlm_frontier_clusters");
+    return out;
+  }
+
   // map clouds for consumers: what rviz_vis::pub_global_local_map / pub_frontier put on the wire
   // (src/rviz_vis.cpp:267-327) and mlmap::visualize_odds' slice (src/mlmap.cpp:200-284), compacted on the device.
   // Points are {x, y, z, w} floats, the layout of pcl::PointXYZ.
