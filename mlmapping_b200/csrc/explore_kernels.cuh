@@ -257,9 +257,11 @@ __global__ void __launch_bounds__(kColThreads, 1) k_frame_explore(MapParams P, D
     }
   }
   MLM_FRAME_WALL(1);
-  grid_barrier(D.grid_bar, G);
+  grid_arrive(D.grid_bar);
+  load_col_tables(P, s_raw);   // the projection is done with shared memory (the loop's last barrier)
+  grid_wait(D.grid_bar, G);
   MLM_FRAME_WALL(2);
-  column_phase(P, D, F, s_raw);
+  column_phase(P, D, F, s_raw, true);
   MLM_FRAME_WALL(3);
   grid_barrier(D.grid_bar, 2 * G);
   MLM_FRAME_WALL(4);

@@ -828,7 +828,10 @@ __host__ __device__ inline size_t col_smem_prefix_bytes(int col_words, int nRho,
 #define MLM_PHASE(i) do { __syncthreads(); if (threadIdx.x == 0) D.debug_cycles[vc * 16 + (i)] = clock64(); } while (0)
 #define MLM_PHASE_G(i, leader) do { if (threadIdx.x == (leader)) D.debug_cycles[vc * 16 + (i)] = clock64(); } while (0)
 #define MLM_WALL(i) do { if (threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); D.debug_cycles[vc * 16 + (i)] = (long long)t_; } } while (0)
+// per-CTA timeline of the fused frame (rows nCol + blockIdx.x of the debug buffer)
+#define MLM_FRAME_WALL(i) do { if (threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); D.debug_cycles[(P.nCol + blockIdx.x) * 16 + (i)] = (long long)t_; } } while (0)
 #else
+#define MLM_FRAME_WALL(i) do { } while (0)
 #define MLM_WALL(i) do { } while (0)
 #define MLM_PHASE(i) do { } while (0)
 #define MLM_PHASE_G(i, leader) do { } while (0)
@@ -1368,23 +1371,33 @@ __device__ __forceinline__ int column_weight(const DeviceBuffers &D, int vc) { r
 // Persistent kernel: one CTA per SM pulls work columns, heaviest first, from a queue every CTA derives
 // identically (stable counting sort of the per-column weights k_project accumulated), so a depth camera's
 // ~80 lit columns (160 halves) spread over all SMs instead of one SM per column.
-__device__ __forceinline__ void column_phase(const MapParams &P, DeviceBuffers &D, const FrameParams &F, unsigned char *s_raw) {
-  const int tid = threadIdx.x;
-  __shared__ int s_item, s_wmax, s_nactive;
-  // shared memory: [miss bitmap][end-cell bitmap][radix counters][warp sums][odds table][k_reach][record index map][queue order][keys A][keys B]
-  uint32_t *s_cnt = reinterpret_cast<uint32_t *>(s_raw) + 2 * P.col_words;
-  uint32_t *s_wsum = s_cnt + kCntTotal;
-  float *s_odds = reinterpret_cast<float *>(s_wsum + kColWarps);
+// The CTA's copies of the odds table and k_reach in shared memory (frame-independent).  The fused frames load them
+// while they wait at the barrier behind the projection, whose shared memory they overlap.
+__device__ __forceinline__ void load_col_tables(const MapParams &P, unsigned char *s_raw) {
+  float *s_odds = reinterpret_cast<float *>(s_raw) + 2 * P.col_words + kCntTotal + kColWarps;
   int *s_reach = reinterpret_cast<int *>(s_odds + kOddsRows * P.nRho);
-  uint16_t *s_order = reinterpret_cast<uint16_t *>(s_reach + P.nRho + kMapCap);
+  for (int i = threadIdx.x; i < kOddsRows * P.nRho; i += blockDim.x) s_odds[i] = __ldg(&P.odds_table[i]);
+  for (int i = threadIdx.x; i < P.nRho; i += blockDim.x) s_reach[i] = __ldg(&P.k_reach[i]);
+}
+
+__device__ __forceinline__ void column_phase(const MapParams &P, DeviceBuffers &D, const FrameParams &F, unsigned char *s_raw,
+                                             bool tables_loaded = false) {
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  __shared__ int s_item, s_wmax, s_nactive, s_nq;
+  __shared__ int s_mh[64];   // merge histogram (below)
+  // shared memory: [miss bitmap][end-cell bitmap][radix counters][warp sums][odds table][k_reach][record index map][queue order][keys A][keys B]
+  uint16_t *s_order = reinterpret_cast<uint16_t *>(reinterpret_cast<int *>(s_raw) + 2 * P.col_words + kCntTotal + kColWarps +
+                                                   kOddsRows * P.nRho + P.nRho + kMapCap);
   uint64_t *s_keys = reinterpret_cast<uint64_t *>(s_raw + col_smem_prefix_bytes(P.col_words, P.nRho, P.nCol));
-  for (int i = tid; i < kOddsRows * P.nRho; i += blockDim.x) s_odds[i] = __ldg(&P.odds_table[i]);
-  for (int i = tid; i < P.nRho; i += blockDim.x) s_reach[i] = __ldg(&P.k_reach[i]);
+  if (!tables_loaded) load_col_tables(P, s_raw);
+  if (tid < 64) s_mh[tid] = 0;
   if (tid == 0) {
     s_wmax = 0;
     s_nactive = 0;
+    s_nq = 0;
   }
   __syncthreads();
+  MLM_FRAME_WALL(13);  // tables loaded
   // per work column: records (0 = idle this frame or cast by another rank) and queue weight, loaded once
   int *s_nrec = reinterpret_cast<int *>(s_keys);          // [nCol]; the key buffers are idle until the first item
   int *s_wgt = s_nrec + P.nCol;
@@ -1408,78 +1421,83 @@ __device__ __forceinline__ void column_phase(const MapParams &P, DeviceBuffers &
     if (my_active) atomicAdd(&s_nactive, my_active);
   }
   __syncthreads();
+  MLM_FRAME_WALL(14);  // weights loaded (slots 13-15: the column prologue; 9-12 are k_frame_explore's)
   // More active halves than CTAs would mean another round of items, and even the lightest item costs ~15 us of
   // barrier-separated phases: work the lightest columns whole instead (both halves as ONE item), as many as it takes to
   // get down to one item per CTA.  The heavy columns stay split: the heaviest item bounds the phase.
   // s_nrec afterwards: > 0 half item, < 0 merged item (even slot, -records), kCovered odd slot of a merged column, 0 idle.
   constexpr int kCovered = (int)0x80000000;
   if (sorted && P.split && P.merge && s_nactive > (int)gridDim.x) {
-    __shared__ int s_mh[64];
-    __shared__ int s_T, s_sh2, s_need;
-    if (tid < 64) s_mh[tid] = 0;
-    if (tid == 0) {
-      int sh2 = 0;
-      while (((2 * s_wmax) >> sh2) > 63) sh2++;
-      s_sh2 = sh2;
-    }
-    __syncthreads();
-    const int sh2 = s_sh2;
+    __shared__ int s_T, s_need, s_below;
+    __shared__ int s_wc[32];
+    int sh2 = 0;
+    while (((2 * s_wmax) >> sh2) > 63) sh2++;
     for (int phi = tid; phi < P.nPhi; phi += blockDim.x)
       if (s_nrec[2 * phi] > 0 && s_nrec[2 * phi + 1] > 0) atomicAdd(&s_mh[(s_wgt[2 * phi] + s_wgt[2 * phi + 1]) >> sh2], 1);
     __syncthreads();
-    if (tid == 0) {
-      int c2 = 0;
-      for (int b = 0; b < 64; b++) c2 += s_mh[b];                       // columns with both halves active
+    if (warp == 0) {
+      // one warp over the 64 buckets (two per lane), prefix sums by shuffles
+      const int m0 = s_mh[2 * lane], m1 = s_mh[2 * lane + 1];
+      int cum = m0 + m1;
+#pragma unroll
+      for (int ofs = 1; ofs < 32; ofs <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, cum, ofs);
+        if (lane >= ofs) cum += t;
+      }
+      const int c2 = __shfl_sync(0xffffffffu, cum, 31);                 // columns with both halves active
       // Down to one item per CTA when that is possible, else every column whole: with more than one round the total work
       // decides, and a whole column costs less than its two halves.  Measured on CFG-C (360 lit columns, 148 CTAs): all
       // whole 175 us; a mix that fills the rounds exactly 193 us; whole except the columns 1.4x heavier than average
       // 199 us; all halves 210 us.  With 2 ranks (180 columns each): 120 / 135 / 123 us.
       const int need = min(c2, s_nactive - (int)gridDim.x);
-      int cum = 0, T = -1;
-      for (int b = 0; b < 64 && need > 0; b++) {
-        cum += s_mh[b];
-        if (cum >= need) {
-          T = b;
-          break;
-        }
+      // threshold bucket T: the first whose cumulative count reaches `need` (none when need <= 0)
+      const int cum0 = cum - m1;                                          // through bucket 2 * lane
+      const unsigned hit = __ballot_sync(0xffffffffu, need > 0 && cum >= need);
+      const int L = hit ? __ffs(hit) - 1 : 0;
+      const int cum0_L = __shfl_sync(0xffffffffu, cum0, L), m0_L = __shfl_sync(0xffffffffu, m0, L);
+      if (lane == 0) {
+        const bool first = cum0_L >= need;
+        s_T = hit ? (first ? 2 * L : 2 * L + 1) : -1;
+        s_below = hit ? (first ? cum0_L - m0_L : cum0_L) : 0;             // candidates in the buckets below T
+        s_need = need;
       }
-      s_T = T;
-      s_need = need;
     }
     __syncthreads();
-    const int need = s_need;
     // exactly `need` columns: every candidate below the threshold bucket, and of the threshold bucket itself the first
     // ones in column order (columns of a LiDAR scan weigh alike: a whole bucket would merge the heavy ones too, and the
-    // heaviest item bounds the phase)
-    int *s_rank = reinterpret_cast<int *>(s_keys + P.sort_cap_smem);   // second key buffer, idle until the queue sort
-    int below = 0;
-    for (int b = 0; b < s_T; b++) below += s_mh[b];
-    const int take = need - below;                                        // how many of bucket s_T to merge (s_T < 0: none at all)
-    for (int phi = tid; phi < P.nPhi; phi += blockDim.x) {
-      const int n0 = s_nrec[2 * phi], n1 = s_nrec[2 * phi + 1];
-      s_rank[phi] = (n0 > 0 && n1 > 0 && ((s_wgt[2 * phi] + s_wgt[2 * phi + 1]) >> sh2) == s_T) ? 1 : 0;
-    }
-    __syncthreads();
-    __shared__ int s_scan_warp[33];
-    block_exclusive_scan(s_rank, P.nPhi, s_scan_warp);
-    int merged_here = 0;
-    for (int phi = tid; phi < P.nPhi; phi += blockDim.x) {
-      const int n0 = s_nrec[2 * phi], n1 = s_nrec[2 * phi + 1];
-      if (n0 > 0 && n1 > 0) {
-        const int w = s_wgt[2 * phi] + s_wgt[2 * phi + 1];
-        const int bkt = w >> sh2;
-        if (bkt < s_T || (bkt == s_T && s_rank[phi] < take)) {
-          s_wgt[2 * phi] = w;
-          s_nrec[2 * phi] = -(n0 + n1);
-          s_nrec[2 * phi + 1] = kCovered;
-          merged_here++;
-          atomicMax(&s_wmax, w);
-        }
+    // heaviest item bounds the phase).  Rank in column order: ballots inside a warp, per-warp counts across warps.
+    const int T = s_T;
+    const int take = s_need - s_below;                                    // how many of bucket T to merge (T < 0: none at all)
+    int merged_here = 0, run = 0;
+    for (int base = 0; base < P.nPhi; base += blockDim.x) {
+      const int phi = base + tid;
+      const bool both = phi < P.nPhi && s_nrec[2 * phi] > 0 && s_nrec[2 * phi + 1] > 0;
+      const int w = both ? s_wgt[2 * phi] + s_wgt[2 * phi + 1] : 0;
+      const int bkt = w >> sh2;
+      const unsigned at_t = __ballot_sync(0xffffffffu, both && bkt == T);
+      if (lane == 0) s_wc[warp] = __popc(at_t);
+      __syncthreads();
+      int wsum = lane < (int)(blockDim.x >> 5) ? s_wc[lane] : 0;          // inclusive scan of the warp counts
+#pragma unroll
+      for (int ofs = 1; ofs < 32; ofs <<= 1) {
+        const int t = __shfl_up_sync(0xffffffffu, wsum, ofs);
+        if (lane >= ofs) wsum += t;
       }
+      const int rank = run + (warp ? __shfl_sync(0xffffffffu, wsum, warp - 1) : 0) + __popc(at_t & ((1u << lane) - 1));
+      run += __shfl_sync(0xffffffffu, wsum, 31);
+      if (both && (bkt < T || (bkt == T && rank < take))) {
+        s_wgt[2 * phi] = w;
+        s_nrec[2 * phi] = -(s_nrec[2 * phi] + s_nrec[2 * phi + 1]);
+        s_nrec[2 * phi + 1] = kCovered;
+        merged_here++;
+        atomicMax(&s_wmax, w);
+      }
+      __syncthreads();                                                    // s_wc is rewritten by the next chunk
     }
     if (merged_here) atomicSub(&s_nactive, merged_here);
     __syncthreads();
   }
+  MLM_FRAME_WALL(15);  // merge done
   auto is_active = [&](int vc) { return sorted ? s_nrec[vc] != 0 : (D.phi_hist[vc] > 0 && !not_mine(vc)); };
   // idle work columns: their own rows of the miss bitmap are empty this frame (spread over the CTAs)
   for (int vc = blockIdx.x; vc < P.nCol; vc += gridDim.x) {
@@ -1496,26 +1514,32 @@ __device__ __forceinline__ void column_phase(const MapParams &P, DeviceBuffers &
     n_active = s_nactive;
     int sh = 0;
     while ((s_wmax >> sh) > 63) sh++;
-    uint64_t *q_src = s_keys + P.sort_cap_smem;           // second key buffer: sort input; output lands in the first
-    uint64_t kq[8];
-    int nk = 0;
-    for (int vc = tid; vc < P.nCol && nk < 8; vc += blockDim.x) {
+    // one distinct 32-bit key per item, (63 - bucket, column, merged): its rank among the items' keys is its queue position
+    // (by bucket, then column).  The items are few (about one per CTA), so counting the smaller keys costs less than a
+    // radix pass over every column with its block-wide barriers.
+    uint32_t *q_key = reinterpret_cast<uint32_t *>(s_keys + P.sort_cap_smem);   // second key buffer (16-byte aligned)
+    for (int vc = tid; vc < P.nCol; vc += blockDim.x) {
       const int nr = s_nrec[vc];
-      const bool item = nr != 0 && nr != kCovered;
-      kq[nk++] = ((item ? (uint64_t)(63 - (s_wgt[vc] >> sh)) : 64ull) << 16) | (uint64_t)(nr < 0 ? P.nCol + (vc >> 1) : vc);
+      if (nr != 0 && nr != kCovered)
+        q_key[agg_inc(&s_nq)] = ((uint32_t)(63 - (s_wgt[vc] >> sh)) << 24) | ((uint32_t)vc << 1) | (nr < 0 ? 1u : 0u);
     }
-    __syncthreads();                                        // s_nrec / s_wgt are dead from here on
-    nk = 0;
-    for (int vc = tid; vc < P.nCol && nk < 8; vc += blockDim.x) q_src[vc] = kq[nk++];
+    if (tid < 3) q_key[n_active + tid] = 0xffffffffu;      // pad to whole uint4s (never smaller than a key)
     __syncthreads();
-    radix_pass(q_src, s_keys, P.nCol, 16, 7, s_cnt, s_wsum);
-    for (int i = tid; i < n_active; i += blockDim.x) s_order[i] = (uint16_t)(s_keys[i] & 0xffffu);
+    const uint4 *q4 = reinterpret_cast<const uint4 *>(q_key);
+    for (int i = tid; i < n_active; i += blockDim.x) {
+      const uint32_t k = q_key[i];
+      int rank = 0;
+      for (int j = 0; j < (n_active + 3) >> 2; j++) {
+        const uint4 q = q4[j];
+        rank += (q.x < k) + (q.y < k) + (q.z < k) + (q.w < k);
+      }
+      const int vc = (int)((k >> 1) & 0x7fffffu);
+      s_order[rank] = (uint16_t)((k & 1u) ? P.nCol + (vc >> 1) : vc);
+    }
   } else {
     n_active = P.nCol;  // more work columns than the sort scratch holds: plain column order, idle ones skipped below
   }
-#ifdef MLM_PHASE_TIMING
-  if (threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); D.debug_cycles[(P.nCol + blockIdx.x) * 16 + 7] = (long long)t_; }
-#endif
+  MLM_FRAME_WALL(7);  // queue ready
   bool first_round = true;
   for (;;) {
     __syncthreads();  // the previous item is done with shared memory; s_order is in place
@@ -1803,9 +1827,7 @@ __device__ __forceinline__ void frame_finish(const MapParams &P, DeviceBuffers &
     __shared__ int s_is_last;
     __threadfence();
     __syncthreads();
-#ifdef MLM_PHASE_TIMING
-    if (threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); D.debug_cycles[(P.nCol + blockIdx.x) * 16 + 8] = (long long)t_; }
-#endif
+    MLM_FRAME_WALL(8);
     if (threadIdx.x == 0) s_is_last = atomicAdd(D.fuse_ticket, 1) == (int)gridDim.x - 1;
     __syncthreads();
     if (s_is_last && threadIdx.x < 32) {
@@ -1867,11 +1889,16 @@ __global__ void __launch_bounds__(256) k_fuse(MapParams P, DeviceBuffers D, Fram
 // boundaries (each boundary costs a drain, a launch and a ramp-up that together outweigh the phase's own
 // tail on a ~70 us frame).  The barrier is a monotone counter in global memory: arrive with a release
 // add, spin on an acquire load; the last CTA through k_fuse's completion ticket rearms it.
-__device__ __forceinline__ void grid_barrier(int *counter, int target) {
+// Split in arrive / wait so that a CTA can do work that does not depend on the other CTAs in between.
+__device__ __forceinline__ void grid_arrive(int *counter) {
   __syncthreads();
   if (threadIdx.x == 0) {
     __threadfence();
     atomicAdd(counter, 1);
+  }
+}
+__device__ __forceinline__ void grid_wait(int *counter, int target) {
+  if (threadIdx.x == 0) {
     int v;
     do {
       asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(counter) : "memory");
@@ -1880,12 +1907,11 @@ __device__ __forceinline__ void grid_barrier(int *counter, int target) {
   }
   __syncthreads();
 }
+__device__ __forceinline__ void grid_barrier(int *counter, int target) {
+  grid_arrive(counter);
+  grid_wait(counter, target);
+}
 
-#ifdef MLM_PHASE_TIMING
-#define MLM_FRAME_WALL(i) do { if (threadIdx.x == 0) { unsigned long long t_; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t_)); D.debug_cycles[(P.nCol + blockIdx.x) * 16 + (i)] = (long long)t_; } } while (0)
-#else
-#define MLM_FRAME_WALL(i) do { } while (0)
-#endif
 template <int kMode>
 __global__ void __launch_bounds__(kColThreads, 1) k_frame(MapParams P, DeviceBuffers D, FrameParams F) {
   extern __shared__ __align__(16) unsigned char s_raw[];
@@ -1900,10 +1926,12 @@ __global__ void __launch_bounds__(kColThreads, 1) k_frame(MapParams P, DeviceBuf
     }
   }
   MLM_FRAME_WALL(1);
-  grid_barrier(D.grid_bar, G);
+  grid_arrive(D.grid_bar);
+  load_col_tables(P, s_raw);   // the projection is done with shared memory (the loop's last barrier)
+  grid_wait(D.grid_bar, G);
   MLM_FRAME_WALL(2);
   // (2) work columns (awareness update + staging into the frame-local voxel grid)
-  column_phase(P, D, F, s_raw);
+  column_phase(P, D, F, s_raw, true);
   MLM_FRAME_WALL(3);
   grid_barrier(D.grid_bar, 2 * G);
   MLM_FRAME_WALL(4);

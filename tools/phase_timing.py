@@ -51,6 +51,9 @@ if len(fa):
     names = ["start", "proj done", "bar1 out", "cols done", "bar2 out", "bar3 out", "end", "col prologue", "fuse ticket"]
     for i, n in enumerate(names):
         print(f"k_frame {n:10s}: min {rel[:, i].min():6.1f}  mean {rel[:, i].mean():6.1f}  max {rel[:, i].max():6.1f} us")
+    # column prologue (bar1 out -> queue ready): odds / k_reach tables, per-column weights, merge of light columns, queue sort
+    pro = np.stack([fa[:, 13] - fa[:, 2], fa[:, 14] - fa[:, 13], fa[:, 15] - fa[:, 14], fa[:, 7] - fa[:, 15]], axis=1) / 1e3
+    print("col prologue us [tables, weights, merge, queue sort]: mean", pro.mean(0).round(2), "max", pro.max(0).round(2))
     ids = np.nonzero(fr[:, 0] > 0)[0]
     o = np.argsort(-rel[:, 8])
     print("fuse ticket times, slowest 12 (cta, bar2 out, ticket):", [(int(ids[i]), round(float(rel[i, 4]), 1), round(float(rel[i, 8]), 1)) for i in o[:12]])
