@@ -15,6 +15,7 @@
 #include <cmath>
 #include <chrono>
 #include <string>
+#include <utility>
 #include <vector>
 
 #include "../../include/mlmap_b200.h"
@@ -33,14 +34,62 @@ namespace {
 
 thread_local std::string g_last_error;
 
+// also clears the failure from the thread's last error, so that a later call's cudaGetLastError() does not report it
 #define CUDA_TRY(expr)                                                                        \
   do {                                                                                        \
     cudaError_t _e = (expr);                                                                  \
     if (_e != cudaSuccess) {                                                                  \
+      cudaGetLastError();                                                                     \
       g_last_error = std::string(#expr) + ": " + cudaGetErrorString(_e);                      \
       return MLM_ERR_CUDA;                                                                    \
     }                                                                                         \
   } while (0)
+
+// A temporary of a host-pointer entry point: one stream-ordered allocation, released on its stream when the owner goes
+// out of scope (or by reset()), so that an error return gives it back to the pool as the success path does.
+template <typename T>
+class StreamTemp {
+ public:
+  explicit StreamTemp(cudaStream_t s) : s_(s) {}
+  StreamTemp(StreamTemp &&o) noexcept : p_(o.p_), s_(o.s_) { o.p_ = nullptr; }
+  ~StreamTemp() { reset(); }
+  cudaError_t alloc(size_t count) {
+    reset();
+    const cudaError_t e = cudaMallocAsync((void **)&p_, count * sizeof(T), s_);
+    if (e != cudaSuccess) p_ = nullptr;
+    return e;
+  }
+  void reset() {
+    if (p_) cudaFreeAsync(p_, s_);
+    p_ = nullptr;
+  }
+  operator T *() const { return p_; }
+
+ private:
+  T *p_ = nullptr;
+  cudaStream_t s_;
+};
+
+// Scratch that a handle keeps and grows: (buffer, bytes) pairs, allocated all together or not at all.
+using ScratchList = std::vector<std::pair<void **, size_t>>;
+void scratch_free(const ScratchList &bufs) {
+  for (const auto &b : bufs) {
+    if (*b.first) cudaFree(*b.first);
+    *b.first = nullptr;
+  }
+}
+int scratch_alloc(const ScratchList &bufs, const char *what) {
+  for (const auto &b : bufs) {
+    const cudaError_t e = cudaMalloc(b.first, b.second);
+    if (e == cudaSuccess) continue;
+    *b.first = nullptr;
+    scratch_free(bufs);
+    cudaGetLastError();
+    g_last_error = std::string(what) + ": " + cudaGetErrorString(e);
+    return MLM_ERR_CUDA;
+  }
+  return MLM_OK;
+}
 
 // ---- Sophus/Eigen subset on the host (reference 3rdPartLib/Sophus/sophus/so3.cpp:42-90, se3.cpp:59-95)
 struct HQuat {
@@ -935,24 +984,22 @@ int ensure_input(mlm_map *h, size_t bytes, size_t capacity = 0) {
   return MLM_OK;
 }
 
-}  // namespace
-
-namespace {
-template <typename OutT, typename Launch>
-int host_query(mlm_handle h, const double *pos, size_t n, OutT *out, size_t out_per, Launch launch) {
+// host variant of a point query: the device variant's launch, with points and results staged through temporaries
+template <typename OutT, typename... Args>
+int host_query(mlm_handle h, const double *pos, size_t n, OutT *out, size_t out_per,
+               void (*launch)(mlm_handle, const double *, size_t, OutT *, Args...), Args... args) {
   if (!h || (!pos && n) || (!out && n)) return MLM_ERR_INVALID_ARG;
   if (n == 0) return MLM_OK;
   CUDA_TRY(cudaSetDevice(h->device));
-  double *d_pos = nullptr;
-  OutT *d_out = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_pos, n * 24, h->stream));
-  CUDA_TRY(cudaMallocAsync((void **)&d_out, n * out_per * sizeof(OutT), h->stream));
-  CUDA_TRY(cudaMemcpyAsync(d_pos, pos, n * 24, cudaMemcpyHostToDevice, h->stream));
-  launch(d_pos, d_out);
-  h->launches++;
-  CUDA_TRY(cudaMemcpyAsync(out, d_out, n * out_per * sizeof(OutT), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_TRY(cudaFreeAsync(d_pos, h->stream));
-  CUDA_TRY(cudaFreeAsync(d_out, h->stream));
+  {
+    StreamTemp<double> d_pos(h->stream);
+    StreamTemp<OutT> d_out(h->stream);
+    CUDA_TRY(d_pos.alloc(n * 3));
+    CUDA_TRY(d_out.alloc(n * out_per));
+    CUDA_TRY(cudaMemcpyAsync(d_pos, pos, n * 24, cudaMemcpyHostToDevice, h->stream));
+    launch(h, d_pos, n, d_out, args...);
+    CUDA_TRY(cudaMemcpyAsync(out, d_out, n * out_per * sizeof(OutT), cudaMemcpyDeviceToHost, h->stream));
+  }
   CUDA_TRY(cudaStreamSynchronize(h->stream));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
@@ -1441,7 +1488,8 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   return MLM_OK;
 }
 
-static void frontier_free(mlm_handle h, bool all);
+static void esdf_free(mlm_handle h);
+static void frontier_free(mlm_handle h);
 
 int mlm_destroy(mlm_handle h) {
   if (!h) return MLM_ERR_INVALID_ARG;
@@ -1456,9 +1504,8 @@ int mlm_destroy(mlm_handle h) {
   mlm_shard_close(h);
   if (h->h_shard_state) cudaFreeHost(h->h_shard_state);
   for (void *p : h->allocs) cudaFree(p);
-  for (void *p : {(void *)h->esdf_blk, (void *)h->esdf_a, (void *)h->esdf_b, (void *)h->esdf_stk})
-    if (p) cudaFree(p);
-  frontier_free(h, true);
+  esdf_free(h);
+  frontier_free(h);
   if (h->d_input) cudaFree(h->d_input);
   if (h->h_stage) cudaFreeHost(h->h_stage);
   if (h->l2_buf) cudaFree(h->l2_buf);
@@ -1692,12 +1739,15 @@ int mlm_frame_finish(mlm_handle h, mlm_frame_stats *stats) {
 }
 
 // getOdd(const Vec3I &glb_id, size_t subbox_id), include/mlmap.h:128,227-235
+static void odd_at_launch(mlm_handle h, const int32_t *d_glb3, const int32_t *d_sub, size_t n, float *d_out) {
+  k_get_odd_at<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_glb3, d_sub, n, d_out);
+  h->launches++;
+}
 int mlm_get_odd_at_device(mlm_handle h, const int32_t *d_glb3, const int32_t *d_sub, size_t n, float *d_out) {
   if (!h || ((!d_glb3 || !d_sub || !d_out) && n)) return MLM_ERR_INVALID_ARG;
   CUDA_TRY(cudaSetDevice(h->device));
   if (n == 0) return MLM_OK;
-  k_get_odd_at<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_glb3, d_sub, n, d_out);
-  h->launches++;
+  odd_at_launch(h, d_glb3, d_sub, n, d_out);
   return MLM_OK;
 }
 int mlm_get_odd_at(mlm_handle h, const int32_t *glb3, const int32_t *sub, size_t n, float *out) {
@@ -1705,23 +1755,17 @@ int mlm_get_odd_at(mlm_handle h, const int32_t *glb3, const int32_t *sub, size_t
   if (n == 0) return MLM_OK;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
-  int32_t *d_g = nullptr, *d_s = nullptr;
-  float *d_o = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_g, n * 12, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_s, n * 4, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_o, n * 4, s));
-  cudaError_t e = cudaMemcpyAsync(d_g, glb3, n * 12, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d_s, sub, n * 4, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) {
-    k_get_odd_at<<<grid_for(n, 256), 256, 0, s>>>(h->P, h->D, d_g, d_s, n, d_o);
-    h->launches++;
-    e = cudaMemcpyAsync(out, d_o, n * 4, cudaMemcpyDeviceToHost, s);
+  {
+    StreamTemp<int32_t> d_in(s);  // glb3, sub
+    StreamTemp<float> d_o(s);
+    CUDA_TRY(d_in.alloc(n * 4));
+    CUDA_TRY(d_o.alloc(n));
+    CUDA_TRY(cudaMemcpyAsync(d_in, glb3, n * 12, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(d_in + 3 * n, sub, n * 4, cudaMemcpyHostToDevice, s));
+    odd_at_launch(h, d_in, d_in + 3 * n, n, d_o);
+    CUDA_TRY(cudaMemcpyAsync(out, d_o, n * 4, cudaMemcpyDeviceToHost, s));
   }
-  cudaFreeAsync(d_g, s);
-  cudaFreeAsync(d_s, s);
-  cudaFreeAsync(d_o, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  CUDA_TRY(e);
+  CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
 }
@@ -1740,17 +1784,18 @@ int mlm_set_free_in_bound(mlm_handle h, const double box_min[3], const double bo
   }
   size_t total = ax[0].size() * ax[1].size() * ax[2].size();
   size_t ncoord = ax[0].size() + ax[1].size() + ax[2].size();
-  double *d_c = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_c, ncoord * sizeof(double), h->stream));
   std::vector<double> flat;
   flat.reserve(ncoord);
   for (int a = 0; a < 3; a++) flat.insert(flat.end(), ax[a].begin(), ax[a].end());
-  CUDA_TRY(cudaMemcpyAsync(d_c, flat.data(), ncoord * sizeof(double), cudaMemcpyHostToDevice, h->stream));
-  k_set_free<<<grid_for(total, 256), 256, 0, h->stream>>>(h->P, h->D, d_c, (int)ax[0].size(), d_c + ax[0].size(),
-                                                           (int)ax[1].size(), d_c + ax[0].size() + ax[1].size(),
-                                                           (int)ax[2].size());
-  h->launches++;
-  CUDA_TRY(cudaFreeAsync(d_c, h->stream));
+  {
+    StreamTemp<double> d_c(h->stream);
+    CUDA_TRY(d_c.alloc(ncoord));
+    CUDA_TRY(cudaMemcpyAsync(d_c, flat.data(), ncoord * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+    k_set_free<<<grid_for(total, 256), 256, 0, h->stream>>>(h->P, h->D, d_c, (int)ax[0].size(), d_c + ax[0].size(),
+                                                             (int)ax[1].size(), d_c + ax[0].size() + ax[1].size(),
+                                                             (int)ax[2].size());
+    h->launches++;
+  }
   CUDA_TRY(cudaStreamSynchronize(h->stream));  // flat must outlive the copy
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
@@ -1769,18 +1814,18 @@ int mlm_inflate_map(mlm_handle h, const double ct_pos[3]) {
   A.height = h->cfg.inflate_height;
   const int W = 2 * A.N + 1, nwin = W * W * W;
   cudaStream_t s = h->stream;
-  int *d_win = nullptr, *d_cnt = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_win, (size_t)nwin * sizeof(int), s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_cnt, 2 * sizeof(int), s));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int), s));
-  k_inflate_reset<<<nwin, 256, 0, s>>>(P, h->D, A, d_win);
-  k_inflate_sources<false><<<nwin, 256, 0, s>>>(P, h->D, A, d_win, d_cnt);
-  k_inflate_sources<true><<<nwin, 256, 0, s>>>(P, h->D, A, d_win, d_cnt);
-  h->launches += 3;
   int cnt[2] = {0, 0};
-  CUDA_TRY(cudaMemcpyAsync(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaFreeAsync(d_win, s));
-  CUDA_TRY(cudaFreeAsync(d_cnt, s));
+  {
+    StreamTemp<int> d_win(s), d_cnt(s);
+    CUDA_TRY(d_win.alloc(nwin));
+    CUDA_TRY(d_cnt.alloc(2));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int), s));
+    k_inflate_reset<<<nwin, 256, 0, s>>>(P, h->D, A, d_win);
+    k_inflate_sources<false><<<nwin, 256, 0, s>>>(P, h->D, A, d_win, d_cnt);
+    k_inflate_sources<true><<<nwin, 256, 0, s>>>(P, h->D, A, d_win, d_cnt);
+    h->launches += 3;
+    CUDA_TRY(cudaMemcpyAsync(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
+  }
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   h->cum_ram_expand += cnt[0];  // allocate_ram from inflate_atpos also counts (include/map_local.h:223)
@@ -1792,53 +1837,79 @@ int mlm_inflate_map(mlm_handle h, const double ct_pos[3]) {
   return MLM_OK;
 }
 
+// point queries: one launch each, called on the caller's buffers by the _device variants and through host_query
+static void occupancy_launch(mlm_handle h, const double *d_pos, size_t n, int32_t *d_out) {
+  k_get_occupancy<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, d_out);
+  h->launches++;
+}
+static void occupancy_inflate_launch(mlm_handle h, const double *d_pos, size_t n, int32_t *d_out, float inflate) {
+  k_get_occupancy_inflate<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, inflate, d_out);
+  h->launches++;
+}
+static void inflate_occupancy_launch(mlm_handle h, const double *d_pos, size_t n, int32_t *d_out) {
+  k_get_inflate_occupancy<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, d_out);
+  h->launches++;
+}
+static void odd_launch(mlm_handle h, const double *d_pos, size_t n, float *d_out) {
+  k_get_odd<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, d_out);
+  h->launches++;
+}
+static void odd_grad_launch(mlm_handle h, const double *d_pos, size_t n, double *d_out3n, size_t max_iter) {
+  k_get_odd_grad<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, (int)max_iter, d_out3n);
+  h->launches++;
+}
 int mlm_get_occupancy(mlm_handle h, const double *pos, size_t n, int32_t *out) {
-  return host_query<int32_t>(h, pos, n, out, 1, [&](double *dp, int32_t *dout) {
-    k_get_occupancy<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, dp, n, dout);
-  });
+  return host_query(h, pos, n, out, 1, occupancy_launch);
 }
 int mlm_get_occupancy_inflate(mlm_handle h, const double *pos, size_t n, float inflate, int32_t *out) {
-  return host_query<int32_t>(h, pos, n, out, 1, [&](double *dp, int32_t *dout) {
-    k_get_occupancy_inflate<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, dp, n, inflate, dout);
-  });
+  return host_query(h, pos, n, out, 1, occupancy_inflate_launch, inflate);
 }
 int mlm_get_inflate_occupancy(mlm_handle h, const double *pos, size_t n, int32_t *out) {
-  return host_query<int32_t>(h, pos, n, out, 1, [&](double *dp, int32_t *dout) {
-    k_get_inflate_occupancy<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, dp, n, dout);
-  });
+  return host_query(h, pos, n, out, 1, inflate_occupancy_launch);
 }
 int mlm_get_odd(mlm_handle h, const double *pos, size_t n, float *out) {
-  return host_query<float>(h, pos, n, out, 1, [&](double *dp, float *dout) {
-    k_get_odd<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, dp, n, dout);
-  });
+  return host_query(h, pos, n, out, 1, odd_launch);
 }
 int mlm_get_odd_grad(mlm_handle h, const double *pos, size_t n, size_t max_iter, double *out3n) {
-  return host_query<double>(h, pos, n, out3n, 3, [&](double *dp, double *dout) {
-    k_get_odd_grad<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, dp, n, (int)max_iter, dout);
-  });
+  return host_query(h, pos, n, out3n, 3, odd_grad_launch, max_iter);
 }
 int mlm_get_occupancy_device(mlm_handle h, const double *d_pos, size_t n, int32_t *d_out) {
   if (!h || (!d_pos && n) || (!d_out && n)) return MLM_ERR_INVALID_ARG;
   CUDA_TRY(cudaSetDevice(h->device));
   if (n == 0) return MLM_OK;
-  k_get_occupancy<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, d_out);
-  h->launches++;
+  occupancy_launch(h, d_pos, n, d_out);
   return MLM_OK;
 }
 int mlm_get_odd_device(mlm_handle h, const double *d_pos, size_t n, float *d_out) {
   if (!h || (!d_pos && n) || (!d_out && n)) return MLM_ERR_INVALID_ARG;
   CUDA_TRY(cudaSetDevice(h->device));
   if (n == 0) return MLM_OK;
-  k_get_odd<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, d_out);
-  h->launches++;
+  odd_launch(h, d_pos, n, d_out);
   return MLM_OK;
 }
 int mlm_get_odd_grad_device(mlm_handle h, const double *d_pos, size_t n, size_t max_iter, double *d_out3n) {
   if (!h || (!d_pos && n) || (!d_out3n && n)) return MLM_ERR_INVALID_ARG;
   CUDA_TRY(cudaSetDevice(h->device));
   if (n == 0) return MLM_OK;
-  k_get_odd_grad<<<grid_for(n, 256), 256, 0, h->stream>>>(h->P, h->D, d_pos, n, (int)max_iter, d_out3n);
-  h->launches++;
+  odd_grad_launch(h, d_pos, n, d_out3n, max_iter);
+  return MLM_OK;
+}
+
+// rays, the distance field and frontier clustering read the whole map
+static int refuse_sharded(mlm_handle h, const char *fn) {
+  if (h->shard_world <= 1) return MLM_OK;
+  g_last_error = std::string(fn) + ": a rank of a sharded map holds only the subboxes it owns";
+  return MLM_ERR_UNSUPPORTED;
+}
+// rule 1 of the ray spec along one axis of a box: cells floor(p / d_sub) of the IEEE quotient, |p / d_sub| < 2^30
+static int box_axis_cells(mlm_handle h, double a, double b, const char *fn, int *lo, int *hi) {
+  const double qa = a / h->P.d_sub, qb = b / h->P.d_sub;
+  if (!(std::fabs(qa) < 1073741824.0) || !(std::fabs(qb) < 1073741824.0) || !(a <= b)) {
+    g_last_error = std::string(fn) + ": a box corner is not finite, |p / d_sub| >= 2^30, or box_min > box_max";
+    return MLM_ERR_INVALID_ARG;
+  }
+  *lo = (int)std::floor(qa);
+  *hi = (int)std::floor(qb);
   return MLM_OK;
 }
 
@@ -1848,11 +1919,7 @@ static_assert(sizeof(mlm_ray_hit) == sizeof(RayHit), "mlm_ray_hit / RayHit layou
 
 static int cast_rays_check(mlm_handle h, const void *from, const void *to, size_t n, int flags, const void *out) {
   if (!h || ((!from || !to || !out) && n) || (flags != 0 && flags != MLM_RAY_INFLATED)) return MLM_ERR_INVALID_ARG;
-  if (h->shard_world > 1) {
-    g_last_error = "mlm_cast_rays: a rank of a sharded map holds only the subboxes it owns";
-    return MLM_ERR_UNSUPPORTED;
-  }
-  return MLM_OK;
+  return refuse_sharded(h, "mlm_cast_rays");
 }
 static void cast_rays_launch(mlm_handle h, const double *d_from, const double *d_to, size_t n, int flags, mlm_ray_hit *d_out) {
   RayHit *o = reinterpret_cast<RayHit *>(d_out);
@@ -1875,33 +1942,25 @@ int mlm_cast_rays(mlm_handle h, const double *from, const double *to, size_t n, 
   if (n == 0) return MLM_OK;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
-  double *d_ft = nullptr;
-  mlm_ray_hit *d_o = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_ft, n * 48, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_o, n * sizeof(mlm_ray_hit), s));
-  cudaError_t e = cudaMemcpyAsync(d_ft, from, n * 24, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) e = cudaMemcpyAsync(d_ft + 3 * n, to, n * 24, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) {
+  {
+    StreamTemp<double> d_ft(s);  // from, to
+    StreamTemp<mlm_ray_hit> d_o(s);
+    CUDA_TRY(d_ft.alloc(n * 6));
+    CUDA_TRY(d_o.alloc(n));
+    CUDA_TRY(cudaMemcpyAsync(d_ft, from, n * 24, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(d_ft + 3 * n, to, n * 24, cudaMemcpyHostToDevice, s));
     cast_rays_launch(h, d_ft, d_ft + 3 * n, n, flags, d_o);
-    e = cudaMemcpyAsync(out, d_o, n * sizeof(mlm_ray_hit), cudaMemcpyDeviceToHost, s);
+    CUDA_TRY(cudaMemcpyAsync(out, d_o, n * sizeof(mlm_ray_hit), cudaMemcpyDeviceToHost, s));
   }
-  cudaFreeAsync(d_ft, s);
-  cudaFreeAsync(d_o, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  CUDA_TRY(e);
+  CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
 }
 
 // ---- signed distance field (esdf_kernels.cuh) ------------------------------------------------------------------
-static int esdf_refuse_sharded(mlm_handle h, const char *fn) {
-  if (h->shard_world <= 1) return MLM_OK;
-  g_last_error = std::string(fn) + ": a rank of a sharded map holds only the subboxes it owns";
-  return MLM_ERR_UNSUPPORTED;
-}
 // a field is there to query / export
 static int esdf_ready(mlm_handle h, const char *fn) {
-  const int rc = esdf_refuse_sharded(h, fn);
+  const int rc = refuse_sharded(h, fn);
   if (rc != MLM_OK) return rc;
   if (!h->esdf_built) {
     g_last_error = std::string(fn) + ": no signed distance field has been built (mlm_esdf_build first)";
@@ -1909,11 +1968,13 @@ static int esdf_ready(mlm_handle h, const char *fn) {
   }
   return MLM_OK;
 }
+// the grid buffers for c cells: blocking bytes, two int2 grids (the first ends as the values), two stacks
+static ScratchList esdf_scratch(mlm_handle h, size_t c) {
+  return {{(void **)&h->esdf_blk, c}, {(void **)&h->esdf_a, c * sizeof(int2)}, {(void **)&h->esdf_b, c * sizeof(int2)},
+          {(void **)&h->esdf_stk, 2 * c * sizeof(int2)}};
+}
 static void esdf_free(mlm_handle h) {
-  for (void *p : {(void *)h->esdf_blk, (void *)h->esdf_a, (void *)h->esdf_b, (void *)h->esdf_stk})
-    if (p) cudaFree(p);
-  h->esdf_blk = nullptr;
-  h->esdf_a = h->esdf_b = h->esdf_stk = nullptr;
+  scratch_free(esdf_scratch(h, 0));
   h->esdf_cap = 0;
   h->esdf_built = false;
 }
@@ -1924,20 +1985,15 @@ int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3
     g_last_error = "mlm_esdf_build: null box, flags other than 0 / MLM_ESDF_INFLATED, or max_dist not finite and > 0";
     return MLM_ERR_INVALID_ARG;
   }
-  int rc = esdf_refuse_sharded(h, "mlm_esdf_build");
+  int rc = refuse_sharded(h, "mlm_esdf_build");
   if (rc != MLM_OK) return rc;
   EsdfGrid G = {};
-  const double d = h->P.d_sub;
   const int n = h->P.n;
   long long cells = 1;
   for (int k = 0; k < 3; k++) {
-    // rule 1 of the ray spec: floor of the IEEE quotient, |p / d_sub| < 2^30
-    const double qa = box_min[k] / d, qb = box_max[k] / d;
-    if (!(std::fabs(qa) < 1073741824.0) || !(std::fabs(qb) < 1073741824.0) || !(box_min[k] <= box_max[k])) {
-      g_last_error = "mlm_esdf_build: a box corner is not finite, |p / d_sub| >= 2^30, or box_min > box_max";
-      return MLM_ERR_INVALID_ARG;
-    }
-    const int lo = (int)std::floor(qa), hi = (int)std::floor(qb);
+    int lo, hi;
+    rc = box_axis_cells(h, box_min[k], box_max[k], "mlm_esdf_build", &lo, &hi);
+    if (rc != MLM_OK) return rc;
     const long long nk = (long long)hi - lo + 1;
     if (nk > kEsdfMaxAxis) {
       g_last_error = "mlm_esdf_build: more than 4096 cells along an axis";
@@ -1953,23 +2009,14 @@ int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3
     g_last_error = "mlm_esdf_build: more than 2^28 cells in the box";
     return MLM_ERR_CAPACITY;
   }
-  G.d = d;
+  G.d = h->P.d_sub;
   G.max_dist = max_dist;
   CUDA_TRY(cudaSetDevice(h->device));
-  if ((size_t)cells > h->esdf_cap) {  // grow: blocking bytes, two int2 grids (the first ends as the values), two stacks
+  if ((size_t)cells > h->esdf_cap) {
     esdf_free(h);
-    const size_t c = (size_t)cells;
-    cudaError_t e = cudaMalloc((void **)&h->esdf_blk, c);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&h->esdf_a, c * sizeof(int2));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&h->esdf_b, c * sizeof(int2));
-    if (e == cudaSuccess) e = cudaMalloc((void **)&h->esdf_stk, 2 * c * sizeof(int2));
-    if (e != cudaSuccess) {
-      esdf_free(h);
-      cudaGetLastError();
-      g_last_error = std::string("mlm_esdf_build: grid buffers: ") + cudaGetErrorString(e);
-      return MLM_ERR_CUDA;
-    }
-    h->esdf_cap = c;
+    rc = scratch_alloc(esdf_scratch(h, (size_t)cells), "mlm_esdf_build: grid buffers");
+    if (rc != MLM_OK) return rc;
+    h->esdf_cap = (size_t)cells;
   }
   cudaStream_t s = h->stream;
   const int subs = G.gdims[0] * G.gdims[1] * G.gdims[2];
@@ -1987,15 +2034,18 @@ int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3
   return MLM_OK;
 }
 
+static void esdf_distance_launch(mlm_handle h, const double *d_pos, size_t n, double *d_dist, double *d_grad3n) {
+  k_esdf_query<<<grid_for(n, 256), 256, 0, h->stream>>>(h->esdf_grid, reinterpret_cast<const double *>(h->esdf_a),
+                                                        d_pos, n, d_dist, d_grad3n);
+  h->launches++;
+}
 int mlm_esdf_distance_device(mlm_handle h, const double *d_pos, size_t n, double *d_dist, double *d_grad3n) {
   if (!h || ((!d_pos || !d_dist) && n)) return MLM_ERR_INVALID_ARG;
   const int rc = esdf_ready(h, "mlm_esdf_distance");
   if (rc != MLM_OK) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
   if (n == 0) return MLM_OK;
-  k_esdf_query<<<grid_for(n, 256), 256, 0, h->stream>>>(h->esdf_grid, reinterpret_cast<const double *>(h->esdf_a),
-                                                        d_pos, n, d_dist, d_grad3n);
-  h->launches++;
+  esdf_distance_launch(h, d_pos, n, d_dist, d_grad3n);
   return MLM_OK;
 }
 // the host variant stages the points, distances and gradients through the handle's stream (like mlm_cast_rays)
@@ -2006,21 +2056,16 @@ int mlm_esdf_distance(mlm_handle h, const double *pos, size_t n, double *dist, d
   if (n == 0) return MLM_OK;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
-  double *d_buf = nullptr;  // points, distances, gradients
-  const size_t words = n * (grad3n ? 7 : 4);
-  CUDA_TRY(cudaMallocAsync((void **)&d_buf, words * sizeof(double), s));
-  double *d_pos = d_buf, *d_dist = d_buf + 3 * n, *d_grad = grad3n ? d_buf + 4 * n : nullptr;
-  cudaError_t e = cudaMemcpyAsync(d_pos, pos, n * 24, cudaMemcpyHostToDevice, s);
-  if (e == cudaSuccess) {
-    k_esdf_query<<<grid_for(n, 256), 256, 0, s>>>(h->esdf_grid, reinterpret_cast<const double *>(h->esdf_a), d_pos, n,
-                                                  d_dist, d_grad);
-    h->launches++;
-    e = cudaMemcpyAsync(dist, d_dist, n * 8, cudaMemcpyDeviceToHost, s);
+  {
+    StreamTemp<double> d_buf(s);  // points, distances, gradients
+    CUDA_TRY(d_buf.alloc(n * (grad3n ? 7 : 4)));
+    double *d_pos = d_buf, *d_dist = d_pos + 3 * n, *d_grad = grad3n ? d_pos + 4 * n : nullptr;
+    CUDA_TRY(cudaMemcpyAsync(d_pos, pos, n * 24, cudaMemcpyHostToDevice, s));
+    esdf_distance_launch(h, d_pos, n, d_dist, d_grad);
+    CUDA_TRY(cudaMemcpyAsync(dist, d_dist, n * 8, cudaMemcpyDeviceToHost, s));
+    if (grad3n) CUDA_TRY(cudaMemcpyAsync(grad3n, d_grad, n * 24, cudaMemcpyDeviceToHost, s));
   }
-  if (e == cudaSuccess && grad3n) e = cudaMemcpyAsync(grad3n, d_grad, n * 24, cudaMemcpyDeviceToHost, s);
-  cudaFreeAsync(d_buf, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  CUDA_TRY(e);
+  CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
 }
@@ -2044,13 +2089,16 @@ static int esdf_export_check(mlm_handle h, const float *out, size_t cap, int32_t
   }
   return MLM_OK;
 }
+static void esdf_export_launch(mlm_handle h, size_t cells, float *d_out) {
+  k_esdf_export<<<grid_for(cells, 256), 256, 0, h->stream>>>(reinterpret_cast<const double *>(h->esdf_a), cells, d_out);
+  h->launches++;
+}
 int mlm_esdf_export_device(mlm_handle h, float *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]) {
   size_t cells = 0;
   const int rc = esdf_export_check(h, d_out, cap, lo3, dims3, cells);
   if (rc != MLM_OK || !d_out) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
-  k_esdf_export<<<grid_for(cells, 256), 256, 0, h->stream>>>(reinterpret_cast<const double *>(h->esdf_a), cells, d_out);
-  h->launches++;
+  esdf_export_launch(h, cells, d_out);
   return MLM_OK;
 }
 int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_t dims3[3]) {
@@ -2058,15 +2106,13 @@ int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_
   const int rc = esdf_export_check(h, out, cap, lo3, dims3, cells);
   if (rc != MLM_OK || !out) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
-  cudaStream_t s = h->stream;
-  float *d_out = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_out, cells * sizeof(float), s));
-  k_esdf_export<<<grid_for(cells, 256), 256, 0, s>>>(reinterpret_cast<const double *>(h->esdf_a), cells, d_out);
-  h->launches++;
-  cudaError_t e = cudaMemcpyAsync(out, d_out, cells * sizeof(float), cudaMemcpyDeviceToHost, s);
-  cudaFreeAsync(d_out, s);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-  CUDA_TRY(e);
+  {
+    StreamTemp<float> d_out(h->stream);
+    CUDA_TRY(d_out.alloc(cells));
+    esdf_export_launch(h, cells, d_out);
+    CUDA_TRY(cudaMemcpyAsync(out, d_out, cells * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  }
+  CUDA_TRY(cudaStreamSynchronize(h->stream));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
 }
@@ -2075,20 +2121,25 @@ int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_
 size_t mlm_sizeof_frontier_cluster(void) { return sizeof(mlm_frontier_cluster); }
 static_assert(sizeof(mlm_frontier_cluster) == sizeof(FrontierCluster), "mlm_frontier_cluster / FrontierCluster layouts differ");
 
-// all: the per-word buffers too (mlm_destroy); else the per-cell buffers only (before they grow)
-static void frontier_free(mlm_handle h, bool all) {
+// per-word buffers, allocated by the first call
+static ScratchList frontier_word_scratch(mlm_handle h) {
   FcScratch &S = h->fc;
-  for (void *p : {(void *)S.parent, (void *)S.acc_n, (void *)S.acc_s, (void *)S.acc_lo, (void *)S.acc_hi,
-                  (void *)S.acc_key, (void *)S.map, (void *)S.sk[0], (void *)S.sk[1], (void *)S.sv[0], (void *)S.sv[1]})
-    if (p) cudaFree(p);
-  S.parent = S.acc_n = S.acc_lo = S.acc_hi = S.map = S.sv[0] = S.sv[1] = nullptr;
-  S.acc_s = S.acc_key = S.sk[0] = S.sk[1] = nullptr;
+  const size_t words = (size_t)h->P.pool_blocks * h->P.front_words, slots = (size_t)h->P.ht_mask + 1;
+  return {{(void **)&S.mword, words * 4}, {(void **)&S.wbase, words * 4}, {(void **)&S.slot_cnt, (slots + 1) * 4},
+          {(void **)&S.counters, 16 * 4}};
+}
+// per-cell buffers for c frontier cells, grown by a larger frontier
+static ScratchList frontier_cell_scratch(mlm_handle h, size_t c) {
+  FcScratch &S = h->fc;
+  return {{(void **)&S.parent, c * 4},     {(void **)&S.acc_n, c * 4},      {(void **)&S.map, c * 4},
+          {(void **)&S.sv[0], c * 4},      {(void **)&S.sv[1], c * 4},      {(void **)&S.acc_lo, 3 * c * 4},
+          {(void **)&S.acc_hi, 3 * c * 4}, {(void **)&S.acc_s, 3 * c * 8},  {(void **)&S.acc_key, c * 8},
+          {(void **)&S.sk[0], c * 8},      {(void **)&S.sk[1], c * 8}};
+}
+static void frontier_free(mlm_handle h) {
+  scratch_free(frontier_cell_scratch(h, 0));
+  scratch_free(frontier_word_scratch(h));
   h->fc_cap_cells = 0;
-  if (!all) return;
-  for (void *p : {(void *)S.mword, (void *)S.wbase, (void *)S.slot_cnt, (void *)S.counters})
-    if (p) cudaFree(p);
-  S.mword = nullptr;
-  S.wbase = S.slot_cnt = S.counters = nullptr;
 }
 
 static int frontier_clusters(mlm_handle h, const double box_min[3], const double box_max[3], int32_t min_cells, int flags,
@@ -2101,45 +2152,25 @@ static int frontier_clusters(mlm_handle h, const double box_min[3], const double
                    "output with a non-zero cap";
     return MLM_ERR_INVALID_ARG;
   }
-  FcBox B = {{INT_MIN, INT_MIN, INT_MIN}, {INT_MAX, INT_MAX, INT_MAX}, 1};
-  if (box_min) {
-    B.whole = 0;
-    const double d = h->P.d_sub;
-    for (int k = 0; k < 3; k++) {
-      const double qa = box_min[k] / d, qb = box_max[k] / d;  // rule 1 of the ray spec
-      if (!(std::fabs(qa) < 1073741824.0) || !(std::fabs(qb) < 1073741824.0) || !(box_min[k] <= box_max[k])) {
-        g_last_error = "mlm_frontier_clusters: a box corner is not finite, |p / d_sub| >= 2^30, or box_min > box_max";
-        return MLM_ERR_INVALID_ARG;
-      }
-      B.lo[k] = (int)std::floor(qa);
-      B.hi[k] = (int)std::floor(qb);
-    }
+  FcBox B = {{INT_MIN, INT_MIN, INT_MIN}, {INT_MAX, INT_MAX, INT_MAX}, box_min ? 0 : 1};
+  for (int k = 0; box_min && k < 3; k++) {
+    const int rc = box_axis_cells(h, box_min[k], box_max[k], "mlm_frontier_clusters", &B.lo[k], &B.hi[k]);
+    if (rc != MLM_OK) return rc;
   }
   if (!h->P.explore) {
     g_last_error = "mlm_frontier_clusters: the handle was created without use_exploration_frontiers";
     return MLM_ERR_UNSUPPORTED;
   }
-  if (h->shard_world > 1) {
-    g_last_error = "mlm_frontier_clusters: a rank of a sharded map holds only the subboxes it owns";
-    return MLM_ERR_UNSUPPORTED;
-  }
+  int rc = refuse_sharded(h, "mlm_frontier_clusters");
+  if (rc != MLM_OK) return rc;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
   const MapParams &P = h->P;
   FcScratch &S = h->fc;
   const int slots = (int)P.ht_mask + 1;
   if (!S.mword) {
-    const size_t words = (size_t)P.pool_blocks * P.front_words;
-    cudaError_t e = cudaMalloc((void **)&S.mword, words * 4);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&S.wbase, words * 4);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&S.slot_cnt, ((size_t)slots + 1) * 4);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&S.counters, 16 * 4);
-    if (e != cudaSuccess) {
-      frontier_free(h, true);
-      cudaGetLastError();
-      g_last_error = std::string("mlm_frontier_clusters: scratch: ") + cudaGetErrorString(e);
-      return MLM_ERR_CUDA;
-    }
+    rc = scratch_alloc(frontier_word_scratch(h), "mlm_frontier_clusters: scratch");
+    if (rc != MLM_OK) return rc;
   }
   const int wgrid = h->sm_count * 8;  // warp-per-slot kernels: one full wave of 256-thread CTAs, grid-stride over the slots
   k_fc_count<<<wgrid, 256, 0, s>>>(P, h->D, B, S);
@@ -2149,23 +2180,11 @@ static int frontier_clusters(mlm_handle h, const double box_min[3], const double
   CUDA_TRY(cudaMemcpyAsync(&total, S.slot_cnt + slots, sizeof(int), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));  // the number of frontier cells sizes the per-cell buffers
   if ((size_t)total > h->fc_cap_cells) {
-    frontier_free(h, false);
-    const size_t c = (size_t)total;
-    cudaError_t e = cudaSuccess;
-    for (int **p : {&S.parent, &S.acc_n, &S.map, &S.sv[0], &S.sv[1]})
-      if (e == cudaSuccess) e = cudaMalloc((void **)p, c * 4);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&S.acc_lo, 3 * c * 4);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&S.acc_hi, 3 * c * 4);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&S.acc_s, 3 * c * 8);
-    for (unsigned long long **p : {&S.acc_key, &S.sk[0], &S.sk[1]})
-      if (e == cudaSuccess) e = cudaMalloc((void **)p, c * 8);
-    if (e != cudaSuccess) {
-      frontier_free(h, false);
-      cudaGetLastError();
-      g_last_error = std::string("mlm_frontier_clusters: per-cell buffers: ") + cudaGetErrorString(e);
-      return MLM_ERR_CUDA;
-    }
-    h->fc_cap_cells = c;
+    scratch_free(frontier_cell_scratch(h, 0));
+    h->fc_cap_cells = 0;
+    rc = scratch_alloc(frontier_cell_scratch(h, (size_t)total), "mlm_frontier_clusters: per-cell buffers");
+    if (rc != MLM_OK) return rc;
+    h->fc_cap_cells = (size_t)total;
   }
   int counts[2] = {0, 0};  // clusters kept, cells of kept clusters
   if (total > 0) {
@@ -2181,41 +2200,32 @@ static int frontier_clusters(mlm_handle h, const double box_min[3], const double
     k_fc_select<<<cgrid, 256, 0, s>>>(S, total, min_cells);
     k_fc_sort<<<1, kFcSortThreads, 0, s>>>(S);
     h->launches += 7;
-    FrontierCluster *d_out = reinterpret_cast<FrontierCluster *>(out);
-    int32_t *d_cells = cells3, *d_of = cluster_of;
     const size_t rec_n = std::min(cap, (size_t)total), lab_n = std::min(cell_cap, (size_t)total);
-    cudaError_t e = cudaSuccess;
+    StreamTemp<FrontierCluster> t_out(s);
+    StreamTemp<int32_t> t_cells(s);  // cells, then labels
+    if (!device_out && rec_n) CUDA_TRY(t_out.alloc(rec_n));
+    if (!device_out && lab_n) CUDA_TRY(t_cells.alloc(lab_n * 4));
+    FrontierCluster *d_out = device_out ? reinterpret_cast<FrontierCluster *>(out) : t_out;
+    int32_t *d_cells = device_out ? cells3 : t_cells, *d_of = device_out ? cluster_of : t_cells + 3 * lab_n;
+    k_fc_records<<<cgrid, 256, 0, s>>>(S, P.d_sub, d_out, rec_n);
+    h->launches++;
+    if (lab_n) {
+      k_fc_labels<false><<<wgrid, 256, 0, s>>>(P, h->D, S, nullptr, nullptr, 0);
+      k_fc_scan<<<1, kFcScanThreads, 0, s>>>(S.slot_cnt, slots);
+      k_fc_labels<true><<<wgrid, 256, 0, s>>>(P, h->D, S, d_cells, d_of, lab_n);
+      h->launches += 3;
+    }
+    CUDA_TRY(cudaMemcpyAsync(counts, S.counters, sizeof(counts), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));  // the counts
     if (!device_out) {
-      d_out = nullptr;
-      d_cells = d_of = nullptr;
-      if (rec_n) e = cudaMallocAsync((void **)&d_out, rec_n * sizeof(FrontierCluster), s);
-      if (e == cudaSuccess && lab_n) e = cudaMallocAsync((void **)&d_cells, lab_n * 16, s);
-      d_of = d_cells ? d_cells + 3 * lab_n : nullptr;
-    }
-    if (e == cudaSuccess) {
-      k_fc_records<<<cgrid, 256, 0, s>>>(S, P.d_sub, d_out, rec_n);
-      h->launches++;
-      if (lab_n) {
-        k_fc_labels<false><<<wgrid, 256, 0, s>>>(P, h->D, S, nullptr, nullptr, 0);
-        k_fc_scan<<<1, kFcScanThreads, 0, s>>>(S.slot_cnt, slots);
-        k_fc_labels<true><<<wgrid, 256, 0, s>>>(P, h->D, S, d_cells, d_of, lab_n);
-        h->launches += 3;
-      }
-      e = cudaMemcpyAsync(counts, S.counters, sizeof(counts), cudaMemcpyDeviceToHost, s);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(s);  // the counts
-    }
-    if (!device_out && e == cudaSuccess) {
       const size_t nr = std::min(rec_n, (size_t)counts[0]), nl = std::min(lab_n, (size_t)counts[1]);
-      if (nr) e = cudaMemcpyAsync(out, d_out, nr * sizeof(FrontierCluster), cudaMemcpyDeviceToHost, s);
-      if (e == cudaSuccess && nl) e = cudaMemcpyAsync(cells3, d_cells, nl * 12, cudaMemcpyDeviceToHost, s);
-      if (e == cudaSuccess && nl) e = cudaMemcpyAsync(cluster_of, d_of, nl * 4, cudaMemcpyDeviceToHost, s);
+      if (nr) CUDA_TRY(cudaMemcpyAsync(out, d_out, nr * sizeof(FrontierCluster), cudaMemcpyDeviceToHost, s));
+      if (nl) CUDA_TRY(cudaMemcpyAsync(cells3, d_cells, nl * 12, cudaMemcpyDeviceToHost, s));
+      if (nl) CUDA_TRY(cudaMemcpyAsync(cluster_of, d_of, nl * 4, cudaMemcpyDeviceToHost, s));
+      t_out.reset();
+      t_cells.reset();
+      CUDA_TRY(cudaStreamSynchronize(s));
     }
-    if (!device_out) {
-      if (d_out) cudaFreeAsync(d_out, s);
-      if (d_cells) cudaFreeAsync(d_cells, s);
-      if (e == cudaSuccess) e = cudaStreamSynchronize(s);
-    }
-    CUDA_TRY(e);
   }
   CUDA_TRY(cudaGetLastError());
   *n_out = (size_t)counts[0];
@@ -2367,16 +2377,16 @@ int mlm_last_frame_hits(mlm_handle h, int32_t *keys3, float *p, size_t cap, size
   k_export_hit_keys<<<grid_for(n_pad, T), T, 0, s>>>(h->P, h->D, h->D.act[h->last_parity], h->d_sort_b, n, n_pad,
                                                       h->last_order_B);
   device_sort(h, h->d_sort_b, n_pad);
-  int *d_k3 = nullptr;
-  float *d_p = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_k3, (size_t)n * 12, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_p, (size_t)n * 4, s));
-  k_export_hit_gather<<<grid_for(n, T), T, 0, s>>>(h->P, h->D, h->d_sort_a, h->d_sort_b, n, d_k3, d_p);
-  h->launches += 3;
-  CUDA_TRY(cudaMemcpyAsync(keys3, d_k3, (size_t)n * 12, cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaMemcpyAsync(p, d_p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaFreeAsync(d_k3, s));
-  CUDA_TRY(cudaFreeAsync(d_p, s));
+  {
+    StreamTemp<int> d_k3(s);
+    StreamTemp<float> d_p(s);
+    CUDA_TRY(d_k3.alloc((size_t)n * 3));
+    CUDA_TRY(d_p.alloc((size_t)n));
+    k_export_hit_gather<<<grid_for(n, T), T, 0, s>>>(h->P, h->D, h->d_sort_a, h->d_sort_b, n, d_k3, d_p);
+    h->launches += 3;
+    CUDA_TRY(cudaMemcpyAsync(keys3, d_k3, (size_t)n * 12, cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(p, d_p, (size_t)n * 4, cudaMemcpyDeviceToHost, s));
+  }
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
@@ -2386,25 +2396,25 @@ int mlm_last_frame_misses(mlm_handle h, uint64_t *idx, size_t cap, size_t *n_out
   if (!h || !n_out) return MLM_ERR_INVALID_ARG;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
-  int *d_cnt = nullptr;
-  unsigned long long *d_out = nullptr;
   const size_t words = (size_t)h->P.nPhi * h->P.col_words;
-  CUDA_TRY(cudaMallocAsync((void **)&d_cnt, sizeof(int), s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_out, std::max<size_t>(cap, 1) * 8, s));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(int), s));
-  k_export_miss<<<grid_for(words, 256), 256, 0, s>>>(h->P, h->D, d_out, d_cnt, (int)std::min<size_t>(cap, 0x7fffffff));
-  h->launches++;
-  int cnt = 0;
-  CUDA_TRY(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaStreamSynchronize(s));
-  *n_out = (size_t)cnt;
-  if (idx && cap >= (size_t)cnt && cnt > 0) {
-    CUDA_TRY(cudaMemcpyAsync(idx, d_out, (size_t)cnt * 8, cudaMemcpyDeviceToHost, s));
+  {
+    StreamTemp<int> d_cnt(s);
+    StreamTemp<unsigned long long> d_out(s);
+    CUDA_TRY(d_cnt.alloc(1));
+    CUDA_TRY(d_out.alloc(std::max<size_t>(cap, 1)));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(int), s));
+    k_export_miss<<<grid_for(words, 256), 256, 0, s>>>(h->P, h->D, d_out, d_cnt, (int)std::min<size_t>(cap, 0x7fffffff));
+    h->launches++;
+    int cnt = 0;
+    CUDA_TRY(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
-    std::sort(idx, idx + cnt);  // export formatting only: ascending cell index
+    *n_out = (size_t)cnt;
+    if (idx && cap >= (size_t)cnt && cnt > 0) {
+      CUDA_TRY(cudaMemcpyAsync(idx, d_out, (size_t)cnt * 8, cudaMemcpyDeviceToHost, s));
+      CUDA_TRY(cudaStreamSynchronize(s));
+      std::sort(idx, idx + cnt);  // export formatting only: ascending cell index
+    }
   }
-  CUDA_TRY(cudaFreeAsync(d_cnt, s));
-  CUDA_TRY(cudaFreeAsync(d_out, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
@@ -2424,46 +2434,40 @@ int export_common(mlm_handle h, size_t cap_submaps, int32_t *glb3, uint8_t *coll
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
   const MapParams &P = h->P;
-  int *d_cnt = nullptr, *d_glb = nullptr, *d_blk = nullptr;
   const size_t cap = std::max<size_t>(cap_submaps, 1);
-  CUDA_TRY(cudaMallocAsync((void **)&d_cnt, sizeof(int), s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_glb, cap * 12, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_blk, cap * 4, s));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(int), s));
-  k_export_list<<<grid_for((size_t)P.ht_mask + 1, 256), 256, 0, s>>>(P, h->D, d_glb, d_blk, d_cnt, (int)cap_submaps);
-  int cnt = 0;
-  CUDA_TRY(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaStreamSynchronize(s));
-  *n_out = (size_t)cnt;
-  if (cnt > 0 && (size_t)cnt <= cap_submaps) {
-    char *d_occ = nullptr, *d_inf = nullptr;
-    float *d_lo = nullptr;
-    unsigned char *d_col = nullptr;
-    uint32_t *d_front = nullptr;
-    const size_t cells = (size_t)cnt * P.cells;
-    CUDA_TRY(cudaMallocAsync((void **)&d_occ, cells, s));
-    CUDA_TRY(cudaMallocAsync((void **)&d_inf, cells, s));
-    CUDA_TRY(cudaMallocAsync((void **)&d_lo, cells * 4, s));
-    CUDA_TRY(cudaMallocAsync((void **)&d_col, (size_t)cnt, s));
-    if (front) CUDA_TRY(cudaMallocAsync((void **)&d_front, (size_t)cnt * P.front_words * 4, s));
-    k_export_blocks<<<cnt, 256, 0, s>>>(P, h->D, d_blk, cnt, d_occ, d_inf, d_lo, d_col, d_front);
-    CUDA_TRY(cudaMemcpyAsync(glb3, d_glb, (size_t)cnt * 12, cudaMemcpyDeviceToHost, s));
-    if (collapsed) CUDA_TRY(cudaMemcpyAsync(collapsed, d_col, (size_t)cnt, cudaMemcpyDeviceToHost, s));
-    if (occupancy) CUDA_TRY(cudaMemcpyAsync(occupancy, d_occ, cells, cudaMemcpyDeviceToHost, s));
-    if (inflate_occupancy) CUDA_TRY(cudaMemcpyAsync(inflate_occupancy, d_inf, cells, cudaMemcpyDeviceToHost, s));
-    if (log_odds) CUDA_TRY(cudaMemcpyAsync(log_odds, d_lo, cells * 4, cudaMemcpyDeviceToHost, s));
-    if (front) CUDA_TRY(cudaMemcpyAsync(front, d_front, (size_t)cnt * P.front_words * 4, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaFreeAsync(d_occ, s));
-    CUDA_TRY(cudaFreeAsync(d_inf, s));
-    CUDA_TRY(cudaFreeAsync(d_lo, s));
-    CUDA_TRY(cudaFreeAsync(d_col, s));
-    if (d_front) CUDA_TRY(cudaFreeAsync(d_front, s));
+  {
+    StreamTemp<int> d_cnt(s), d_glb(s), d_blk(s);
+    CUDA_TRY(d_cnt.alloc(1));
+    CUDA_TRY(d_glb.alloc(cap * 3));
+    CUDA_TRY(d_blk.alloc(cap));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(int), s));
+    k_export_list<<<grid_for((size_t)P.ht_mask + 1, 256), 256, 0, s>>>(P, h->D, d_glb, d_blk, d_cnt, (int)cap_submaps);
+    int cnt = 0;
+    CUDA_TRY(cudaMemcpyAsync(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
-    h->launches += 2;
+    *n_out = (size_t)cnt;
+    if (cnt > 0 && (size_t)cnt <= cap_submaps) {
+      const size_t cells = (size_t)cnt * P.cells;
+      StreamTemp<char> d_occ(s), d_inf(s);
+      StreamTemp<float> d_lo(s);
+      StreamTemp<unsigned char> d_col(s);
+      StreamTemp<uint32_t> d_front(s);
+      CUDA_TRY(d_occ.alloc(cells));
+      CUDA_TRY(d_inf.alloc(cells));
+      CUDA_TRY(d_lo.alloc(cells));
+      CUDA_TRY(d_col.alloc((size_t)cnt));
+      if (front) CUDA_TRY(d_front.alloc((size_t)cnt * P.front_words));
+      k_export_blocks<<<cnt, 256, 0, s>>>(P, h->D, d_blk, cnt, d_occ, d_inf, d_lo, d_col, d_front);
+      CUDA_TRY(cudaMemcpyAsync(glb3, d_glb, (size_t)cnt * 12, cudaMemcpyDeviceToHost, s));
+      if (collapsed) CUDA_TRY(cudaMemcpyAsync(collapsed, d_col, (size_t)cnt, cudaMemcpyDeviceToHost, s));
+      if (occupancy) CUDA_TRY(cudaMemcpyAsync(occupancy, d_occ, cells, cudaMemcpyDeviceToHost, s));
+      if (inflate_occupancy) CUDA_TRY(cudaMemcpyAsync(inflate_occupancy, d_inf, cells, cudaMemcpyDeviceToHost, s));
+      if (log_odds) CUDA_TRY(cudaMemcpyAsync(log_odds, d_lo, cells * 4, cudaMemcpyDeviceToHost, s));
+      if (front) CUDA_TRY(cudaMemcpyAsync(front, d_front, (size_t)cnt * P.front_words * 4, cudaMemcpyDeviceToHost, s));
+      CUDA_TRY(cudaStreamSynchronize(s));
+      h->launches += 2;
+    }
   }
-  CUDA_TRY(cudaFreeAsync(d_cnt, s));
-  CUDA_TRY(cudaFreeAsync(d_glb, s));
-  CUDA_TRY(cudaFreeAsync(d_blk, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
@@ -2488,27 +2492,26 @@ int export_points(mlm_handle h, int kind, double height, float *xyzw, size_t cap
   if (!h || !n_out || (cap && !xyzw) || kind > MLM_CLOUD_FRONTIER) return MLM_ERR_INVALID_ARG;
   CUDA_TRY(cudaSetDevice(h->device));
   cudaStream_t s = h->stream;
-  unsigned long long *d_cnt = nullptr;
-  float4 *d_out = device_out ? reinterpret_cast<float4 *>(xyzw) : nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_cnt, sizeof(unsigned long long), s));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), s));
-  if (!device_out && cap) CUDA_TRY(cudaMallocAsync((void **)&d_out, cap * sizeof(float4), s));
-  const int grid = h->sm_count * 8;  // 8 resident CTAs of 256 threads per SM: one full wave, grid-stride over the slots
-  if (kind >= 0)
-    k_export_cloud<<<grid, 256, 0, s>>>(h->P, h->D, kind, d_out, d_cnt, (unsigned long long)cap);
-  else
-    k_export_odds_slice<<<grid, 256, 0, s>>>(h->P, h->D, height, d_out, d_cnt, (unsigned long long)cap);
-  h->launches++;
-  unsigned long long cnt = 0;
-  CUDA_TRY(cudaMemcpyAsync(&cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaStreamSynchronize(s));
-  *n_out = (size_t)cnt;
-  if (!device_out && cap) {
+  {
+    StreamTemp<unsigned long long> d_cnt(s);
+    StreamTemp<float4> t_out(s);
+    CUDA_TRY(d_cnt.alloc(1));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(unsigned long long), s));
+    if (!device_out && cap) CUDA_TRY(t_out.alloc(cap));
+    float4 *d_out = device_out ? reinterpret_cast<float4 *>(xyzw) : t_out;
+    const int grid = h->sm_count * 8;  // 8 resident CTAs of 256 threads per SM: one full wave, grid-stride over the slots
+    if (kind >= 0)
+      k_export_cloud<<<grid, 256, 0, s>>>(h->P, h->D, kind, d_out, d_cnt, (unsigned long long)cap);
+    else
+      k_export_odds_slice<<<grid, 256, 0, s>>>(h->P, h->D, height, d_out, d_cnt, (unsigned long long)cap);
+    h->launches++;
+    unsigned long long cnt = 0;
+    CUDA_TRY(cudaMemcpyAsync(&cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    *n_out = (size_t)cnt;
     const size_t n_copy = std::min<size_t>((size_t)cnt, cap);
-    if (n_copy) CUDA_TRY(cudaMemcpyAsync(xyzw, d_out, n_copy * sizeof(float4), cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaFreeAsync(d_out, s));
+    if (!device_out && n_copy) CUDA_TRY(cudaMemcpyAsync(xyzw, d_out, n_copy * sizeof(float4), cudaMemcpyDeviceToHost, s));
   }
-  CUDA_TRY(cudaFreeAsync(d_cnt, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
@@ -2619,27 +2622,25 @@ int mlm_checkpoint_save(mlm_handle h, void *buf, size_t cap, size_t *written) {
   hd.checksum = fnv1a64(nullptr, 0);
   memcpy(buf, &hd, sizeof(hd));
   if (n == 0) return MLM_OK;
-  int *d_cnt = nullptr, *d_glb = nullptr, *d_blk = nullptr;
-  unsigned char *d_rec = nullptr;
   const size_t batch = std::max<size_t>(1, std::min<size_t>(n, ((size_t)256 << 20) / rb));
-  CUDA_TRY(cudaMallocAsync((void **)&d_cnt, sizeof(int), s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_glb, n * 12, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_blk, n * 4, s));
-  CUDA_TRY(cudaMallocAsync((void **)&d_rec, batch * rb, s));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(int), s));
-  k_export_list<<<grid_for((size_t)P.ht_mask + 1, 256), 256, 0, s>>>(P, h->D, d_glb, d_blk, d_cnt, (int)n);
   unsigned char *dst = reinterpret_cast<unsigned char *>(buf) + sizeof(hd);
-  for (size_t first = 0; first < n; first += batch) {
-    const size_t m = std::min(batch, n - first);
-    k_ckpt_pack<<<(unsigned)m, 256, 0, s>>>(P, h->D, d_glb, d_blk, (int)first, (int)m, d_rec);
-    CUDA_TRY(cudaMemcpyAsync(dst + first * rb, d_rec, m * rb, cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaStreamSynchronize(s));
-    h->launches++;
+  {
+    StreamTemp<int> d_cnt(s), d_glb(s), d_blk(s);
+    StreamTemp<unsigned char> d_rec(s);
+    CUDA_TRY(d_cnt.alloc(1));
+    CUDA_TRY(d_glb.alloc(n * 3));
+    CUDA_TRY(d_blk.alloc(n));
+    CUDA_TRY(d_rec.alloc(batch * rb));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, sizeof(int), s));
+    k_export_list<<<grid_for((size_t)P.ht_mask + 1, 256), 256, 0, s>>>(P, h->D, d_glb, d_blk, d_cnt, (int)n);
+    for (size_t first = 0; first < n; first += batch) {
+      const size_t m = std::min(batch, n - first);
+      k_ckpt_pack<<<(unsigned)m, 256, 0, s>>>(P, h->D, d_glb, d_blk, (int)first, (int)m, d_rec);
+      CUDA_TRY(cudaMemcpyAsync(dst + first * rb, d_rec, m * rb, cudaMemcpyDeviceToHost, s));
+      CUDA_TRY(cudaStreamSynchronize(s));
+      h->launches++;
+    }
   }
-  CUDA_TRY(cudaFreeAsync(d_cnt, s));
-  CUDA_TRY(cudaFreeAsync(d_glb, s));
-  CUDA_TRY(cudaFreeAsync(d_blk, s));
-  CUDA_TRY(cudaFreeAsync(d_rec, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   hd.checksum = fnv1a64(dst, n * rb);
@@ -2747,32 +2748,30 @@ int mlm_checkpoint_restore(mlm_handle h, const void *buf, size_t bytes) {
   memset(h->h_fc, 0, sizeof(FrameCounters));
   int rc = MLM_OK;
   if (hd.n_records) {
-    int *d_status = nullptr;
-    unsigned char *d_rec = nullptr;
     const size_t n = (size_t)hd.n_records;
     const size_t batch = std::max<size_t>(1, std::min<size_t>(n, ((size_t)256 << 20) / rb));
-    CUDA_TRY(cudaMallocAsync((void **)&d_status, sizeof(int), s));
-    if (cudaMallocAsync((void **)&d_rec, batch * rb, s) != cudaSuccess) {
-      cudaFreeAsync(d_status, s);
+    StreamTemp<int> d_status(s);
+    StreamTemp<unsigned char> d_rec(s);
+    CUDA_TRY(d_status.alloc(1));
+    if (d_rec.alloc(batch * rb) != cudaSuccess) {
+      cudaGetLastError();
       g_last_error = "checkpoint restore: out of device memory for the staging buffer";
       return MLM_ERR_CUDA;
     }
     int status = 0;
-    cudaError_t ce = cudaMemsetAsync(d_status, 0, sizeof(int), s);
+    CUDA_TRY(cudaMemsetAsync(d_status, 0, sizeof(int), s));
     const unsigned char *src = reinterpret_cast<const unsigned char *>(buf) + sizeof(hd);
-    for (size_t first = 0; first < n && ce == cudaSuccess; first += batch) {
+    for (size_t first = 0; first < n; first += batch) {
       const size_t m = std::min(batch, n - first);
-      ce = cudaMemcpyAsync(d_rec, src + first * rb, m * rb, cudaMemcpyHostToDevice, s);
-      if (ce != cudaSuccess) break;
+      CUDA_TRY(cudaMemcpyAsync(d_rec, src + first * rb, m * rb, cudaMemcpyHostToDevice, s));
       k_ckpt_unpack<<<(unsigned)m, 256, 0, s>>>(P, D, (int)m, d_rec, d_status);
-      ce = cudaStreamSynchronize(s);
       h->launches++;
+      CUDA_TRY(cudaStreamSynchronize(s));
     }
-    if (ce == cudaSuccess) ce = cudaMemcpyAsync(&status, d_status, sizeof(int), cudaMemcpyDeviceToHost, s);
-    cudaFreeAsync(d_status, s);  // the temporaries are released on every path
-    cudaFreeAsync(d_rec, s);
-    if (ce == cudaSuccess) ce = cudaStreamSynchronize(s);
-    CUDA_TRY(ce);
+    CUDA_TRY(cudaMemcpyAsync(&status, d_status, sizeof(int), cudaMemcpyDeviceToHost, s));
+    d_status.reset();
+    d_rec.reset();
+    CUDA_TRY(cudaStreamSynchronize(s));
     if (status) {
       g_last_error = "checkpoint restore: device raised error code " + std::to_string(status);
       rc = map_device_error(status);
@@ -3291,14 +3290,15 @@ int mlm_dirty_import(mlm_handle h, const void *d_in, int32_t n_blocks) {
   CUDA_TRY(cudaSetDevice(h->device));
   if (h->P.explore) return MLM_ERR_UNSUPPORTED;
   cudaStream_t s = h->stream;
-  int *d_cnt = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_cnt, 2 * sizeof(int), s));
-  CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int), s));
-  if (n_blocks) k_dirty_import<<<n_blocks, 256, 0, s>>>(h->P, h->D, n_blocks, (const unsigned char *)d_in, d_cnt);
-  h->launches++;
   int cnt[2] = {0, 0};
-  CUDA_TRY(cudaMemcpyAsync(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
-  CUDA_TRY(cudaFreeAsync(d_cnt, s));
+  {
+    StreamTemp<int> d_cnt(s);
+    CUDA_TRY(d_cnt.alloc(2));
+    CUDA_TRY(cudaMemsetAsync(d_cnt, 0, 2 * sizeof(int), s));
+    if (n_blocks) k_dirty_import<<<n_blocks, 256, 0, s>>>(h->P, h->D, n_blocks, (const unsigned char *)d_in, d_cnt);
+    h->launches++;
+    CUDA_TRY(cudaMemcpyAsync(cnt, d_cnt, sizeof(cnt), cudaMemcpyDeviceToHost, s));
+  }
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   h->cum_ram_expand += cnt[0];
@@ -3509,15 +3509,14 @@ int mlm_debug_log10f(mlm_handle h, const float *x, size_t n, float *out) {
   if (!h || (!x && n) || (!out && n)) return MLM_ERR_INVALID_ARG;
   if (n == 0) return MLM_OK;
   CUDA_TRY(cudaSetDevice(h->device));
-  float *d_x = nullptr, *d_o = nullptr;
-  CUDA_TRY(cudaMallocAsync((void **)&d_x, n * 4, h->stream));
-  CUDA_TRY(cudaMallocAsync((void **)&d_o, n * 4, h->stream));
-  CUDA_TRY(cudaMemcpyAsync(d_x, x, n * 4, cudaMemcpyHostToDevice, h->stream));
-  k_debug_log10f<<<grid_for(n, 256), 256, 0, h->stream>>>(d_x, n, d_o, h->P.log10f_fma);
-  h->launches++;
-  CUDA_TRY(cudaMemcpyAsync(out, d_o, n * 4, cudaMemcpyDeviceToHost, h->stream));
-  CUDA_TRY(cudaFreeAsync(d_x, h->stream));
-  CUDA_TRY(cudaFreeAsync(d_o, h->stream));
+  {
+    StreamTemp<float> d_buf(h->stream);  // x, out
+    CUDA_TRY(d_buf.alloc(n * 2));
+    CUDA_TRY(cudaMemcpyAsync(d_buf, x, n * 4, cudaMemcpyHostToDevice, h->stream));
+    k_debug_log10f<<<grid_for(n, 256), 256, 0, h->stream>>>(d_buf, n, d_buf + n, h->P.log10f_fma);
+    h->launches++;
+    CUDA_TRY(cudaMemcpyAsync(out, d_buf + n, n * 4, cudaMemcpyDeviceToHost, h->stream));
+  }
   CUDA_TRY(cudaStreamSynchronize(h->stream));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
