@@ -312,6 +312,59 @@ int mlm_frontier_clusters_device(mlm_handle h, const double box_min[3], const do
                                  int flags, mlm_frontier_cluster *d_out, size_t cap, size_t *n_out, int32_t *d_cells3,
                                  int32_t *d_cluster_of, size_t cell_cap, size_t *n_cells_out);
 
+/* Candidate-view gain (no reference counterpart; the second step of a frontier-based explorer's planning cycle, which
+ * scores candidate viewpoints by what a depth camera there would see): per pose T_wb[i] (pose[7], the body pose as the
+ * frames take it), the target cells in the frustum of a pinhole sensor and how many of them it sees through free space.
+ * All arithmetic is IEEE double, correctly rounded, without fused multiply-add, in the order written.
+ *  1. Pose: T_ws = T_wb * T_bs with T_bs from the handle's config and T_sw = T_ws.inverse(), both formed as the frames
+ *     form theirs (Sophus SE3 from pose[7] normalising the quaternion, SE3::operator*, SE3::inverse); the origin is
+ *     o = T_ws.t.  A view is MLM_VIEW_INVALID (and reports 0 / 0) when a pose component is not finite, when the
+ *     quaternion's squared norm (qx^2 + qz^2) + (qy^2 + qw^2) is not > 0 or not finite, when cell(o) fails the ray spec's
+ *     rule 1, or, with boxes, when lo > hi on an axis.  These are statuses per view, not call errors.
+ *  2. Cells: the centre of cell c is x_k = ((double)c_k + 0.5) * d_sub (cell(x) == c), its sensor coordinates
+ *     p = rotate(T_sw.q, x) + T_sw.t (Eigen's _transformVector, then the sum per axis).
+ *  3. Frustum: c is in view when min_depth <= p_z <= max_depth, u = (p_x / p_z) * fx + cx and v = (p_y / p_z) * fy + cy
+ *     satisfy -0.5 <= u < (double)cols - 0.5 and -0.5 <= v < (double)rows - 0.5 (the pixel centres of project_depth:
+ *     pixel u back-projects through (u - cx) / fx), and, with boxes, lo_k <= c_k <= hi_k (boxes[6 i .. 6 i + 5] =
+ *     inclusive cells lo[3], hi[3]).
+ *  4. Targets: by default the cells whose state under the ray spec's rule 3 is UNKNOWN (neither free nor occupied; an
+ *     absent subbox is unknown, a collapsed one its element 0).  With MLM_VIEW_FRONTIER the cells whose bit is set in the
+ *     frontier sets (the frontier-clustering spec's rule 1), whatever their state.  n_target counts the targets in view,
+ *     occluded or not.
+ *  5. Line of sight: the walk of the ray spec's rule 2 from o to x, which ends in c.  The target is visible when every cell
+ *     the walk visits before c is FREE and, with MLM_VIEW_INFLATED, does not block by inflation (as with MLM_RAY_INFLATED).
+ *     The start cell counts when it is not c, so a view whose origin cell is not free sees nothing beyond it; the
+ *     target's own state and inflation are not looked at.  n_visible counts the visible targets.
+ *  6. MLM_ERR_INVALID_ARG: null handle, sensor or out; null poses with n > 0; flags other than MLM_VIEW_FRONTIER |
+ *     MLM_VIEW_INFLATED; a sensor field that is not finite; fx or fy <= 0; cols or rows < 1; not 0 <= min_depth <
+ *     max_depth.  MLM_ERR_CAPACITY: max_depth > 256 * d_sub, or a far corner off the optical axis by more than that,
+ *     max(|(-0.5 - cx) / fx|, |((double)cols - 0.5 - cx) / fx|) * max_depth > 256 * d_sub (likewise with fy, cy and
+ *     rows); this bounds a view's cells and walks.  MLM_ERR_UNSUPPORTED: MLM_VIEW_FRONTIER on a handle created without
+ *     use_exploration_frontiers, or a rank of a sharded map with world > 1 (as mlm_cast_rays).
+ *  7. The result is a snapshot of the map in stream order.  mlm_view_gain stages through the handle's stream and returns
+ *     when the records are in `out`; mlm_view_gain_device takes device pointers for the poses, boxes and records and only
+ *     enqueues (no host synchronisation).  The per-view scratch belongs to the handle: allocated by the first call, grown
+ *     for a larger batch, freed by mlm_destroy. */
+#define MLM_VIEW_FRONTIER 1 /* targets: the frontier-set cells (exploration handles only); default: the UNKNOWN cells */
+#define MLM_VIEW_INFLATED 2 /* the inflation layer blocks the line of sight, as with MLM_RAY_INFLATED */
+#define MLM_VIEW_INVALID (-2)
+typedef struct mlm_view_sensor { /* pinhole depth sensor, the project_depth model */
+  double fx, fy, cx, cy;         /* pixels */
+  int32_t cols, rows;
+  double min_depth, max_depth;   /* metres, along the optical axis */
+} mlm_view_sensor;
+typedef struct mlm_view_gain_record {
+  int32_t status;    /* 0, or MLM_VIEW_INVALID */
+  int32_t n_target;  /* target cells in the frustum (and the view's box), occluded or not */
+  int32_t n_visible; /* ... of which the line of sight is clear */
+  int32_t _pad;
+} mlm_view_gain_record; /* 16 bytes */
+size_t mlm_sizeof_view_gain(void);
+int mlm_view_gain(mlm_handle h, const double *T_wb /* n x 7 */, size_t n, const mlm_view_sensor *sensor,
+                  const int32_t *boxes /* n x 6, may be NULL */, int flags, mlm_view_gain_record *out);
+int mlm_view_gain_device(mlm_handle h, const double *d_T_wb, size_t n, const mlm_view_sensor *sensor,
+                         const int32_t *d_boxes /* may be NULL */, int flags, mlm_view_gain_record *d_out);
+
 /* ---- stream control / timing (CUDA events on the handle's own stream) ------------------------- */
 
 int mlm_sync(mlm_handle h);

@@ -127,6 +127,18 @@ FRONTIER_CONN6 = 1  # MLM_FRONTIER_CONN6
 FRONTIER_CLUSTER_DTYPE = np.dtype([("n_cells", "<i4"), ("key", "<i4", (3,)), ("lo", "<i4", (3,)), ("hi", "<i4", (3,)),
                                    ("centroid", "<f8", (3,))])
 
+VIEW_FRONTIER, VIEW_INFLATED, VIEW_INVALID = 1, 2, -2  # MLM_VIEW_FRONTIER, MLM_VIEW_INFLATED, MLM_VIEW_INVALID
+
+
+class ViewSensor(C.Structure):
+    """mirror of mlm_view_sensor (include/mlmap_b200.h): a pinhole depth sensor, the project_depth model"""
+    _fields_ = [("fx", C.c_double), ("fy", C.c_double), ("cx", C.c_double), ("cy", C.c_double), ("cols", C.c_int32),
+                ("rows", C.c_int32), ("min_depth", C.c_double), ("max_depth", C.c_double)]
+
+
+# mlm_view_gain_record (include/mlmap_b200.h): one record of mlm_view_gain, 16 bytes
+VIEW_GAIN_DTYPE = np.dtype([("status", "<i4"), ("n_target", "<i4"), ("n_visible", "<i4"), ("_pad", "<i4")])
+
 
 # every symbol include/mlmap_b200.h declares (checked by tests/test_abi.py)
 ABI_SYMBOLS = [
@@ -151,6 +163,7 @@ ABI_SYMBOLS = [
     "mlm_cast_rays", "mlm_cast_rays_device", "mlm_sizeof_ray_hit",
     "mlm_esdf_build", "mlm_esdf_distance", "mlm_esdf_distance_device", "mlm_esdf_export", "mlm_esdf_export_device",
     "mlm_frontier_clusters", "mlm_frontier_clusters_device", "mlm_sizeof_frontier_cluster",
+    "mlm_view_gain", "mlm_view_gain_device", "mlm_sizeof_view_gain",
 ]
 FRAME_KERNELS = ["k_project", "k_column", "k_fuse"]
 
@@ -217,6 +230,9 @@ def load_library() -> C.CDLL:
         "mlm_frontier_clusters_device": ([vp, dp, dp, C.c_int32, C.c_int, vp, sz, C.POINTER(sz), vp, vp, sz, C.POINTER(sz)],
                                          C.c_int),
         "mlm_sizeof_frontier_cluster": ([], C.c_size_t),
+        "mlm_view_gain": ([vp, vp, sz, C.POINTER(ViewSensor), vp, C.c_int, vp], C.c_int),
+        "mlm_view_gain_device": ([vp, vp, sz, C.POINTER(ViewSensor), vp, C.c_int, vp], C.c_int),
+        "mlm_sizeof_view_gain": ([], C.c_size_t),
         "mlm_sync": ([vp], C.c_int),
         "mlm_timer_start": ([vp], C.c_int),
         "mlm_timer_stop_ms": ([vp, fp], C.c_int),
@@ -280,7 +296,8 @@ def load_library() -> C.CDLL:
         fn.restype = ret
     if (lib.mlm_sizeof_config() != C.sizeof(MlmConfig) or lib.mlm_sizeof_frame_stats() != C.sizeof(FrameStats)
             or not lib.mlm_sizeof_ray_hit() == C.sizeof(RayHit) == RAY_HIT_DTYPE.itemsize
-            or lib.mlm_sizeof_frontier_cluster() != FRONTIER_CLUSTER_DTYPE.itemsize):
+            or lib.mlm_sizeof_frontier_cluster() != FRONTIER_CLUSTER_DTYPE.itemsize
+            or lib.mlm_sizeof_view_gain() != VIEW_GAIN_DTYPE.itemsize):
         raise MlmError(1, "ctypes struct layout does not match include/mlmap_b200.h")
     _lib = lib
     return lib
@@ -627,6 +644,34 @@ class MLMap:
                                                            d_out or None, cap, C.byref(n), d_cells3 or None,
                                                            d_cluster_of or None, cell_cap, C.byref(m)))
         return n.value, m.value
+
+    # ---- candidate-view gain (no reference counterpart; spec in include/mlmap_b200.h) --------------------------
+    @staticmethod
+    def _view_flags(frontier: bool, inflated: bool) -> int:
+        return (VIEW_FRONTIER if frontier else 0) | (VIEW_INFLATED if inflated else 0)
+
+    def view_gain(self, poses, sensor: ViewSensor, boxes=None, frontier: bool = False, inflated: bool = False) -> np.ndarray:
+        """per body pose ((n, 7) tx ty tz qw qx qy qz, as the frames take them) the target cells in the frustum of a depth
+        sensor mounted at T_bs (unknown cells, or with frontier the frontier-set cells) and how many of them it sees
+        through free cells (inflated: the inflation layer blocks too): VIEW_GAIN_DTYPE records (status 0 or
+        VIEW_INVALID, n_target, n_visible).  boxes: (n, 6) int32 inclusive cells lo[3], hi[3] that bound each view."""
+        p = np.ascontiguousarray(np.asarray(poses, dtype=np.float64).reshape(-1, 7))
+        b = None
+        if boxes is not None:
+            b = np.ascontiguousarray(np.asarray(boxes, dtype=np.int32).reshape(-1, 6))
+            if b.shape[0] != p.shape[0]:
+                raise ValueError(f"{p.shape[0]} poses but {b.shape[0]} boxes")
+        out = np.zeros(p.shape[0], dtype=VIEW_GAIN_DTYPE)
+        self._check(self._lib.mlm_view_gain(self._h, p.ctypes.data, p.shape[0], C.byref(sensor),
+                                            None if b is None else b.ctypes.data, self._view_flags(frontier, inflated),
+                                            out.ctypes.data))
+        return out
+
+    def view_gain_device(self, d_poses: int, n: int, sensor: ViewSensor, d_out: int, d_boxes: int = 0,
+                         frontier: bool = False, inflated: bool = False):
+        """the same on device memory (n x 7 doubles, n x 6 int32 boxes or 0, n 16-byte records); only enqueues"""
+        self._check(self._lib.mlm_view_gain_device(self._h, d_poses, n, C.byref(sensor), d_boxes or None,
+                                                   self._view_flags(frontier, inflated), d_out))
 
     # ---- stream / timing -------------------------------------------------------------------------
     def sync(self):

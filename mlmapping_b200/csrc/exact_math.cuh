@@ -136,4 +136,69 @@ __device__ __forceinline__ int fast_floor_div(int c, int n, uint32_t mul, int sh
   return (int)fast_div((uint32_t)(c + n * bias_q), mul, shift) - bias_q;
 }
 
+// ---- Sophus/Eigen subset, host and device (reference 3rdPartLib/Sophus/sophus/so3.cpp:42-90, se3.cpp:59-95)
+struct HQuat {
+  double w, x, y, z;
+};
+struct HPose {
+  HQuat q;
+  double t[3];
+};
+// Evaluation order as Eigen's x86-64 SSE2 build of the reference has it (packets of 2 doubles; CMakeLists.txt:4 sets no
+// -march): squaredNorm of the 4 coefficients x,y,z,w adds the two packets first, the quaternion product is the kernel
+// of Eigen/src/Geometry/arch/Geometry_SSE.h.  Checked bit for bit against oracle/_ref in tests/test_reference_pin.py.
+// The frame path composes its poses on the host, the view gain (view_kernels.cuh) on the device: one definition serves
+// both (the device code is built with -fmad=false, so no product is fused into an add there either).
+MLM_HD HQuat h_normalized(const HQuat &q) {  // MatrixBase::normalize(): z = squaredNorm(); if (z > 0) coeffs /= sqrt(z)
+  double n2 = (q.x * q.x + q.z * q.z) + (q.y * q.y + q.w * q.w);
+  if (!(n2 > 0)) return q;
+  double n = sqrt(n2);
+  return HQuat{q.w / n, q.x / n, q.y / n, q.z / n};
+}
+MLM_HD HQuat h_mul(const HQuat &a, const HQuat &b) {
+  HQuat r;
+  r.x = (a.w * b.x + a.y * b.z) - (a.z * b.y - a.x * b.w);
+  r.y = (a.w * b.y + a.y * b.w) + (a.z * b.x - a.x * b.z);
+  r.z = (a.w * b.z - a.y * b.x) + (a.z * b.w + a.x * b.y);
+  r.w = (a.w * b.w - a.y * b.y) - (a.z * b.z + a.x * b.x);
+  return r;
+}
+MLM_HD void h_rotate(const HQuat &q, const double v[3], double out[3]) {  // Eigen _transformVector
+  double uvx = q.y * v[2] - q.z * v[1];
+  double uvy = q.z * v[0] - q.x * v[2];
+  double uvz = q.x * v[1] - q.y * v[0];
+  uvx += uvx;
+  uvy += uvy;
+  uvz += uvz;
+  double cx = q.y * uvz - q.z * uvy;
+  double cy = q.z * uvx - q.x * uvz;
+  double cz = q.x * uvy - q.y * uvx;
+  out[0] = v[0] + q.w * uvx + cx;
+  out[1] = v[1] + q.w * uvy + cy;
+  out[2] = v[2] + q.w * uvz + cz;
+}
+MLM_HD HPose h_pose_from7(const double p[7]) {  // SE3(SO3(Quaterniond), t): the SO3 ctor normalises
+  HPose r;
+  r.q = h_normalized(HQuat{p[3], p[4], p[5], p[6]});
+  r.t[0] = p[0];
+  r.t[1] = p[1];
+  r.t[2] = p[2];
+  return r;
+}
+MLM_HD HPose h_compose(const HPose &a, const HPose &b) {  // SE3::operator*
+  HPose r = a;
+  double rt[3];
+  h_rotate(a.q, b.t, rt);
+  for (int i = 0; i < 3; i++) r.t[i] = r.t[i] + rt[i];
+  r.q = h_normalized(h_mul(a.q, b.q));
+  return r;
+}
+MLM_HD HPose h_inverse(const HPose &a) {  // SE3::inverse
+  HPose r;
+  r.q = h_normalized(HQuat{a.q.w, -a.q.x, -a.q.y, -a.q.z});
+  double nt[3] = {a.t[0] * -1., a.t[1] * -1., a.t[2] * -1.};
+  h_rotate(r.q, nt, r.t);
+  return r;
+}
+
 }  // namespace mlm

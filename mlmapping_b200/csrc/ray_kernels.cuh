@@ -66,31 +66,22 @@ __device__ __forceinline__ double ray_next_t(int c, int s, double d, double from
   return ((double)(c + (s > 0 ? 1 : 0)) * d - from) * inv;
 }
 
-template <bool kInflated>
-__device__ __forceinline__ RayHit cast_ray(const MapParams &P, const DeviceBuffers &D, const double *a, const double *b) {
-  RayHit r = {kRayInvalid, {0, 0, 0}, 0, 0, 0.0};
-  const double f[3] = {a[0], a[1], a[2]};
-  const double e_w[3] = {b[0], b[1], b[2]};
-  const double d = P.d_sub;
-  int c[3], e[3];
-  bool ok = true;
-#pragma unroll
-  for (int k = 0; k < 3; k++) {
-    ok = ray_cell(f[k], d, c[k]) && ok;
-    ok = ray_cell(e_w[k], d, e[k]) && ok;
-  }
-  if (!ok) return r;
+// The DDA of the spec's rule 2 from the point f in cell c to the point e_w in cell e, `total` = |e - c|_1 steps.  visit(view,
+// sub, left) sees every cell of the walk in order (its subbox, its index there, the steps still to go) and returns true to
+// stop; it must stop when left == 0.  On return c is the last cell visited and t_enter its entry t.  Rays stop at the
+// first blocking cell (cast_ray), views at the first non-free cell before the target (view_kernels.cuh).
+template <class Visit>
+__device__ __forceinline__ void ray_walk(const MapParams &P, const DeviceBuffers &D, const double f[3], const double e_w[3],
+                                         int c[3], const int e[3], long long total, double &t_enter, Visit visit) {
   int rem[3], s[3];
-  long long total = 0;
 #pragma unroll
   for (int k = 0; k < 3; k++) {
     const long long dl = (long long)e[k] - c[k];
-    total += dl < 0 ? -dl : dl;
     s[k] = dl > 0 ? 1 : (dl < 0 ? -1 : 0);
   }
-  if (total > kRayMaxCells) return r;
   double inv[3], t[3];
   int g[3], loc[3];
+  const double d = P.d_sub;
   const int n = P.n;
   const int stride[3] = {1, n, n * n};
   int sub = 0;
@@ -105,21 +96,10 @@ __device__ __forceinline__ RayHit cast_ray(const MapParams &P, const DeviceBuffe
   }
   // The current subbox (SubboxView): every step does the same one or two loads whatever kind of subbox it is in.
   SubboxView view = subbox_view(P, D, g);
-  int left = (int)total, n_free = 0, n_unknown = 0;
-  double t_enter = 0.0;
-  int status;
+  int left = (int)total;
+  t_enter = 0.0;
   for (;;) {
-    char st;
-    if (view_blocks<kInflated>(view, sub, st)) {
-      status = 0;  // MLM_OCCUPIED
-      break;
-    }
-    n_free += st == 'f' ? 1 : 0;
-    n_unknown += st == 'f' ? 0 : 1;
-    if (left == 0) {
-      status = 1;  // MLM_FREE
-      break;
-    }
+    if (visit(view, sub, left)) break;
     // the axis whose boundary comes first among those with steps left; ties go to x, then y, then z
     int ax = -1;
     double tb = 0.0;
@@ -163,6 +143,45 @@ __device__ __forceinline__ RayHit cast_ray(const MapParams &P, const DeviceBuffe
       view = subbox_view(P, D, g);
     }
   }
+}
+
+template <bool kInflated>
+__device__ __forceinline__ RayHit cast_ray(const MapParams &P, const DeviceBuffers &D, const double *a, const double *b) {
+  RayHit r = {kRayInvalid, {0, 0, 0}, 0, 0, 0.0};
+  const double f[3] = {a[0], a[1], a[2]};
+  const double e_w[3] = {b[0], b[1], b[2]};
+  const double d = P.d_sub;
+  int c[3], e[3];
+  bool ok = true;
+#pragma unroll
+  for (int k = 0; k < 3; k++) {
+    ok = ray_cell(f[k], d, c[k]) && ok;
+    ok = ray_cell(e_w[k], d, e[k]) && ok;
+  }
+  if (!ok) return r;
+  long long total = 0;
+#pragma unroll
+  for (int k = 0; k < 3; k++) {
+    const long long dl = (long long)e[k] - c[k];
+    total += dl < 0 ? -dl : dl;
+  }
+  if (total > kRayMaxCells) return r;
+  int n_free = 0, n_unknown = 0, status = 0;
+  double t_enter;
+  ray_walk(P, D, f, e_w, c, e, total, t_enter, [&](const SubboxView &view, int sub, int left) {
+    char st;
+    if (view_blocks<kInflated>(view, sub, st)) {
+      status = 0;  // MLM_OCCUPIED
+      return true;
+    }
+    n_free += st == 'f' ? 1 : 0;
+    n_unknown += st == 'f' ? 0 : 1;
+    if (left == 0) {
+      status = 1;  // MLM_FREE
+      return true;
+    }
+    return false;
+  });
   r.status = status;
   r.cell[0] = c[0];
   r.cell[1] = c[1];

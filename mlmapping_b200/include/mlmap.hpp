@@ -228,6 +228,19 @@ class mlmap {
     return out;
   }
 
+  // candidate-view gain (no reference counterpart; spec at mlm_view_gain): per body pose (pose[7] each) the target
+  // cells (unknown, or frontier) in the sensor's frustum and how many of them it sees through free cells; boxes
+  // (n x 6 inclusive cells lo, hi) may be null
+  std::vector<mlm_view_gain_record> viewGain(const double *T_wb, size_t n, const mlm_view_sensor &sensor,
+                                             const int32_t *boxes = nullptr, bool frontier = false,
+                                             bool inflated = false) {
+    std::vector<mlm_view_gain_record> out(n);
+    if (n == 0) return out;
+    const int flags = (frontier ? MLM_VIEW_FRONTIER : 0) | (inflated ? MLM_VIEW_INFLATED : 0);
+    check(mlm_view_gain(h_, T_wb, n, &sensor, boxes, flags, out.data()), "mlm_view_gain");
+    return out;
+  }
+
   // map clouds for consumers: what rviz_vis::pub_global_local_map / pub_frontier put on the wire
   // (src/rviz_vis.cpp:267-327) and mlmap::visualize_odds' slice (src/mlmap.cpp:200-284), compacted on the device.
   // Points are {x, y, z, w} floats, the layout of pcl::PointXYZ.
