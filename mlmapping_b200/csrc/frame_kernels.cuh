@@ -1427,7 +1427,7 @@ __device__ __forceinline__ void column_phase(const MapParams &P, DeviceBuffers &
   // get down to one item per CTA.  The heavy columns stay split: the heaviest item bounds the phase.
   // s_nrec afterwards: > 0 half item, < 0 merged item (even slot, -records), kCovered odd slot of a merged column, 0 idle.
   constexpr int kCovered = (int)0x80000000;
-  if (sorted && P.split && P.merge && s_nactive > (int)gridDim.x) {
+  if (sorted && P.split && s_nactive > (int)gridDim.x) {
     __shared__ int s_T, s_need, s_below;
     __shared__ int s_wc[32];
     int sh2 = 0;

@@ -109,6 +109,17 @@ uint32_t chain_cover(uint32_t n) {  // smallest chain value >= n
     if (kBucketChain[i] >= n) return kBucketChain[i];
   return 0;
 }
+// bucket count of a table with B buckets after a frame put n distinct keys in it (clear() keeps the bucket array): the
+// first insert into an empty table allocates 13 buckets, then the chain grows until the keys fit
+uint32_t bucket_growth(uint32_t B, int n) {
+  if (n > 0 && B == 1) B = 13;
+  while ((uint32_t)n > B) {
+    const uint32_t nb = chain_next(B);
+    if (nb == 0) break;
+    B = nb;
+  }
+  return B;
+}
 
 // glibc rand() == random_r() TYPE_3 (x^31 + x^3 + 1 additive feedback), stdlib/random_r.c: the reference
 // samples pixels with rand() (src/mlmap.cpp:324-325) and never calls srand(), i.e. seed 1.  Own state per
@@ -203,7 +214,6 @@ struct mlm_map {
   int pending_mode = 0;
   int frame_sms = 0;           // CTAs of k_frame when the handle shares the GPU with other maps (0: one per SM)
   bool poisoned = false;       // a frame failed after it had staged its sets: the staging was never consumed
-  int poll_counters = 1;       // the host polls the frame's sequence word in mapped memory instead of draining the stream
   uint32_t frame_seq = 0;
   int *d_sample_info = nullptr;  // sampled projection of a device image: {points, tries used}
   uint2 *d_sample_tries = nullptr;
@@ -225,7 +235,6 @@ struct mlm_map {
   cudaGraphExec_t graph_exec[3] = {nullptr, nullptr, nullptr};  // by input mode: points, depth image, sampled pixels
   cudaGraph_t graph[3] = {nullptr, nullptr, nullptr};
   cudaGraphNode_t graph_nodes[3][3] = {};
-  int use_graph = 1;
   int col_grid = 1;        // CTAs of the persistent k_column: one per SM, at most one per work column
   int use_fused = 0;       // frames run as one cooperative k_frame launch
   int frame_grid = 1;      // CTAs of k_frame (all co-resident)
@@ -382,6 +391,12 @@ int map_device_error(int e) {
 
 inline int grid_for(size_t n, int threads) { return (int)std::max<size_t>(1, (n + threads - 1) / threads); }
 
+// the frame kernels of each input mode: 0 = points, 1 = full depth image, 2 = sampled depth pixels
+using FrameKernel = void (*)(MapParams, DeviceBuffers, FrameParams);
+const FrameKernel kProjectKernels[3] = {k_project<0>, k_project<1>, k_project<2>};
+const FrameKernel kFrameKernels[3] = {k_frame<0>, k_frame<1>, k_frame<2>};
+const FrameKernel kFrameExploreKernels[3] = {k_frame_explore<0>, k_frame_explore<1>, k_frame_explore<2>};
+
 // full bitonic sort of keys[0..n_pad) ascending on the handle's stream
 void device_sort(mlm_map *h, uint64_t *keys, int n_pad) {
   if (n_pad <= 1) return;
@@ -399,19 +414,12 @@ void device_sort(mlm_map *h, uint64_t *keys, int n_pad) {
   }
 }
 
-// Slow ordering path: the frame's distinct hit keys exceed the emulated bucket count, so
-// libstdc++ would rehash mid-frame (possibly several times).  Produces virtual positions in
-// hit_t and bucket activations for the final bucket count.  Returns the final bucket count.
-// kind 0: the hit map (hit_key / hit_t / hit_bucket, act[parity]); kind 1: the miss set of exploration mode
-int order_slow_path(mlm_map *h, int n, int kind, uint32_t B_start, uint32_t *B_final_out) {
+// Re-sequences a set whose n distinct keys (O) exceed its emulated bucket count B_start, so that libstdc++ would rehash
+// mid-frame (possibly several times).  Produces virtual positions in O.stamp and bucket activations in act for the
+// final bucket count, which it returns in *B_final.
+int resequence(mlm_map *h, const OrderArrays &O, int n, uint32_t *act, uint32_t act_cap, uint32_t B_start,
+               uint32_t *B_final) {
   cudaStream_t s = h->stream;
-  uint32_t *act = kind == 0 ? h->D.act[h->last_parity] : h->D.act_miss[h->last_parity];
-  const uint32_t act_cap = kind == 0 ? h->act_cap : h->act_miss_cap;
-  OrderArrays O;
-  O.key = kind == 0 ? h->D.hit_key : h->D.miss_idx;
-  O.stamp = kind == 0 ? h->D.hit_t : h->D.miss_t;
-  O.bucket = kind == 0 ? h->D.hit_bucket : h->D.miss_bucket;
-  O.kind = kind;
   const int T = 256;
   int n_pad = next_pow2(n);
   k_order_seed<<<grid_for(n_pad, T), T, 0, s>>>(O, h->d_sort_a, n, n_pad);
@@ -441,7 +449,43 @@ int order_slow_path(mlm_map *h, int n, int kind, uint32_t B_start, uint32_t *B_f
   k_fill_u32<<<grid_for(B, T), T, 0, s>>>(act, 0xffffffffu, (int)B);
   k_order_final<<<grid_for(n, T), T, 0, s>>>(h->P, O, act, h->d_seq_a, n, B);
   h->launches += 2;
-  *B_final_out = B;
+  *B_final = B;
+  return MLM_OK;
+}
+
+// Slow ordering path of the frame's own sets.  kind 0: the hit map (hit_key / hit_t / hit_bucket, act[parity]);
+// kind 1: the miss set of exploration mode
+int order_slow_path(mlm_map *h, int n, int kind, uint32_t B_start, uint32_t *B_final_out) {
+  OrderArrays O;
+  O.key = kind == 0 ? h->D.hit_key : h->D.miss_idx;
+  O.stamp = kind == 0 ? h->D.hit_t : h->D.miss_t;
+  O.bucket = kind == 0 ? h->D.hit_bucket : h->D.miss_bucket;
+  O.kind = kind;
+  uint32_t *act = kind == 0 ? h->D.act[h->last_parity] : h->D.act_miss[h->last_parity];
+  return resequence(h, O, n, act, kind == 0 ? h->act_cap : h->act_miss_cap, B_start, B_final_out);
+}
+
+// The ordering of a frame whose staged sets cross a rehash: re-sequences the hit map (n_hit keys) and, in the
+// exploration mode, the miss set (n_miss keys; 0 otherwise) when they outgrow their emulated bucket counts, and gives
+// the frame's parameters the final counts.  Sets *slow and *order_B (the hit map's final count) when it re-sequences.
+int settle_rehash(mlm_map *h, int n_hit, int n_miss, int *slow, uint32_t *order_B) {
+  if (n_hit > h->sort_cap || n_miss > h->sort_cap) {
+    g_last_error = "hit / miss count exceeds ordering scratch";
+    return MLM_ERR_CAPACITY;
+  }
+  FrameParams &F = *h->h_fp;
+  if ((uint32_t)n_hit > h->bucket_count) {
+    *slow = 1;
+    const int rc = order_slow_path(h, n_hit, 0, h->bucket_count, order_B);
+    if (rc != MLM_OK) return rc;
+    F.bucket_count = *order_B;
+    F.bucket_c64 = pow64_mod(F.bucket_count);
+  }
+  if ((uint32_t)n_miss > h->bucket_count_miss) {
+    *slow = 1;
+    const int rc = order_slow_path(h, n_miss, 1, h->bucket_count_miss, &F.bucket_count_miss);
+    if (rc != MLM_OK) return rc;
+  }
   return MLM_OK;
 }
 
@@ -452,15 +496,6 @@ int run_frame_complete(mlm_map *h, mlm_frame_stats *stats);
 // the miss pass, and the miss-set iteration order, so it runs as direct launches with one host check of the
 // container sizes in the middle (rehash detection for both emulated containers).
 int run_frame_explore_direct(mlm_map *h, int slow, uint32_t order_B, mlm_frame_stats *stats);
-// bucket-count evolution of miss_idx_set (clear() keeps the buckets)
-void miss_set_bucket_growth(mlm_map *h, int n_miss) {
-  if (n_miss > 0 && h->bucket_count_miss == 1) h->bucket_count_miss = 13;
-  while ((uint32_t)n_miss > h->bucket_count_miss) {
-    uint32_t nb = chain_next(h->bucket_count_miss);
-    if (nb == 0) break;
-    h->bucket_count_miss = nb;
-  }
-}
 int run_frame_explore(mlm_map *h, int mode, int N, mlm_frame_stats *stats) {
   const MapParams &P = h->P;
   cudaStream_t s = h->stream;
@@ -468,12 +503,7 @@ int run_frame_explore(mlm_map *h, int mode, int N, mlm_frame_stats *stats) {
   const int parity = F.parity;
   const int proj_grid = grid_for((size_t)std::max(N, 1), kProjThreads * 2);
   F.order_mode = 1;  // rehash detection happens on the host below, not inside k_fuse
-  if (mode == 1)
-    k_project<1><<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
-  else if (mode == 2)
-    k_project<2><<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
-  else
-    k_project<0><<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
+  kProjectKernels[mode]<<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
   k_column<<<h->col_grid, kColThreads, h->col_smem_bytes, s>>>(P, h->D, F);
   if (P.split) {
     k_miss_finalize<<<h->sm_count * 4, 256, 0, s>>>(P, h->D, F);
@@ -487,23 +517,10 @@ int run_frame_explore(mlm_map *h, int mode, int N, mlm_frame_stats *stats) {
   int slow = 0;
   uint32_t order_B = h->bucket_count;
   if (mid.error == 0) {
-    if (mid.n_hit > h->sort_cap || mid.n_miss_list > h->sort_cap) {
+    const int rc = settle_rehash(h, mid.n_hit, mid.n_miss_list, &slow, &order_B);
+    if (rc != MLM_OK) {
       h->poisoned = true;  // the frame's staging stays unconsumed
-      return MLM_ERR_CAPACITY;
-    }
-    if ((uint32_t)mid.n_hit > h->bucket_count) {
-      slow = 1;
-      int rc = order_slow_path(h, mid.n_hit, 0, h->bucket_count, &order_B);
-      if (rc != MLM_OK) return rc;
-      F.bucket_count = order_B;
-      F.bucket_c64 = pow64_mod(F.bucket_count);
-    }
-    if ((uint32_t)mid.n_miss_list > h->bucket_count_miss) {
-      slow = 1;
-      uint32_t Bm = 0;
-      int rc = order_slow_path(h, mid.n_miss_list, 1, h->bucket_count_miss, &Bm);
-      if (rc != MLM_OK) return rc;
-      F.bucket_count_miss = Bm;
+      return rc;
     }
   }
   if (h->stage_call) {  // awareness layer only: the local layer follows with mlm_local_input_pc_pose_direct
@@ -533,7 +550,16 @@ int run_frame_explore_direct(mlm_map *h, int slow, uint32_t order_B, mlm_frame_s
   CUDA_TRY(cudaMemcpyAsync(h->h_fc, h->D.fc[parity], sizeof(FrameCounters), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
-  miss_set_bucket_growth(h, h->h_fc->n_miss_list);
+  h->bucket_count_miss = bucket_growth(h->bucket_count_miss, h->h_fc->n_miss_list);
+  return finish_frame(h, slow, order_B, stats);
+}
+// the rest of a normal frame whose sets are staged and ordered: the fusion pass as a stand-alone kernel
+int run_frame_fuse_direct(mlm_map *h, int slow, uint32_t order_B, mlm_frame_stats *stats) {
+  cudaStream_t s = h->stream;
+  k_fuse<0><<<h->sm_count * 4, 256, 0, s>>>(h->P, h->D, *h->h_fp);
+  h->launches++;
+  CUDA_TRY(cudaStreamSynchronize(s));
+  CUDA_TRY(cudaGetLastError());
   return finish_frame(h, slow, order_B, stats);
 }
 
@@ -625,17 +651,12 @@ int run_frame(mlm_map *h, int mode, const void *d_in, int rows, int cols, int n_
   }
   // exploration mode: one cooperative launch like a normal frame; the stand-alone passes serve the two-call interface,
   // profiling runs and devices / configurations without the cooperative launch
-  if (P.explore && (h->stage_call || h->profiling || !h->use_graph || !h->use_fused)) return run_frame_explore(h, mode, N, stats);
+  if (P.explore && (h->stage_call || h->profiling || !h->use_fused)) return run_frame_explore(h, mode, N, stats);
   if (h->stage_call) {
     // awareness layer only (awareness_map_cylindrical::input_pc_pose): hit map + miss set of the frame, staged in the
     // frame-local voxel grid; the ordering of a rehash frame is settled here so that the frame's sets can be read
     const int pg = grid_for((size_t)std::max(N, 1), kProjThreads * 2);
-    if (mode == 1)
-      k_project<1><<<pg, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
-    else if (mode == 2)
-      k_project<2><<<pg, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
-    else
-      k_project<0><<<pg, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
+    kProjectKernels[mode]<<<pg, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(P, h->D, F);
     k_column<<<h->col_grid, kColThreads, h->col_smem_bytes, s>>>(P, h->D, F);
     h->launches += 2;
     CUDA_TRY(cudaMemcpyAsync(h->h_fc, h->D.fc[parity], sizeof(FrameCounters), cudaMemcpyDeviceToHost, s));
@@ -645,15 +666,8 @@ int run_frame(mlm_map *h, int mode, const void *d_in, int rows, int cols, int n_
     uint32_t order_B = h->bucket_count;
     const int n = h->h_fc->n_hit;
     if (h->h_fc->error == 0 && (uint32_t)n > h->bucket_count) {
-      if (n > h->sort_cap) {
-        g_last_error = "hit count exceeds ordering scratch";
-        return MLM_ERR_CAPACITY;
-      }
-      slow = 1;
-      int rc = order_slow_path(h, n, 0, h->bucket_count, &order_B);
+      const int rc = settle_rehash(h, n, 0, &slow, &order_B);
       if (rc != MLM_OK) return rc;
-      F.bucket_count = order_B;
-      F.bucket_c64 = pow64_mod(order_B);
       F.order_mode = 1;
       CUDA_TRY(cudaStreamSynchronize(s));
     }
@@ -681,46 +695,33 @@ int run_frame(mlm_map *h, int mode, const void *d_in, int rows, int cols, int n_
   DeviceBuffers Dk = h->D;
   FrameParams Fk = F;
   void *kargs[3] = {&Pk, &Dk, &Fk};
-  if (prof || !h->use_graph) {
-#define MLM_MARK(i) do { if (prof) cudaEventRecord(h->kev[i], s); } while (0)
-    MLM_MARK(0);
-    if (mode == 1)
-      k_project<1><<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(Pk, Dk, Fk);
-    else if (mode == 2)
-      k_project<2><<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(Pk, Dk, Fk);
-    else
-      k_project<0><<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(Pk, Dk, Fk);
-    MLM_MARK(1);
+  if (prof) {
+    cudaEventRecord(h->kev[0], s);
+    kProjectKernels[mode]<<<proj_grid, kProjThreads, project_smem_bytes(P.nCol, kProjThreads), s>>>(Pk, Dk, Fk);
+    cudaEventRecord(h->kev[1], s);
     k_column<<<h->col_grid, kColThreads, h->col_smem_bytes, s>>>(Pk, Dk, Fk);
-    MLM_MARK(2);
+    cudaEventRecord(h->kev[2], s);
     k_fuse<0><<<h->sm_count * 4, 256, 0, s>>>(Pk, Dk, Fk);
-    MLM_MARK(3);
-#undef MLM_MARK
+    cudaEventRecord(h->kev[3], s);
   } else if (h->use_fused) {
     // the whole frame is ONE cooperative kernel (k_frame), replayed as a single-node graph
     const int G = h->frame_sms > 0 ? std::min(h->frame_sms, h->frame_grid) : h->frame_grid;
     // one tile per CTA when the frame allows it: N points dealt evenly, in 32-point rounds, at most 128 per warp
     Fk.tile_pts = std::min(kProjMaxPts * kColThreads, std::max(32, (((N + G - 1) / G) + 31) & ~31));
     F.tile_pts = Fk.tile_pts;
-    if (h->poll_counters && !h->async_call) {
+    if (!h->async_call) {
       Fk.frame_seq = F.frame_seq = ++h->frame_seq ? h->frame_seq : ++h->frame_seq;
       h->h_fc->seq = 0;
     }
     Fk.inline_resolve = F.inline_resolve = 1;
     const int gi = mode;
     cudaKernelNodeParams np = {};
-    if (P.explore)
-      np.func = mode == 1 ? (void *)k_frame_explore<1> : (mode == 2 ? (void *)k_frame_explore<2> : (void *)k_frame_explore<0>);
-    else
-      np.func = mode == 1 ? (void *)k_frame<1> : (mode == 2 ? (void *)k_frame<2> : (void *)k_frame<0>);
+    np.func = (void *)(P.explore ? kFrameExploreKernels : kFrameKernels)[mode];
     np.gridDim = dim3(G);
     np.blockDim = dim3(kColThreads);
     np.sharedMemBytes = (unsigned)h->col_smem_bytes;
     np.kernelParams = kargs;
-    static const int direct = getenv("MLM_FUSED_DIRECT") ? atoi(getenv("MLM_FUSED_DIRECT")) : 0;
-    if (direct) {
-      CUDA_TRY(cudaLaunchCooperativeKernel(np.func, np.gridDim, np.blockDim, kargs, np.sharedMemBytes, s));
-    } else if (!h->fgraph_exec[gi]) {
+    if (!h->fgraph_exec[gi]) {
       CUDA_TRY(cudaGraphCreate(&h->fgraph[gi], 0));
       CUDA_TRY(cudaGraphAddKernelNode(&h->fgraph_node[gi], h->fgraph[gi], nullptr, 0, &np));
       cudaKernelNodeAttrValue av = {};
@@ -730,13 +731,12 @@ int run_frame(mlm_map *h, int mode, const void *d_in, int rows, int cols, int n_
     } else {
       CUDA_TRY(cudaGraphExecKernelNodeSetParams(h->fgraph_exec[gi], h->fgraph_node[gi], &np));
     }
-    if (!direct) CUDA_TRY(cudaGraphLaunch(h->fgraph_exec[gi], s));
+    CUDA_TRY(cudaGraphLaunch(h->fgraph_exec[gi], s));
   } else {
     // the whole frame is one launch of a 3-kernel graph; the per-frame values travel as kernel arguments
-    const auto t0 = std::chrono::steady_clock::now();
     const int gi = mode;
     cudaKernelNodeParams np[3] = {};
-    np[0].func = mode == 1 ? (void *)k_project<1> : (mode == 2 ? (void *)k_project<2> : (void *)k_project<0>);
+    np[0].func = (void *)kProjectKernels[mode];
     np[0].gridDim = dim3(full_grid);  // fixed grid: CTAs beyond this frame's point count return at once
     np[0].blockDim = dim3(kProjThreads);
     np[0].sharedMemBytes = (unsigned)(project_smem_bytes(P.nCol, kProjThreads));
@@ -758,18 +758,9 @@ int run_frame(mlm_map *h, int mode, const void *d_in, int rows, int cols, int n_
     } else {
       for (int i = 0; i < 3; i++) CUDA_TRY(cudaGraphExecKernelNodeSetParams(h->graph_exec[gi], h->graph_nodes[gi][i], &np[i]));
     }
-    const auto t1 = std::chrono::steady_clock::now();
     CUDA_TRY(cudaGraphLaunch(h->graph_exec[gi], s));
-    const auto t2 = std::chrono::steady_clock::now();
-    if (getenv("MLM_DEBUG_HOST_TIMING")) {
-      static double acc[2] = {0, 0};
-      static int cnt = 0;
-      acc[0] += std::chrono::duration<double, std::micro>(t1 - t0).count();
-      acc[1] += std::chrono::duration<double, std::micro>(t2 - t1).count();
-      if (++cnt % 50 == 0) fprintf(stderr, "host us: setparams %.2f launch %.2f\n", acc[0] / cnt, acc[1] / cnt);
-    }
   }
-  h->launches += (prof || !h->use_graph || !h->use_fused) ? 3 : 1;
+  h->launches += (prof || !h->use_fused) ? 3 : 1;
   if (h->async_call) {  // mlm_frame_finish waits, settles a rehash frame and returns the counters
     h->frame_pending = true;
     h->pending_mode = mode;
@@ -811,65 +802,18 @@ int run_frame_complete(mlm_map *h, mlm_frame_stats *stats) {
     for (int i = 0; i < MLM_NUM_FRAME_KERNELS; i++) cudaEventElapsedTime(&h->kms[i], h->kev[i], h->kev[i + 1]);
   int slow = 0;
   uint32_t order_B = h->bucket_count;
-  if (P.explore) {
-    // fused exploration frame: done, unless the hit map or the miss set crosses a rehash (the kernel returned after
-    // staging): re-sequence what needs it and run the passes as stand-alone kernels
-    if (h->h_fc->error == 0 && h->h_fc->overflow) {
-      const int n_hit = h->h_fc->n_hit, n_miss = h->h_fc->n_miss_list;
-      if (n_hit > h->sort_cap || n_miss > h->sort_cap) {
-        g_last_error = "hit / miss count exceeds ordering scratch";
-        h->poisoned = true;  // the frame's staging stays unconsumed
-        return MLM_ERR_CAPACITY;
-      }
-      F.order_mode = 1;
-      if ((uint32_t)n_hit > h->bucket_count) {
-        slow = 1;
-        int rc = order_slow_path(h, n_hit, 0, h->bucket_count, &order_B);
-        if (rc != MLM_OK) {
-          h->poisoned = true;
-          return rc;
-        }
-        F.bucket_count = order_B;
-        F.bucket_c64 = pow64_mod(F.bucket_count);
-      }
-      if ((uint32_t)n_miss > h->bucket_count_miss) {
-        slow = 1;
-        uint32_t Bm = 0;
-        int rc = order_slow_path(h, n_miss, 1, h->bucket_count_miss, &Bm);
-        if (rc != MLM_OK) {
-          h->poisoned = true;
-          return rc;
-        }
-        F.bucket_count_miss = Bm;
-      }
-      return run_frame_explore_direct(h, slow, order_B, stats);
-    }
-    miss_set_bucket_growth(h, h->h_fc->n_miss_list);
-    return finish_frame(h, slow, order_B, stats);
-  }
   if (h->h_fc->error == 0 && h->h_fc->overflow) {
-    slow = 1;
-    const int n = h->h_fc->n_hit;
-    if (n > h->sort_cap) {
-      g_last_error = "hit count exceeds ordering scratch";
-      h->poisoned = true;  // the frame's staging stays unconsumed
-      return MLM_ERR_CAPACITY;
-    }
-    uint32_t Bf = 0;
-    int rc = order_slow_path(h, n, 0, h->bucket_count, &Bf);
+    // the frame crosses a rehash of the hit map (exploration mode: or of the miss set) and the kernel returned after
+    // staging: re-sequence what needs it and run the rest of the frame as stand-alone kernels
+    F.order_mode = 1;
+    const int rc = settle_rehash(h, h->h_fc->n_hit, P.explore ? h->h_fc->n_miss_list : 0, &slow, &order_B);
     if (rc != MLM_OK) {
-      h->poisoned = true;
+      h->poisoned = true;  // the frame's staging stays unconsumed
       return rc;
     }
-    order_B = Bf;
-    F.bucket_count = Bf;
-    F.bucket_c64 = pow64_mod(F.bucket_count);
-    F.order_mode = 1;
-    k_fuse<0><<<h->sm_count * 4, 256, 0, s>>>(P, h->D, F);
-    h->launches += 1;
-    CUDA_TRY(cudaStreamSynchronize(s));
-    CUDA_TRY(cudaGetLastError());
+    return P.explore ? run_frame_explore_direct(h, slow, order_B, stats) : run_frame_fuse_direct(h, slow, order_B, stats);
   }
+  if (P.explore) h->bucket_count_miss = bucket_growth(h->bucket_count_miss, h->h_fc->n_miss_list);
   return finish_frame(h, slow, order_B, stats);
 }
 
@@ -880,13 +824,7 @@ int finish_frame(mlm_map *h, int slow, uint32_t order_B, mlm_frame_stats *stats)
     h->cum_obs += C.obs_delta;
     h->n_submaps += C.n_new_blocks;
   }
-  // bucket-count evolution of hit_idx_odds_hashmap (clear() keeps the bucket array)
-  if (C.n_hit > 0 && h->bucket_count == 1) h->bucket_count = 13;
-  while ((uint32_t)C.n_hit > h->bucket_count) {
-    uint32_t nb = chain_next(h->bucket_count);
-    if (nb == 0) break;
-    h->bucket_count = nb;
-  }
+  h->bucket_count = bucket_growth(h->bucket_count, C.n_hit);  // hit_idx_odds_hashmap
   h->last_order_B = order_B;
   h->last_n_hit = C.n_hit;
   if (stats) {
@@ -1087,6 +1025,15 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
     }
     maxK = std::max(maxK, T.k_reach[r]);
   }
+  // test hooks: force the paths that other devices and configurations take.  MLM_NO_FUSED: the three-kernel graph of
+  // devices without the cooperative launch; MLM_DEBUG_NO_SPLIT: whole phi columns as work items; MLM_DEBUG_SORT_CAP /
+  // MLM_DEBUG_MAP_CAP: smaller shared-memory capacities, i.e. the global-memory fallback paths
+  const auto env_flag = [](const char *name) {
+    const char *e = getenv(name);
+    return e && atoi(e) != 0;
+  };
+  const bool no_fused = env_flag("MLM_NO_FUSED"), no_split = env_flag("MLM_DEBUG_NO_SPLIT");
+  const char *sort_cap_env = getenv("MLM_DEBUG_SORT_CAP"), *map_cap_env = getenv("MLM_DEBUG_MAP_CAP");
 
   mlm_map *h = new mlm_map();
   h->cfg = *cfg;
@@ -1117,14 +1064,11 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   // exploration mode the first-insert stamps of that row's miss cells come from both halves: they are settled after
   // all columns (miss_finalize_body).
   P.split = 1;
-  if (const char *e = getenv("MLM_DEBUG_NO_SPLIT_EXPLORE")) if (atoi(e) && cfg->use_exploration_frontiers) P.split = 0;
   for (int r = 0; r < P.nRho; r++)
     if (T.k_reach[r] > 0 && 2 * T.k_reach[r] >= r) P.split = 0;
   if (P.n_below < 1 || P.n_below >= P.nZ - 1 || P.nRho >= 4096 || 2 * P.nPhi > kMaxPhi) P.split = 0;
-  if (const char *e = getenv("MLM_DEBUG_NO_SPLIT")) if (atoi(e)) P.split = 0;
+  if (no_split) P.split = 0;
   P.nCol = P.nPhi * (P.split ? 2 : 1);
-  P.merge = 1;
-  if (const char *e = getenv("MLM_DEBUG_NO_MERGE")) if (atoi(e)) P.merge = 0;
   // per end cell: the ray's slope and the z rows of its neighbour contributions, with the reference's arithmetic
   // (rate = (z - n_below) / (rho * 1.0); (int)round(z +/- d * rate)), src/map_awareness.cpp:64-71,151,161
   T.rate.resize((size_t)P.nZ * P.nRho);
@@ -1215,10 +1159,8 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   int cap = (int)(avail / 16) & ~127;
   P.sort_cap_smem = cap;
   P.map_cap = kMapCap;
-  // test hooks: shrink the shared-memory capacities to force the global-memory fallback paths
-  if (const char *e = getenv("MLM_NO_GRAPH")) h->use_graph = atoi(e) ? 0 : 1;
-  if (const char *e = getenv("MLM_DEBUG_SORT_CAP")) P.sort_cap_smem = std::max(128, std::min(cap, atoi(e)) & ~127);
-  if (const char *e = getenv("MLM_DEBUG_MAP_CAP")) P.map_cap = std::max(1, std::min(kMapCap, atoi(e)));
+  if (sort_cap_env) P.sort_cap_smem = std::max(128, std::min(cap, atoi(sort_cap_env)) & ~127);
+  if (map_cap_env) P.map_cap = std::max(1, std::min(kMapCap, atoi(map_cap_env)));
   h->col_smem_bytes = (int)(bm_bytes + (size_t)cap * 16);
   h->col_grid = std::max(1, std::min(P.nCol, h->sm_count));
 
@@ -1241,7 +1183,6 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   } while (0)
 
   CUDA_TRY_H(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking));
-  if (const char *e = getenv("MLM_NO_POLL")) if (atoi(e)) h->poll_counters = 0;
   CUDA_TRY_H(cudaEventCreate(&h->ev0));
   CUDA_TRY_H(cudaEventCreate(&h->ev1));
   CUDA_TRY_H(cudaMallocHost((void **)&h->h_fp, sizeof(FrameParams)));
@@ -1252,6 +1193,9 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   // under a live handle with a larger one (two configurations in one process, e.g. a depth map next to a LiDAR map)
   const int smem_ceiling = max_optin - 1024;
   CUDA_TRY_H(cudaFuncSetAttribute(k_column, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
+  for (const FrameKernel *table : {kProjectKernels, kFrameKernels, kFrameExploreKernels})
+    for (int mode = 0; mode < 3; mode++)
+      CUDA_TRY_H(cudaFuncSetAttribute(table[mode], cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
   if ((long long)project_smem_bytes(P.nCol, kProjThreads) > (long long)max_optin - 1024) {
     mlm_destroy(h);
     g_last_error = "n_Phi too large for the projection's shared-memory histogram";
@@ -1260,26 +1204,13 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   // one cooperative launch per frame when every phase fits the resident CTA (exploration mode: k_frame_explore, with
   // its ordered passes behind further device-wide barriers)
   {
-    CUDA_TRY_H(cudaFuncSetAttribute(k_frame<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-    CUDA_TRY_H(cudaFuncSetAttribute(k_frame<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-    CUDA_TRY_H(cudaFuncSetAttribute(k_frame<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-    CUDA_TRY_H(cudaFuncSetAttribute(k_frame_explore<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-    CUDA_TRY_H(cudaFuncSetAttribute(k_frame_explore<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-    CUDA_TRY_H(cudaFuncSetAttribute(k_frame_explore<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
     int per_sm = 0, coop = 0;
-    if (P.explore)
-      CUDA_TRY_H(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_frame_explore<1>, kColThreads, h->col_smem_bytes));
-    else
-      CUDA_TRY_H(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_frame<1>, kColThreads, h->col_smem_bytes));
+    const FrameKernel k_frame_depth = (P.explore ? kFrameExploreKernels : kFrameKernels)[1];
+    CUDA_TRY_H(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_frame_depth, kColThreads, h->col_smem_bytes));
     cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, device);
     h->frame_grid = h->sm_count * std::min(per_sm, 1);
-    h->use_fused = coop && per_sm >= 1 && project_smem_bytes(P.nCol, kColThreads) <= (size_t)h->col_smem_bytes;
-    if (const char *e = getenv("MLM_NO_FUSED")) if (atoi(e)) h->use_fused = 0;
-    if (const char *e = getenv("MLM_NO_FUSED_EXPLORE")) if (atoi(e) && P.explore) h->use_fused = 0;
+    h->use_fused = coop && per_sm >= 1 && project_smem_bytes(P.nCol, kColThreads) <= (size_t)h->col_smem_bytes && !no_fused;
   }
-  CUDA_TRY_H(cudaFuncSetAttribute(k_project<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-  CUDA_TRY_H(cudaFuncSetAttribute(k_project<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
-  CUDA_TRY_H(cudaFuncSetAttribute(k_project<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_ceiling));
 
   DeviceBuffers &D = h->D;
   memset(&D, 0, sizeof(D));
@@ -1514,15 +1445,6 @@ int mlm_integrate_depth_u16(mlm_handle h, const uint16_t *img, int rows, int col
     }
     src = h->h_stage;
   }
-  // The projection reads every pixel exactly once, so page-locked input is read in place over PCIe by the
-  // kernel itself (zero-copy): the transfer overlaps the projection instead of preceding it as a separate copy.
-  static const int zero_copy = getenv("MLM_ZERO_COPY") ? atoi(getenv("MLM_ZERO_COPY")) : 0;  // opt-in: measured equal to the staged copy on this box
-  if (zero_copy) {
-    cudaPointerAttributes a2;
-    if (cudaPointerGetAttributes(&a2, src) == cudaSuccess && a2.type == cudaMemoryTypeHost && a2.devicePointer)
-      return run_frame(h, 1, a2.devicePointer, rows, cols, 0, T_wb, stats);
-    cudaGetLastError();
-  }
   // Overlapping the transfer with the projection was measured twice on B200 and lost both times against this one DMA
   // (102.7 us per frame end to end): a second DMA for the lower half of the rows with a ready word the tiles wait for
   // (+6 us: the extra copies cost more than the overlap returns), and reading that half in place over PCIe (+2 to +7 us).
@@ -1632,13 +1554,8 @@ int mlm_local_input_pc_pose_direct(mlm_handle h, mlm_frame_stats *stats) {
   }
   CUDA_TRY(cudaSetDevice(h->device));
   h->staged = false;
-  if (h->P.explore) return run_frame_explore_direct(h, h->staged_slow, h->staged_order_B, stats);
-  cudaStream_t s = h->stream;
-  k_fuse<0><<<h->sm_count * 4, 256, 0, s>>>(h->P, h->D, *h->h_fp);
-  h->launches++;
-  CUDA_TRY(cudaStreamSynchronize(s));
-  CUDA_TRY(cudaGetLastError());
-  return finish_frame(h, h->staged_slow, h->staged_order_B, stats);
+  return h->P.explore ? run_frame_explore_direct(h, h->staged_slow, h->staged_order_B, stats)
+                      : run_frame_fuse_direct(h, h->staged_slow, h->staged_order_B, stats);
 }
 
 // ---- asynchronous frames: several maps of one process share a GPU (CFG-D: 8 agent maps) -------------------------------
@@ -2902,11 +2819,6 @@ int shard_enqueue(mlm_handle h, const double *d_xyz, int n, const double T_wb[7]
   if (prof && !h->sev[0])
     for (int i = 0; i <= MLM_NUM_SHARD_KERNELS; i++) CUDA_TRY(cudaEventCreate(&h->sev[i]));
 #define MLM_SMARK(i) do { if (prof) cudaEventRecord(h->sev[i], s); } while (0)
-  static const bool host_timing = getenv("MLM_DEBUG_HOST_TIMING") != nullptr;
-  std::chrono::steady_clock::time_point ht[8];
-  int hn = 0;
-#define MLM_HT() do { if (host_timing && hn < 8) ht[hn++] = std::chrono::steady_clock::now(); } while (0)
-  MLM_HT();
   MLM_SMARK(0);
   if (h2d_src && n > 0) CUDA_TRY(cudaMemcpyAsync(h->d_input, h2d_src, (size_t)n * 24, cudaMemcpyHostToDevice, s));
   // resets of the scan in one launch (only the buckets in use: the count can at most step up the growth chain on a rehash
@@ -2916,16 +2828,13 @@ int shard_enqueue(mlm_handle h, const double *d_xyz, int n, const double T_wb[7]
                                                                             X.a[X.rank].cursor + (par ^ 1));
   h->launches++;
   MLM_SMARK(1);
-  MLM_HT();
   h->shard_stage_pending = true;
   int rc = run_frame(h, 0, d_xyz, 0, 0, n, T_wb, nullptr);
   h->shard_stage_pending = false;
   if (rc != MLM_OK) return rc;
   MLM_SMARK(3);
-  MLM_HT();
   FrameParams F = *h->h_fp;  // as the staging kernels saw it (bucket_count already lifted from 1 to 13)
   int *skip = h->d_shard_cursor + kMaxWorld;
-  const int G = h->sm_count * 2;
   // latency-bound list walks; one reservation (a same-address atomic per destination) per 1024 list entries
   // from here on the owner-side view of the frame: the first record of a subbox (or, in the push kernel, the first voxel
   // that stays on this rank) resolves / allocates it (k_fuse's tail rearms the flags)
@@ -2949,13 +2858,6 @@ int shard_enqueue(mlm_handle h, const double *d_xyz, int n, const double T_wb[7]
   CUDA_TRY(cudaMemcpyAsync(h->h_shard_state, h->d_shard_state, sizeof(ShardState), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaMemcpyAsync(h->h_fc, h->D.fc[F.parity], sizeof(FrameCounters), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaGetLastError());
-  MLM_HT();
-  if (host_timing) {
-    fprintf(stderr, "shard_enqueue host us:");
-    for (int i = 1; i < hn; i++) fprintf(stderr, " %.1f", std::chrono::duration<double, std::micro>(ht[i] - ht[i - 1]).count());
-    fprintf(stderr, "\n");
-  }
-#undef MLM_HT
   h->shard_pending = true;
   return MLM_OK;
 }
@@ -2964,7 +2866,7 @@ int shard_enqueue(mlm_handle h, const double *d_xyz, int n, const double T_wb[7]
 // Every rank holds the full gathered (key, stamp) list, so each re-sequences it on its own (same result everywhere),
 // then ingests its records with the virtual positions and fuses.  Host-driven like order_slow_path; only the first
 // scans of a map take this path (the bucket array keeps its size across clear()).
-int shard_rehash_path(mlm_handle h, const ShardState &st, uint32_t *B_out) {
+int shard_rehash_path(mlm_handle h, const ShardState &st) {
   cudaStream_t s = h->stream;
   const ShardPeers &X = h->shard_peers;
   const int par = (int)(h->shard_epoch & 1);
@@ -2984,40 +2886,20 @@ int shard_rehash_path(mlm_handle h, const ShardState &st, uint32_t *B_out) {
     off += st.cnt_hits[r];
   }
   const int T = 256;
-  FrameParams F = *h->h_fp;
-  uint32_t *act = h->D.act[F.parity];
+  FrameParams F = *h->h_fp;  // as the staging kernels saw it (bucket_count already lifted from 1 to 13)
   OrderArrays O;
   O.key = h->d_keys_all;
   O.stamp = h->d_stamps_all;
   O.bucket = h->d_bucket_all;
   O.kind = 0;
-  int n_pad = next_pow2(n_total);
-  k_order_seed<<<grid_for(n_pad, T), T, 0, s>>>(O, h->d_sort_a, n_total, n_pad);
-  device_sort(h, h->d_sort_a, n_pad);
-  k_order_take_seq<<<grid_for(n_total, T), T, 0, s>>>(h->d_sort_a, h->d_seq_a, n_total);
-  uint32_t Bs = h->bucket_count;
-  while ((uint32_t)n_total > Bs) {
-    int m = (int)std::min<uint32_t>(Bs, (uint32_t)n_total);
-    if (m > 1) {
-      int m_pad = next_pow2(m);
-      k_fill_u32<<<grid_for(Bs, T), T, 0, s>>>(act, 0xffffffffu, (int)Bs);
-      k_stage_act<<<grid_for(m, T), T, 0, s>>>(h->P, O, act, h->d_seq_a, m, Bs);
-      k_stage_keys<<<grid_for(m_pad, T), T, 0, s>>>(h->P, O, act, h->d_seq_a, h->d_sort_b, m, m_pad, Bs);
-      device_sort(h, h->d_sort_b, m_pad);
-      k_stage_apply<<<grid_for(m, T), T, 0, s>>>(h->d_sort_b, h->d_seq_a, h->d_seq_b, m);
-      k_copy_i32<<<grid_for(m, T), T, 0, s>>>(h->d_seq_a, h->d_seq_b, m);
-    }
-    uint32_t nb = chain_next(Bs);
-    if (nb == 0 || nb > h->act_cap) {
-      g_last_error = "bucket chain of the emulated container exceeded";
-      return MLM_ERR_CAPACITY;
-    }
-    Bs = nb;
-  }
-  k_fill_u32<<<grid_for(Bs, T), T, 0, s>>>(act, 0xffffffffu, (int)Bs);
-  k_order_final<<<grid_for(n_total, T), T, 0, s>>>(h->P, O, act, h->d_seq_a, n_total, Bs);
+  uint32_t Bs = 0;
+  const int rc = resequence(h, O, n_total, h->D.act[F.parity], h->act_cap, F.bucket_count, &Bs);
+  if (rc != MLM_OK) return rc;
   k_shard_scatter_stamps<<<grid_for(n_total, T), T, 0, s>>>(h->d_keys_all, h->d_stamps_all, n_total, h->d_key_stamp);
-  if (st.hit_base > 0) k_shard_restamp<<<grid_for(st.hit_base, T), T, 0, s>>>(h->P, h->D, st.hit_base, h->d_key_stamp, Bs);
+  if (st.hit_base > 0) {
+    k_shard_restamp<<<grid_for(st.hit_base, T), T, 0, s>>>(h->P, h->D, st.hit_base, h->d_key_stamp, Bs);
+    h->launches++;
+  }
   F.stage_only = 0;
   F.order_mode = 1;
   F.shard_world = 1;
@@ -3028,11 +2910,10 @@ int shard_rehash_path(mlm_handle h, const ShardState &st, uint32_t *B_out) {
   const int G = h->sm_count * 2;
   k_shard_ingest<<<G * 2, 256, 0, s>>>(X, h->P, h->D, F, par, h->d_shard_state, h->d_key_stamp);
   k_fuse<0><<<h->sm_count * 4, 256, 0, s>>>(h->P, h->D, F);
-  h->launches += 8;
+  h->launches += 3;
   CUDA_TRY(cudaMemcpyAsync(h->h_fc, h->D.fc[F.parity], sizeof(FrameCounters), cudaMemcpyDeviceToHost, s));
   CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
-  *B_out = Bs;
   return MLM_OK;
 }
 }  // namespace
@@ -3270,16 +3151,12 @@ int mlm_shard_finish(mlm_handle h, mlm_frame_stats *stats) {
                                         : "device raised error code " + std::to_string(st.error);
     return st.error == kErrPeer ? MLM_ERR_CUDA : map_device_error(st.error);
   }
-  uint32_t B = h->bucket_count;
-  if (st.n_total > 0 && B == 1) B = 13;
-  int slow = 0;
+  const uint32_t B = bucket_growth(h->bucket_count, st.n_total);
   if (st.rehash) {
-    slow = 1;
-    h->bucket_count = B;
-    rc = shard_rehash_path(h, st, &B);
+    rc = shard_rehash_path(h, st);
     if (rc != MLM_OK) return rc;
   }
-  rc = finish_frame(h, slow, B, stats);
+  rc = finish_frame(h, st.rehash, B, stats);
   h->bucket_count = B;  // finish_frame grows it from the LOCAL record count; the gathered count decides
   h->last_order_B = B;
   if (stats) {

@@ -187,22 +187,24 @@ def test_fallback_paths_global_sort_spill_and_oversized_columns(monkeypatch):
 
 def test_alternative_launch_paths_give_the_same_map(monkeypatch):
     """the frame runs as one cooperative k_frame launch by default; the three stand-alone kernels (graph or direct
-    launches) and whole-column work items (no split at the sensor row) must give the same cell sets and map"""
+    launches, the latter as profiling runs them) and whole-column work items (no split at the sensor row) must give the
+    same cell sets and map"""
     cfg = config_cfg_a()
     frames = []
     for k in range(3):
         pose = scenes.corridor_trajectory_pose(35 * k)
         frames.append((scenes.corridor_depth_frame(cfg, pose, frame_idx=k), pose))
-    for env in ({"MLM_NO_FUSED": "1"}, {"MLM_DEBUG_NO_SPLIT": "1"}, {"MLM_NO_FUSED": "1", "MLM_NO_GRAPH": "1"},
-                {"MLM_NO_FUSED": "1", "MLM_DEBUG_NO_SPLIT": "1"}):
+    for env, direct in (({"MLM_NO_FUSED": "1"}, False), ({"MLM_DEBUG_NO_SPLIT": "1"}, False),
+                        ({"MLM_NO_FUSED": "1"}, True), ({"MLM_NO_FUSED": "1", "MLM_DEBUG_NO_SPLIT": "1"}, False)):
         for k_, v_ in env.items():
             monkeypatch.setenv(k_, v_)
         gpu, orc = MLMap(cfg), Oracle(cfg)
         for k_ in env:
             monkeypatch.delenv(k_)
+        gpu.set_profiling(direct)
         for i, (img, pose) in enumerate(frames):
             st_g, st_o = gpu.integrate_depth(img, pose), orc.integrate_depth(img, pose)
-            assert_frame_parity(gpu, orc, st_g, st_o, tag=f"{env} frame{i}")
+            assert_frame_parity(gpu, orc, st_g, st_o, tag=f"{env} direct={direct} frame{i}")
         expected_launches = 3 * len(frames) if "MLM_NO_FUSED" in env else len(frames)
         assert gpu.kernel_launch_count() >= expected_launches
         assert_map_parity(gpu, orc, LO_TOL)
@@ -299,7 +301,7 @@ def test_exploration_frontiers_and_memory_release(one_launch, monkeypatch):
     that cross a rehash of the hit map or the miss set fall back to the stand-alone passes), once with the
     stand-alone passes for every frame."""
     if not one_launch:
-        monkeypatch.setenv("MLM_NO_FUSED_EXPLORE", "1")
+        monkeypatch.setenv("MLM_NO_FUSED", "1")
     cfg = config_cfg_a()
     cfg.use_exploration_frontiers = 1
     gpu, orc = MLMap(cfg), Oracle(cfg)

@@ -1,4 +1,4 @@
-"""host-side cost of mlm_shard_submit (MLM_DEBUG_HOST_TIMING=1 prints the per-section times)"""
+"""host-side cost of mlm_shard_submit and mlm_shard_finish"""
 import sys, time
 from pathlib import Path
 ROOT = Path(__file__).resolve().parent.parent
