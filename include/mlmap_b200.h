@@ -63,7 +63,7 @@ typedef struct mlm_config {
 
   /* local_map_cartesian::init_map arguments (reference src/map_local.cpp:46-53) */
   double subbox_d_xyz;  /* mlmapping_subbox_d_xyz */
-  int32_t subbox_n;     /* mlmapping_subbox_n     */
+  int32_t subbox_n;     /* mlmapping_subbox_n, 2..64 (1 is refused: the reference reads a one-cell subbox as collapsed) */
   float log_odds_min;   /* mlmapping_lm_log_odds_min */
   float log_odds_max;   /* mlmapping_lm_log_odds_max */
   float log_odds_hit;   /* mlmapping_lm_measurement_hit (read, stored, never used: map_local.cpp:128) */

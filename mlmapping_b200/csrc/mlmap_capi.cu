@@ -327,6 +327,36 @@ float host_get_odds(double coe, double dRho, int diff, size_t r) {
   res = res >= 0.999 ? 0.999 : res;
   return res;
 }
+// K(rho): the last diff_r of update_hits' loop, diff_r < 3 * sigma_in_dr(rho)   (int -> float compare)
+int host_k_reach(const mlm_config &c, int r) {
+  int K = 0;
+  for (int d = 1; d < 3 * host_sigma_in_dr(c.depth_noise_coe, c.am_d_rho, r); d++) {
+    K = d;
+    if (d > 4 * kDiffRange) break;
+  }
+  return K;
+}
+// Half-column split: records below the sensor row (z_idx < n_below) and at/above it never feed the same hit
+// cell when every neighbour step stays on its side of the row, i.e. z - n_below and
+// round(z -/+ d*rate) - n_below = round((z - n_below) * (1 -/+ d/rho)) have the same sign: 2*K(rho) < rho.
+// Their ray walks share only the row n_below itself (arbitrated through the global miss bitmap).  In the
+// exploration mode the first-insert stamps of that row's miss cells come from both halves: they are settled after
+// all columns (miss_finalize_body).
+int half_column_split(const mlm_config &c, const std::vector<int> &k_reach, int nPhi) {
+  const int nZ = c.am_n_z_below + c.am_n_z_over + 1;
+  for (int r = 0; r < c.am_n_rho; r++)
+    if (k_reach[r] > 0 && 2 * k_reach[r] >= r) return 0;
+  if (c.am_n_z_below < 1 || c.am_n_z_below >= nZ - 1 || c.am_n_rho >= 4096 || 2 * nPhi > kMaxPhi) return 0;
+  return 1;
+}
+// frame-local voxel grid: the awareness range in voxels plus a margin of a subbox and a cell on every side
+void lvg_dims(const mlm_config &c, double *dim_xy, double *dim_z) {
+  const int nZ = c.am_n_z_below + c.am_n_z_over + 1;
+  const double R = c.am_n_rho * c.am_d_rho, margin = c.subbox_n + 1;
+  *dim_xy = ceil(2 * R / c.subbox_d_xyz) + 2 * margin + 2;
+  *dim_z = ceil(nZ * c.am_d_z / c.subbox_d_xyz) + 2 * margin + 2;
+}
+
 int build_awareness_tables(const mlm_config &c, AwarenessTables &T) {
   const int nRho = c.am_n_rho;
   T.dPhi = c.am_d_phi_deg * M_PI / 180;
@@ -338,15 +368,7 @@ int build_awareness_tables(const mlm_config &c, AwarenessTables &T) {
     for (int r = 0; r < nRho; r++)
       T.odds[(size_t)(diff + kDiffRange) * nRho + r] = host_get_odds(c.depth_noise_coe, c.am_d_rho, diff, r);
   T.k_reach.resize(nRho);
-  for (int r = 0; r < nRho; r++) {
-    // loop bound of update_hits: diff_r < 3 * sigma_in_dr(rho)   (int -> float compare)
-    int K = 0;
-    for (int d = 1; d < 3 * host_sigma_in_dr(c.depth_noise_coe, c.am_d_rho, r); d++) {
-      K = d;
-      if (d > 4 * kDiffRange) break;
-    }
-    T.k_reach[r] = K;
-  }
+  for (int r = 0; r < nRho; r++) T.k_reach[r] = host_k_reach(c, r);
   T.centre_z.resize(T.nZ);
   for (int z = 0; z < T.nZ; z++) T.centre_z[z] = T.z_border_min + (c.am_d_z / 2) + (z * c.am_d_z);
   T.centre_xy.resize((size_t)T.nPhi * nRho);
@@ -368,6 +390,9 @@ int validate_config(const mlm_config &c, std::string &why) {
   if (c.am_n_rho < 2 || c.am_n_z_below < 0 || c.am_n_z_over < 0) return bad("awareness extents");
   if (c.am_n_rho >= 4096) return bad("n_Rho must be < 4096");
   if (!(c.subbox_d_xyz > 0) || c.subbox_n < 1 || c.subbox_n > 64) return bad("subbox size");
+  // the reference marks a collapsed subbox by a one-element cell vector (map_local.h:215-231): with one cell per subbox
+  // every subbox looks collapsed once it exists, so later frames and queries skip it
+  if (c.subbox_n == 1) return bad("subbox_n must be >= 2: a one-cell subbox is indistinguishable from a collapsed one");
   if (!(c.depth_noise_coe >= 0)) return bad("depth_noise_coe");
   if (c.max_points < 1 || c.max_points > (1 << 26)) return bad("max_points must be in [1, 2^26]");
   if (c.pool_submaps < 1) return bad("pool_submaps");
@@ -376,6 +401,24 @@ int validate_config(const mlm_config &c, std::string &why) {
   int nZ = c.am_n_z_below + c.am_n_z_over + 1;
   if ((long long)nZ * c.am_n_rho >= (1ll << kCellBits)) return bad("n_Z*n_Rho must be < 2^20");
   if ((long long)nZ * c.am_n_rho * nPhi >= (1ll << 31)) return bad("awareness cell count must be < 2^31");
+  // preconditions of update_hits (SURVEY §8a a3): table row index diff_r+10 <= 20 and rho-diff_r >= 0
+  std::vector<int> K(c.am_n_rho);
+  for (int r = 0; r < c.am_n_rho; r++) {
+    K[r] = host_k_reach(c, r);
+    if (K[r] > kDiffRange || K[r] > r)
+      return bad("depth_noise_coe too large: 3*sigma_in_dr(rho) reaches outside the odds table / below rho 0");
+  }
+  double lvg_xy, lvg_z;
+  lvg_dims(c, &lvg_xy, &lvg_z);
+  if (!(lvg_xy * lvg_xy * lvg_z < 2147483648.0)) return bad("frame-local voxel grid too large (awareness range / voxel size)");
+  // shared memory per block of the frame kernels on sm_100 (227 KB opt-in, 1 KB reserved); mlm_create checks the
+  // device's own limit again.  The projection keeps a histogram per work column; the column item keeps two column
+  // bitmaps, the odds table and at least a 32 KB sort buffer.
+  const int nCol = nPhi * (half_column_split(c, K, nPhi) ? 2 : 1);
+  const long long smem = kSmemOptinSm100 - 1024;
+  if ((long long)project_smem_bytes(nCol, kProjThreads) > smem) return bad("n_Phi too large for the projection's shared-memory histogram");
+  if (smem - (long long)col_smem_prefix_bytes(nZ * ((c.am_n_rho + 31) / 32), c.am_n_rho, nCol) < 32 * 1024)
+    return bad("awareness column (n_Z*n_Rho bits) does not fit shared memory");
   return MLM_OK;
 }
 
@@ -1016,15 +1059,8 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
 
   AwarenessTables T;
   build_awareness_tables(*cfg, T);
-  int maxK = 0;
-  for (int r = 0; r < cfg->am_n_rho; r++) {
-    // preconditions of update_hits (SURVEY §8a a3): table row index diff_r+10 <= 20 and rho-diff_r >= 0
-    if (T.k_reach[r] > kDiffRange || T.k_reach[r] > r) {
-      g_last_error = "depth_noise_coe too large: 3*sigma_in_dr(rho) reaches outside the odds table / below rho 0";
-      return MLM_ERR_INVALID_CONFIG;
-    }
-    maxK = std::max(maxK, T.k_reach[r]);
-  }
+  int maxK = 0;  // validate_config has checked update_hits' preconditions
+  for (int r = 0; r < cfg->am_n_rho; r++) maxK = std::max(maxK, T.k_reach[r]);
   // test hooks: force the paths that other devices and configurations take.  MLM_NO_FUSED: the three-kernel graph of
   // devices without the cooperative launch; MLM_DEBUG_NO_SPLIT: whole phi columns as work items; MLM_DEBUG_SORT_CAP /
   // MLM_DEBUG_MAP_CAP: smaller shared-memory capacities, i.e. the global-memory fallback paths
@@ -1057,17 +1093,7 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   P.cell_bits = 1;
   while ((1 << P.cell_bits) < P.nZ * P.nRho) P.cell_bits++;
   P.nRho_magic = (uint32_t)(((1ull << 32) + (uint64_t)P.nRho - 1) / (uint64_t)P.nRho);
-  // Half-column split: records below the sensor row (z_idx < n_below) and at/above it never feed the same hit
-  // cell when every neighbour step stays on its side of the row, i.e. z - n_below and
-  // round(z -/+ d*rate) - n_below = round((z - n_below) * (1 -/+ d/rho)) have the same sign: 2*K(rho) < rho.
-  // Their ray walks share only the row n_below itself (arbitrated through the global miss bitmap).  In the
-  // exploration mode the first-insert stamps of that row's miss cells come from both halves: they are settled after
-  // all columns (miss_finalize_body).
-  P.split = 1;
-  for (int r = 0; r < P.nRho; r++)
-    if (T.k_reach[r] > 0 && 2 * T.k_reach[r] >= r) P.split = 0;
-  if (P.n_below < 1 || P.n_below >= P.nZ - 1 || P.nRho >= 4096 || 2 * P.nPhi > kMaxPhi) P.split = 0;
-  if (no_split) P.split = 0;
+  P.split = no_split ? 0 : half_column_split(*cfg, T.k_reach, P.nPhi);
   P.nCol = P.nPhi * (P.split ? 2 : 1);
   // per end cell: the ray's slope and the z rows of its neighbour contributions, with the reference's arithmetic
   // (rate = (z - n_below) / (rho * 1.0); (int)round(z +/- d * rate)), src/map_awareness.cpp:64-71,151,161
@@ -1120,9 +1146,12 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   // glibc dispatches __logf to its FMA build when FMA and AVX2 are usable (ifunc-fma.h)
   P.log10f_fma = (__builtin_cpu_supports("fma") && __builtin_cpu_supports("avx2")) ? 1 : 0;
   P.lvg_margin = P.n + 1;
-  const double R = P.nRho * P.dRho;
-  P.lvg_dim_xy = (int)ceil(2 * R / P.d_sub) + 2 * P.lvg_margin + 2;
-  P.lvg_dim_z = (int)ceil(P.nZ * P.dZ / P.d_sub) + 2 * P.lvg_margin + 2;
+  {
+    double xy, z;  // below 2^31 cells (validate_config)
+    lvg_dims(*cfg, &xy, &z);
+    P.lvg_dim_xy = (int)xy;
+    P.lvg_dim_z = (int)z;
+  }
   make_div_magic((uint32_t)P.lvg_dim_xy, &P.dxy_mul, &P.dxy_shift);
   make_div_magic((uint32_t)P.lvg_dim_xy * (uint32_t)P.lvg_dim_xy, &P.dxy2_mul, &P.dxy2_shift);
   make_div_magic((uint32_t)P.n, &P.n_mul, &P.n_shift);
@@ -1131,11 +1160,6 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
   const long long n_cells = (long long)P.nZ * P.nPhi * P.nRho;
   const long long lvg_cells = (long long)P.lvg_dim_xy * P.lvg_dim_xy * P.lvg_dim_z;
   const long long lsg_cells = (long long)P.lsg_dim_xy * P.lsg_dim_xy * P.lsg_dim_z;
-  if (lvg_cells >= (1ll << 31)) {
-    delete h;
-    g_last_error = "frame-local voxel grid too large (awareness range / voxel size)";
-    return MLM_ERR_INVALID_CONFIG;
-  }
   P.max_points = cfg->max_points;
   P.contrib_per_point = 1 + 2 * maxK;
   P.max_hits = (int)std::min<long long>(n_cells, (long long)P.max_points * P.contrib_per_point);
@@ -3196,7 +3220,10 @@ int mlm_shard_last_exchange(mlm_handle h, mlm_shard_exchange *out) {
 // ---- replicated map: ship the subbox blocks touched by the last frame --------------------------------------
 int mlm_dirty_count(mlm_handle h, int32_t *n_blocks, size_t *record_bytes) {
   if (!h || !n_blocks || !record_bytes) return MLM_ERR_INVALID_ARG;
-  if (h->P.explore) return MLM_ERR_UNSUPPORTED;
+  if (h->P.explore) {
+    g_last_error = "mlm_dirty_count: dirty-block shipping does not carry frontier sets or collapses (exploration mode)";
+    return MLM_ERR_UNSUPPORTED;
+  }
   *n_blocks = h->h_fc->n_touched_sub;
   *record_bytes = dirty_record_bytes(h->P.cells);
   return MLM_OK;

@@ -8,7 +8,8 @@ namespace mlm {
 
 constexpr int kDiffRange = 10;          // awareness_map_cylindrical::diff_range (map_awareness.cpp:36)
 constexpr int kOddsRows = 2 * kDiffRange + 1;
-constexpr int kMaxPhi = 4096;           // upper bound on nPhi for the shared-memory histogram
+constexpr int kMaxPhi = 4096;           // n_Phi range of validate_config; above kMaxPhi / 2 columns are not split
+constexpr int kSmemOptinSm100 = 227 * 1024;  // opt-in shared memory per block on sm_100 (validate_config's limits)
 constexpr uint64_t kEmptyKey = ~0ull;   // empty slot of the submap hash table
 constexpr int kBlockPending = -1;
 constexpr int kBlockCollapsed = -2;     // ht_val of a subbox collapsed by the release pass (map_local.cpp:208-232)

@@ -13,7 +13,7 @@ from pathlib import Path
 import numpy as np
 
 from mlmapping_b200.capi import ESDF_INFLATED, MlmConfig, MlmError
-from oracle_binding import _prototypes
+from oracle_binding import _prototypes, create_handle
 from ray_oracle import RayOracle
 
 _ORACLE_DIR = Path(__file__).resolve().parent.parent / "oracle"
@@ -86,7 +86,7 @@ class EsdfOracle(RayOracle):
         self.impl = "port"
         self.lib = load()
         self.cfg = cfg.copy()
-        self.h = C.c_void_p(self.lib.orc_create(C.byref(self.cfg)))
+        self.h = create_handle(self.lib, self.cfg)
         self.lib.orc_set_bookkeeping(self.h, 1 if bookkeeping else 0)
         self.cells = cfg.subbox_n ** 3
         self.last_seconds = 0.0

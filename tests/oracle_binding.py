@@ -126,6 +126,43 @@ def best_oracle(cfg, **kw):
     return Oracle(cfg, impl="reference" if reference_available() else "port", **kw)
 
 
+K_DIFF_RANGE = 10  # rows either side of the odds table (awareness_map_cylindrical::diff_range)
+
+
+def k_reach(cfg) -> np.ndarray:
+    """K(rho): the last diff_r of update_hits' loop `diff_r < 3 * sigma_in_dr(rho)`, with the float arithmetic of
+    build_awareness_tables (mlmap_capi.cu): dis = (float)(rho * dRho), sigma = (float)(coe * dis * dis / dRho)"""
+    out = np.zeros(cfg.am_n_rho, dtype=np.int64)
+    for r in range(cfg.am_n_rho):
+        dis = float(np.float32(r * cfg.am_d_rho))
+        bound = np.float32(3) * np.float32(cfg.depth_noise_coe * dis * dis / cfg.am_d_rho)
+        k, d = 0, 1
+        while np.float32(d) < bound:
+            k = d
+            if d > 4 * K_DIFF_RANGE:
+                break
+            d += 1
+        out[r] = k
+    return out
+
+
+def update_hits_ok(cfg) -> bool:
+    """mlm_create's precondition of update_hits: K(rho) <= min(10, rho) for every rho, so that the odds-table row
+    diff_r + 10 stays within its 21 rows and the neighbour rho - diff_r stays >= 0"""
+    k = k_reach(cfg)
+    return bool((k <= np.minimum(K_DIFF_RANGE, np.arange(cfg.am_n_rho))).all())
+
+
+def create_handle(lib, cfg) -> C.c_void_p:
+    """orc_create, for configurations the library accepts: update_hits (the reference's code, restated) reads outside
+    the odds table and the awareness map when 3 sigma(rho) reaches past them, so such a configuration is refused here
+    instead of crashing the process"""
+    if not (cfg.am_n_rho >= 2 and cfg.am_d_rho > 0 and cfg.depth_noise_coe >= 0) or not update_hits_ok(cfg):
+        raise ValueError("configuration outside update_hits' preconditions: K(rho) <= min(10, rho) fails "
+                         f"(am_d_rho {cfg.am_d_rho}, am_n_rho {cfg.am_n_rho}, depth_noise_coe {cfg.depth_noise_coe})")
+    return C.c_void_p(lib.orc_create(C.byref(cfg)))
+
+
 def _d7(a):
     a = np.asarray(a, dtype=np.float64).reshape(-1)
     return (C.c_double * len(a))(*a.tolist())
@@ -140,7 +177,7 @@ class Oracle:
         self.impl = impl
         self.lib = load_reference() if impl == "reference" else load_oracle()
         self.cfg = cfg.copy()
-        self.h = C.c_void_p(self.lib.orc_create(C.byref(self.cfg)))
+        self.h = create_handle(self.lib, self.cfg)
         self.lib.orc_set_bookkeeping(self.h, 1 if bookkeeping else 0)
         self.cells = cfg.subbox_n ** 3
         self.last_seconds = 0.0

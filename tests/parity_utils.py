@@ -44,6 +44,8 @@ def assert_map_parity(gpu, orc, lo_tol=1e-6, tag=""):
 
 def _sorted_rows(a):
     a = np.ascontiguousarray(a)
+    if a.shape[0] == 0:
+        return a
     v = a.view(np.uint32).reshape(a.shape[0], -1)
     return a[np.lexsort(tuple(v[:, c] for c in range(v.shape[1] - 1, -1, -1)))]
 

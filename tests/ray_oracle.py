@@ -12,7 +12,7 @@ from pathlib import Path
 import numpy as np
 
 from mlmapping_b200.capi import RAY_HIT_DTYPE, RAY_INFLATED, MlmConfig
-from oracle_binding import Oracle, _prototypes
+from oracle_binding import Oracle, _prototypes, create_handle
 
 _ORACLE_DIR = Path(__file__).resolve().parent.parent / "oracle"
 _SOURCES = [_ORACLE_DIR / "oracle_rays.cpp", _ORACLE_DIR / "oracle_capi.cpp", _ORACLE_DIR / "mlmap_oracle.hpp",
@@ -58,7 +58,7 @@ class RayOracle(Oracle):
         self.impl = "port"
         self.lib = load()
         self.cfg = cfg.copy()
-        self.h = C.c_void_p(self.lib.orc_create(C.byref(self.cfg)))
+        self.h = create_handle(self.lib, self.cfg)
         self.lib.orc_set_bookkeeping(self.h, 1 if bookkeeping else 0)
         self.cells = cfg.subbox_n ** 3
         self.last_seconds = 0.0
