@@ -8,8 +8,9 @@
 namespace mlm {
 
 // logit_inv, include/mlmap.h:40: pow(10, x) / (1 + pow(10, x)) in double, returned as float.  10^x through exp10
-// (1 ulp in double, a third of pow's instructions): the float result differs from glibc's in the last bit at most,
-// which is the tolerance the parity tests state for getOdd
+// (1 ulp in double, a third of pow's instructions).  Moving 10^x by one double ulp either way changes the float result
+// for no float x with 2^-28 <= |x| <= 64 (tests/test_query_grad_host.py scans every one; below 2^-28 the odd is 0.5),
+// so getOdd equals glibc's bit for bit wherever exp10 keeps its documented bound
 __device__ __forceinline__ float logit_inv_f(float lo) {
   double y = exp10((double)lo);
   return (float)(y / (1 + y));
@@ -284,11 +285,13 @@ __global__ void __launch_bounds__(256, MLM_GRAD_MINB) k_get_odd_grad(MapParams P
   // below the running minimum; a round that finds one ends the search.  logit_inv is monotone non-decreasing in the
   // log-odds (also after the cast to float), so the round's winner is the neighbour with the lowest log-odds (the first
   // of those), unless an EARLIER neighbour with a slightly higher log-odds rounds to the same float odd; those rare
-  // near-ties (within kTie, far more than one float ulp of the odd anywhere in the clamped range) are settled with
-  // their own pow.  The walk itself compares log-odds only: the first round whose minimum lies below the origin's is the
-  // candidate, and its odd is computed AFTER the loop, next to the origin's, where the warp is converged again (a pow
-  // inside the loop runs for the few lanes whose search ends in that round, once per round).
-  const float kTie = 1e-2f;
+  // near-ties are settled with their own pow.  Below kNearOne every float log-odds with the same float odd as lo_m lies
+  // within kTie of it (tests/test_query_grad_host.py computes the first lo_m where this fails: 5.586); closer to odd 1
+  // the float odd's spacing of 2^-24 spans more than kTie of log-odds, and below -30 the odd underflows, so there every
+  // earlier direction is checked.  The walk itself compares log-odds only: the first round whose minimum lies below the
+  // origin's is the candidate, and its odd is computed AFTER the loop, next to the origin's, where the warp is converged
+  // again (a pow inside the loop runs for the few lanes whose search ends in that round, once per round).
+  const float kTie = 1e-2f, kNearOne = 5.5f;
   float lo_d[6];
   int m = 0, k = max_iter + 1;
   float lo_m = lo0;
@@ -339,7 +342,7 @@ __global__ void __launch_bounds__(256, MLM_GRAD_MINB) k_get_odd_grad(MapParams P
       // earlier directions whose log-odds is a hair above the minimum: same float odd -> the reference keeps the earlier one
 #pragma unroll
       for (int d = 0; d < 5; d++)
-        if (d < m && (lo_d[d] - lo_m <= kTie || lo_m < -30.0f) && lo_d[d] < lo0) {  // (below 10^-30 the float odd underflows: any gap can tie)
+        if (d < m && (lo_d[d] - lo_m <= kTie || lo_m < -30.0f || lo_m > kNearOne) && lo_d[d] < lo0) {
           if (logit_inv_f(lo_d[d]) == odd_m) {
             best_d = d;
             break;

@@ -143,10 +143,11 @@ extern "C" int orc_view_gain(void *h, const double *T_wb, size_t n, const mlm_vi
 }
 
 // Replaces the restatement's map with m subboxes given as mlm_export_map / orc_export_frontier lay them out (glb3,
-// collapsed flags, occupancy and inflation bytes per cell, frontier bits per cell): the crafted maps of the tests.
-// A collapsed subbox keeps element 0 of its occupancy and inflation only, and no frontier.
+// collapsed flags, occupancy and inflation bytes per cell, frontier bits per cell, log-odds per cell): the crafted maps
+// of the tests.  A collapsed subbox keeps element 0 of its occupancy, inflation and log-odds only, and no frontier.
+// log_odds may be NULL: every log-odds 0.
 extern "C" void orc_view_set_map(void *h, size_t m, const int32_t *glb3, const uint8_t *collapsed, const char *occ,
-                                 const char *infl, const uint8_t *front_bits) {
+                                 const char *infl, const uint8_t *front_bits, const float *log_odds) {
   auto *L = static_cast<orc::mlmap *>(h)->local;
   const size_t cells = L->cell_num_subbox, nb = (cells + 7) / 8;
   L->observed_group_map.clear();
@@ -155,7 +156,10 @@ extern "C" void orc_view_set_map(void *h, size_t m, const int32_t *glb3, const u
     const size_t k = collapsed[i] ? 1 : cells;
     sb.occupancy.assign(occ + i * cells, occ + i * cells + k);
     sb.inflate_occupancy.assign(infl + i * cells, infl + i * cells + k);
-    sb.log_odds.assign(k, 0.0f);
+    if (log_odds)
+      sb.log_odds.assign(log_odds + i * cells, log_odds + i * cells + k);
+    else
+      sb.log_odds.assign(k, 0.0f);
     sb.frontier.clear();
     for (size_t c = 0; !collapsed[i] && c < cells; c++)
       if (front_bits[i * nb + c / 8] >> (c & 7) & 1) sb.frontier.insert((int)c);

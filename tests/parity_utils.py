@@ -53,7 +53,7 @@ def _sorted_rows(a):
 def assert_cloud_parity(gpu, orc, kinds=(0, 1), heights=(0.75, 1.25), tag=""):
     """map clouds for consumers (rviz_vis.cpp:267-327, mlmap.cpp:200-284): same point SETS bit for bit (the order
     of the reference's clouds is its unordered_map iteration order, which no consumer can rely on); the slice's
-    odd within one float ulp like getOdd"""
+    odd bit for bit like getOdd"""
     sizes = {}
     for kind in kinds:
         g, o = _sorted_rows(gpu.export_cloud(kind)), _sorted_rows(orc.export_cloud(kind))
@@ -67,6 +67,6 @@ def assert_cloud_parity(gpu, orc, kinds=(0, 1), heights=(0.75, 1.25), tag=""):
         oi = np.lexsort((o[:, 2], o[:, 1], o[:, 0]))
         g, o = g[gi], o[oi]
         assert np.array_equal(g[:, :3].view(np.uint32), o[:, :3].view(np.uint32)), (tag, "slice xyz", hgt)
-        assert np.abs(g[:, 3].astype(np.float64) - o[:, 3]).max(initial=0.0) <= 1.2e-7, (tag, "slice odd", hgt)
+        assert np.array_equal(g[:, 3].view(np.uint32), o[:, 3].view(np.uint32)), (tag, "slice odd", hgt)
         sizes[("slice", hgt)] = g.shape[0]
     return sizes

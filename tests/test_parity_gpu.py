@@ -7,6 +7,7 @@ import pytest
 from mlmapping_b200 import MLMap, config_cfg_a, config_cfg_c, scenes
 from mlmapping_b200.capi import MlmError
 from oracle_binding import best_oracle as Oracle  # the reference's own sources when oracle/_ref is there, else the restatement
+from grad_spec import odds
 from parity_utils import assert_cloud_parity, assert_frame_parity, assert_map_parity
 
 pytestmark = pytest.mark.gpu
@@ -122,13 +123,13 @@ def test_queries_and_set_free():
     pos = np.concatenate([pos, lattice, -lattice[:100]])
     assert np.array_equal(gpu.getOccupancy(pos), orc.getOccupancy(pos))
     og, oo = gpu.getOdd(pos), orc.getOdd(pos)
-    assert np.abs(og.astype(np.float64) - oo.astype(np.float64)).max() <= 1.2e-7  # <= 1 float ulp of odds in [0.5,1]
+    assert np.array_equal(og.view(np.uint32), oo.view(np.uint32))
     gg, go = gpu.getOddGrad(pos[:100000]), orc.getOddGrad(pos[:100000])
-    assert np.abs(gg - go).max() <= 1e-6
+    assert np.array_equal(gg.view(np.uint64), go.view(np.uint64))
     # one-step walks, walks that stay inside a subbox less often, and walks longer than a subbox (several borders crossed)
     for it in (1, 3, cfg.subbox_n + 3, 2 * cfg.subbox_n + 1):
         q = pos[100000:140000]
-        assert np.abs(gpu.getOddGrad(q, it) - orc.getOddGrad(q, it)).max() <= 1e-6, it
+        assert np.array_equal(gpu.getOddGrad(q, it).view(np.uint64), orc.getOddGrad(q, it).view(np.uint64)), it
     assert np.array_equal(gpu.getOccupancy(pos[:50000], 0.15), orc.getOccupancy(pos[:50000], 0.15))
     # setFree_map_in_bound, then everything again
     bmin, bmax = [5.0, -0.5, 0.3], [8.0, 0.5, 2.0]
@@ -317,8 +318,8 @@ def test_exploration_frontiers_and_memory_release(one_launch, monkeypatch):
     hi = (m["glb"].max(0) + 1) * 1.0
     pos = scenes.query_positions(200000, lo, hi, seed=9, inflate=1.0)
     assert np.array_equal(gpu.getOccupancy(pos), orc.getOccupancy(pos))
-    assert np.abs(gpu.getOdd(pos).astype(np.float64) - orc.getOdd(pos)).max() <= 1.2e-7
-    assert np.abs(gpu.getOddGrad(pos[:50000]) - orc.getOddGrad(pos[:50000])).max() <= 1e-6
+    assert np.array_equal(gpu.getOdd(pos).view(np.uint32), orc.getOdd(pos).view(np.uint32))
+    assert np.array_equal(gpu.getOddGrad(pos[:50000]).view(np.uint64), orc.getOddGrad(pos[:50000]).view(np.uint64))
     # box fill and inflation must skip collapsed subboxes like the reference
     gpu.setFree_map_in_bound([5.0, -1.0, 0.2], [9.0, 1.0, 2.2])
     orc.setFree_map_in_bound([5.0, -1.0, 0.2], [9.0, 1.0, 2.2])
@@ -665,15 +666,15 @@ def test_get_odd_by_subbox_index():
     glb[:200] += 1000                      # absent subboxes -> 0.5
     sub = rs.randint(0, 1000, 4000).astype(np.int32)
     got = gpu.getOdd_at(glb, sub)
-    lo = np.where(m["collapsed"][sel] == 1, m["log_odds"][sel, 0], m["log_odds"][sel, sub]).astype(np.float64)
-    want = (np.power(10.0, lo) / (1 + np.power(10.0, lo)))
+    lo = np.where(m["collapsed"][sel] == 1, m["log_odds"][sel, 0], m["log_odds"][sel, sub])
+    want = odds(lo)   # glibc's pow, like the reference
     want[:200] = 0.5
-    assert m["collapsed"].sum() > 0 and np.abs(got.astype(np.float64) - want).max() <= 1.2e-7
+    assert m["collapsed"].sum() > 0 and np.array_equal(got.view(np.uint32), want.view(np.uint32))
     if getattr(orc, "impl", "port") == "reference":   # the reference's own overload
         ref = np.empty(4000, dtype=np.float32)
         g32 = np.ascontiguousarray(glb.astype(np.int32))
         orc.lib.orc_get_odd_at(orc.h, g32.ctypes.data, sub.ctypes.data, 4000, ref.ctypes.data)
-        assert np.abs(got.astype(np.float64) - ref).max() <= 1.2e-7
+        assert np.array_equal(got.view(np.uint32), ref.view(np.uint32))
 
 
 def test_asynchronous_frames_of_several_maps_on_one_gpu():

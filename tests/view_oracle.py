@@ -52,7 +52,7 @@ def load():
     lib.orc_cast_rays.argtypes = [vp, vp, vp, sz, C.c_int, vp]
     lib.orc_view_gain.argtypes = [vp, vp, sz, C.POINTER(ViewSensor), vp, C.c_int, vp, vp]
     lib.orc_view_gain.restype = C.c_int
-    lib.orc_view_set_map.argtypes = [vp, sz, vp, vp, vp, vp, vp]
+    lib.orc_view_set_map.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp]
     lib.orc_view_set_map.restype = None
     _lib = lib
     return lib
@@ -89,11 +89,15 @@ class ViewOracle(RayOracle):
         return out
 
     def set_map(self, ex):
-        """replace the map with the subboxes of an export-like dict (glb, collapsed, occupancy, inflate, frontier bytes)"""
+        """replace the map with the subboxes of an export-like dict (glb, collapsed, occupancy, inflate, frontier bytes and,
+        when it has them, log_odds; else every log-odds is 0)"""
         glb = np.ascontiguousarray(ex["glb"], dtype=np.int32)
         col = np.ascontiguousarray(ex["collapsed"], dtype=np.uint8)
         occ = np.ascontiguousarray(ex["occupancy"]).view(np.uint8)
         inf = np.ascontiguousarray(ex["inflate"]).view(np.uint8)
         fr = np.ascontiguousarray(ex["frontier"], dtype=np.uint8)
+        lo = None if "log_odds" not in ex else np.ascontiguousarray(ex["log_odds"], dtype=np.float32)
+        if lo is not None:
+            assert lo.shape == (glb.shape[0], self.cells), lo.shape
         self.lib.orc_view_set_map(self.h, glb.shape[0], glb.ctypes.data, col.ctypes.data, occ.ctypes.data,
-                                  inf.ctypes.data, fr.ctypes.data)
+                                  inf.ctypes.data, fr.ctypes.data, None if lo is None else lo.ctypes.data)

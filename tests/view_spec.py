@@ -184,8 +184,8 @@ def candidates_around(centroids, T_bs7, seed, per_cluster=8, r_lo=1.0, r_hi=3.0)
 # ---- checkpoint images of arbitrary maps --------------------------------------------------------------------------
 def write_map_checkpoint(template: bytes, cfg, ex) -> bytes:
     """a checkpoint image with the template's header (a fresh exploration handle's) and one record per subbox of the
-    export-like dict ex: occupancy and inflation bytes per cell, collapsed flags (element 0 kept), frontier bytes;
-    log-odds 0.  n_records, n_submaps and the checksum are fixed."""
+    export-like dict ex: occupancy and inflation bytes per cell, collapsed flags (element 0 kept), frontier bytes, and
+    the log-odds of ex["log_odds"] when it has them (else 0).  n_records, n_submaps and the checksum are fixed."""
     hd = CkptHeader.from_buffer_copy(template[:C.sizeof(CkptHeader)])
     n = cfg.subbox_n
     cells, fw = n ** 3, (n ** 3 + 31) // 32
@@ -196,14 +196,17 @@ def write_map_checkpoint(template: bytes, cfg, ex) -> bytes:
     col = np.asarray(ex["collapsed"], dtype=bool)
     occ = np.asarray(ex["occupancy"]).view(np.uint8).reshape(m, cells)
     inf = np.asarray(ex["inflate"]).view(np.uint8).reshape(m, cells)
+    lo = np.zeros((m, cells), np.float32) if "log_odds" not in ex else np.asarray(ex["log_odds"], np.float32)
+    assert lo.shape == (m, cells), lo.shape
     recs = np.zeros((m, rb), dtype=np.uint8)
     head = np.zeros(m, dtype=[("g", "<i4", (3,)), ("flags", "<i4"), ("col_lo", "<f4"), ("col_occ", "u1"),
                               ("col_inf", "u1"), ("pad", "S10")])
     head["g"] = glb
     head["flags"] = col.astype(np.int32)
-    head["col_occ"], head["col_inf"] = occ[:, 0], inf[:, 0]
+    head["col_lo"], head["col_occ"], head["col_inf"] = lo[:, 0], occ[:, 0], inf[:, 0]
     recs[:, :32] = head.view(np.uint8).reshape(m, 32)
     full = ~col
+    recs[full, 32:32 + 4 * cells] = lo[full].astype("<f4").view(np.uint8).reshape(-1, 4 * cells)
     recs[full, 32 + 4 * cells:32 + 5 * cells] = occ[full]
     recs[full, 32 + 5 * cells:32 + 6 * cells] = inf[full]
     fr = np.zeros((m, 4 * fw), dtype=np.uint8)
