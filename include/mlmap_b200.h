@@ -365,6 +365,62 @@ int mlm_view_gain(mlm_handle h, const double *T_wb /* n x 7 */, size_t n, const 
 int mlm_view_gain_device(mlm_handle h, const double *d_T_wb, size_t n, const mlm_view_sensor *sensor,
                          const int32_t *d_boxes /* may be NULL */, int flags, mlm_view_gain_record *d_out);
 
+/* Reachability field over a box of the map (no reference counterpart; the third step of a frontier-based explorer's
+ * planning cycle, which ranks viewpoints by gain over the cost of travelling there): the exact shortest-path cost from a
+ * set of start cells through traversable cells, with batched cost queries and shortest paths.  Costs are integers, so
+ * the field does not depend on the order anything is computed in.
+ *  1. Box: the distance-field spec's rule 1 and its limits: lo_k = cell(box_min_k), hi_k = cell(box_max_k) (the ray
+ *     spec's rule 1), N_k = hi_k - lo_k + 1; MLM_ERR_CAPACITY for N_k > 4096 or more than 2^28 cells.
+ *  2. Traversable set T: the cells of the box whose state under the ray spec's rule 3 is FREE (an absent subbox is
+ *     unknown, a collapsed one takes its element 0).  With MLM_REACH_INFLATED a cell that blocks by inflation is
+ *     excluded, as for MLM_RAY_INFLATED (a collapsed subbox never blocks by inflation).  With MLM_REACH_UNKNOWN the
+ *     UNKNOWN cells (neither free nor occupied) are traversable too (the optimistic mode of grid planners).  Cells
+ *     outside the box are never in T.
+ *  3. Sources S: cell(starts[i]) for the n_starts >= 1 points; a start whose cell fails rule 1 or lies outside the box
+ *     is ignored.  A start cell inside the box is a source of cost 0 whatever its state, and counts as traversable (the
+ *     robot's own cell is often in the inflation layer or unknown).  *n_sources (may be NULL) = the number of distinct
+ *     source cells; it is computed on the host, so the call does not synchronise.
+ *  4. Moves: from a to b = a + d, d in {-1, 0, 1}^3 \ {0}.  A move is allowed when every cell a + d' with d'_k in {0, d_k}
+ *     is in T or S: the 1x1x2, 1x2x2 or 2x2x2 block a and b span, so a move never cuts a corner (the rule is symmetric in
+ *     a and b).  Its cost w(d) by the number of non-zero components: 1000, 1414, 1732 (floor(1000 sqrt(k))).
+ *  5. Field: cost(c) = the minimum over move sequences from any source to c of the summed move costs, an exact integer.
+ *     The budget is K = (int64)floor((max_dist / d_sub) * 1000.0) in IEEE double; a cell without a path, or whose
+ *     minimum exceeds K, is unreachable.
+ *  6. Cost query at p: the quiet NaN 0x7ff8000000000000 when cell(p) fails rule 1 or lies outside the box; +inf when
+ *     the cell is unreachable; else ((double)cost / 1000.0) * d_sub, each operation correctly rounded.
+ *  7. Path to goal g, c = cell(g): length -2 when c fails rule 1 or lies outside the box, -1 when it is unreachable.
+ *     Otherwise the path starts at c; while cost(c) > 0 the next cell is p = c + d for the first d in lexicographic
+ *     order of (dz, dy, dx) (z slowest, each -1, 0, 1) such that p is in the box and reachable, the move p -> c is
+ *     allowed, and cost(p) + w(d) == cost(c).  Such a p always exists; the path ends at a source.  Cells are written
+ *     goal first as int32 triples, at most max_cells per goal at cells3[(i * max_cells + j) * 3 ...]; len[i] = the full
+ *     length L, which may exceed max_cells (as mlm_export_cloud's n_out), L <= cost / 1000 + 1.
+ *  8. Lifetime: the field is a snapshot of the map at mlm_reach_build, in stream order; later frames, inflate_map,
+ *     set_free_in_bound or a checkpoint restore leave it as it is until the next build.  Querying or exporting before
+ *     any build returns MLM_ERR_INVALID_ARG, and so does querying after a build that failed once it had started work on
+ *     the device (MLM_ERR_CUDA): the earlier field is gone.  A build refused for its arguments keeps the earlier field.
+ * mlm_reach_build and the _device calls only enqueue on the handle's stream; the host variants stage through it and
+ * return when the data is in place.  MLM_ERR_INVALID_ARG: null handle; null box or starts; n_starts == 0; a null
+ * pointer with a non-zero count (cells3 when n * max_cells > 0); flags outside MLM_REACH_INFLATED | MLM_REACH_UNKNOWN;
+ * max_dist not finite or <= 0; a box corner that fails rule 1; box_min > box_max on an axis.  MLM_ERR_CAPACITY: the
+ * box limits of rule 1, or K > 2^30 (sums stay in int32).  A rank of a sharded map with world > 1 returns
+ * MLM_ERR_UNSUPPORTED like mlm_cast_rays.  The buffers belong to the handle: allocated by the first build, grown for a
+ * larger box, freed by mlm_destroy.
+ * mlm_reach_export writes cost(c) as int32, -1 where unreachable, x fastest as mlm_esdf_export: index
+ * (z * N_y + y) * N_x + x, x = c_x - lo_x...; lo3 and dims3 are always filled; out may be NULL with cap 0 to ask for the
+ * size; cap < N_x * N_y * N_z returns MLM_ERR_CAPACITY. */
+#define MLM_REACH_INFLATED 1 /* cells that block by inflation are not traversable */
+#define MLM_REACH_UNKNOWN 2  /* UNKNOWN cells are traversable */
+int mlm_reach_build(mlm_handle h, const double box_min[3], const double box_max[3], const double *starts /* n x 3 */,
+                    size_t n_starts, double max_dist, int flags, int32_t *n_sources /* may be NULL */);
+int mlm_reach_cost(mlm_handle h, const double *pos, size_t n, double *out);
+int mlm_reach_cost_device(mlm_handle h, const double *d_pos, size_t n, double *d_out);
+int mlm_reach_paths(mlm_handle h, const double *goals, size_t n, size_t max_cells, int32_t *cells3 /* n*max_cells*3 */,
+                    int32_t *len /* n */);
+int mlm_reach_paths_device(mlm_handle h, const double *d_goals, size_t n, size_t max_cells, int32_t *d_cells3,
+                           int32_t *d_len);
+int mlm_reach_export(mlm_handle h, int32_t *out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
+int mlm_reach_export_device(mlm_handle h, int32_t *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
+
 /* ---- stream control / timing (CUDA events on the handle's own stream) ------------------------- */
 
 int mlm_sync(mlm_handle h);

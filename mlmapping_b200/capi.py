@@ -128,6 +128,7 @@ FRONTIER_CLUSTER_DTYPE = np.dtype([("n_cells", "<i4"), ("key", "<i4", (3,)), ("l
                                    ("centroid", "<f8", (3,))])
 
 VIEW_FRONTIER, VIEW_INFLATED, VIEW_INVALID = 1, 2, -2  # MLM_VIEW_FRONTIER, MLM_VIEW_INFLATED, MLM_VIEW_INVALID
+REACH_INFLATED, REACH_UNKNOWN = 1, 2  # MLM_REACH_INFLATED, MLM_REACH_UNKNOWN
 
 
 class ViewSensor(C.Structure):
@@ -164,6 +165,8 @@ ABI_SYMBOLS = [
     "mlm_esdf_build", "mlm_esdf_distance", "mlm_esdf_distance_device", "mlm_esdf_export", "mlm_esdf_export_device",
     "mlm_frontier_clusters", "mlm_frontier_clusters_device", "mlm_sizeof_frontier_cluster",
     "mlm_view_gain", "mlm_view_gain_device", "mlm_sizeof_view_gain",
+    "mlm_reach_build", "mlm_reach_cost", "mlm_reach_cost_device", "mlm_reach_paths", "mlm_reach_paths_device",
+    "mlm_reach_export", "mlm_reach_export_device",
 ]
 FRAME_KERNELS = ["k_project", "k_column", "k_fuse"]
 
@@ -233,6 +236,13 @@ def load_library() -> C.CDLL:
         "mlm_view_gain": ([vp, vp, sz, C.POINTER(ViewSensor), vp, C.c_int, vp], C.c_int),
         "mlm_view_gain_device": ([vp, vp, sz, C.POINTER(ViewSensor), vp, C.c_int, vp], C.c_int),
         "mlm_sizeof_view_gain": ([], C.c_size_t),
+        "mlm_reach_build": ([vp, dp, dp, vp, sz, C.c_double, C.c_int, ip], C.c_int),
+        "mlm_reach_cost": ([vp, vp, sz, vp], C.c_int),
+        "mlm_reach_cost_device": ([vp, vp, sz, vp], C.c_int),
+        "mlm_reach_paths": ([vp, vp, sz, sz, vp, vp], C.c_int),
+        "mlm_reach_paths_device": ([vp, vp, sz, sz, vp, vp], C.c_int),
+        "mlm_reach_export": ([vp, vp, sz, ip, ip], C.c_int),
+        "mlm_reach_export_device": ([vp, vp, sz, ip, ip], C.c_int),
         "mlm_sync": ([vp], C.c_int),
         "mlm_timer_start": ([vp], C.c_int),
         "mlm_timer_stop_ms": ([vp, fp], C.c_int),
@@ -672,6 +682,58 @@ class MLMap:
         """the same on device memory (n x 7 doubles, n x 6 int32 boxes or 0, n 16-byte records); only enqueues"""
         self._check(self._lib.mlm_view_gain_device(self._h, d_poses, n, C.byref(sensor), d_boxes or None,
                                                    self._view_flags(frontier, inflated), d_out))
+
+    # ---- reachability field over a box (no reference counterpart; spec in include/mlmap_b200.h) ---------------
+    def build_reach(self, box_min, box_max, starts, max_dist: float, inflated: bool = False, unknown: bool = False) -> int:
+        """exact 26-connected shortest-path costs from the cells of `starts` ((n,3) world points) through the box's free
+        cells (inflated: not the inflation layer; unknown: unknown cells too), moves never cutting a corner, up to
+        max_dist; a snapshot of the map until the next build.  Returns the number of distinct source cells."""
+        a = (C.c_double * 3)(*[float(v) for v in np.asarray(box_min, dtype=np.float64).reshape(3)])
+        b = (C.c_double * 3)(*[float(v) for v in np.asarray(box_max, dtype=np.float64).reshape(3)])
+        s = self._pos(starts)
+        n = C.c_int32()
+        flags = (REACH_INFLATED if inflated else 0) | (REACH_UNKNOWN if unknown else 0)
+        self._check(self._lib.mlm_reach_build(self._h, a, b, s.ctypes.data, s.shape[0], float(max_dist), flags, C.byref(n)))
+        return n.value
+
+    def reach_cost(self, pos_w) -> np.ndarray:
+        """path cost in metres at (n,3) world points: +inf where unreachable, NaN outside the box"""
+        p = self._pos(pos_w)
+        out = np.empty(p.shape[0], dtype=np.float64)
+        self._check(self._lib.mlm_reach_cost(self._h, p.ctypes.data, p.shape[0], out.ctypes.data))
+        return out
+
+    def reach_cost_device(self, d_pos: int, n: int, d_out: int):
+        """the same on device memory (n x 3 doubles in, n doubles out); only enqueues"""
+        self._check(self._lib.mlm_reach_cost_device(self._h, d_pos, n, d_out))
+
+    def reach_paths(self, goals, max_cells: int):
+        """shortest paths from each goal back to a source: (cells[n, max_cells, 3] int32, goal first, len[n] int32 = the
+        full length, which may exceed max_cells; -1 unreachable, -2 outside the box)"""
+        g = self._pos(goals)
+        n = g.shape[0]
+        cells = np.zeros((n, max_cells, 3), dtype=np.int32)
+        ln = np.empty(n, dtype=np.int32)
+        self._check(self._lib.mlm_reach_paths(self._h, g.ctypes.data, n, max_cells, cells.ctypes.data, ln.ctypes.data))
+        return cells, ln
+
+    def reach_paths_device(self, d_goals: int, n: int, max_cells: int, d_cells3: int, d_len: int):
+        """the same on device memory (n x 3 doubles, n * max_cells * 3 and n int32); only enqueues"""
+        self._check(self._lib.mlm_reach_paths_device(self._h, d_goals, n, max_cells, d_cells3 or None, d_len))
+
+    def export_reach(self):
+        """(grid[N_z, N_y, N_x] int32, lo[3] int32): the costs of the last build, -1 where unreachable"""
+        lo, dims = (C.c_int32 * 3)(), (C.c_int32 * 3)()
+        self._check(self._lib.mlm_reach_export(self._h, None, 0, lo, dims))
+        out = np.empty((dims[2], dims[1], dims[0]), dtype=np.int32)
+        self._check(self._lib.mlm_reach_export(self._h, out.ctypes.data, out.size, lo, dims))
+        return out, np.array(lo[:], dtype=np.int32)
+
+    def export_reach_device(self, d_out: int, cap: int):
+        """the grid into device memory of cap int32 (only enqueues): (lo[3], dims[3] = N_x, N_y, N_z)"""
+        lo, dims = (C.c_int32 * 3)(), (C.c_int32 * 3)()
+        self._check(self._lib.mlm_reach_export_device(self._h, d_out or None, cap, lo, dims))
+        return np.array(lo[:], dtype=np.int32), np.array(dims[:], dtype=np.int32)
 
     # ---- stream / timing -------------------------------------------------------------------------
     def sync(self):

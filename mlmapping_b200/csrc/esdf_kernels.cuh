@@ -3,8 +3,9 @@
 // grid and the queries agree bit for bit.
 //
 // Build, four launches on the handle's stream:
-//   k_esdf_gather   one CTA per subbox meeting the box: one hash probe, then the blocking byte of each of its cells in the
-//                   box, read through the ray walk's SubboxView (the same blocking rule)
+//   k_esdf_gather   one CTA per subbox meeting the box: one hash probe, then the class byte (free / blocking / unknown) of
+//                   each of its cells in the box, read through the ray walk's SubboxView (the same blocking rule); the
+//                   reachability field (reach_kernels.cuh) builds on the same bytes
 //   k_esdf_x        one CTA per x line, staged in shared memory: 1-D distance to the nearest blocking and non-blocking
 //                   cell of the line (prefix scans of the last / first index), squared
 //   k_esdf_y        one thread per y line, threads over x: lower envelope of parabolas (Felzenszwalb-Huttenlocher), both
@@ -22,6 +23,8 @@ constexpr int kEsdfMaxAxis = 4096;             // N_k <= 4096
 constexpr long long kEsdfMaxCells = 1ll << 28; // N_x * N_y * N_z <= 2^28
 constexpr int kEsdfInf = 0x7fffffff;           // an empty set's squared distance
 constexpr int kEsdfLineThreads = 64;           // threads (x lines) per CTA of k_esdf_y / k_esdf_z
+// the class byte of a cell under the ray spec's rule 3: blocking, else FREE, else unknown
+constexpr uint8_t kCellFree = 0, kCellBlocking = 1, kCellUnknown = 2;
 
 struct EsdfGrid {
   int lo[3];        // first cell of the box
@@ -36,9 +39,9 @@ __device__ __forceinline__ size_t esdf_index(const EsdfGrid &G, int x, int y, in
   return ((size_t)z * G.dims[1] + y) * G.dims[0] + x;
 }
 
-// blk[cell] = 1 when the cell blocks (rule 2)
+// cls[cell] = kCellBlocking when the cell blocks (rule 2), else kCellFree / kCellUnknown by its state
 template <bool kInflated>
-__global__ void __launch_bounds__(256) k_esdf_gather(MapParams P, DeviceBuffers D, EsdfGrid G, uint8_t *blk) {
+__global__ void __launch_bounds__(256) k_esdf_gather(MapParams P, DeviceBuffers D, EsdfGrid G, uint8_t *cls) {
   __shared__ SubboxView s_view;
   const int b = blockIdx.x;
   const int g[3] = {G.glo[0] + b % G.gdims[0], G.glo[1] + (b / G.gdims[0]) % G.gdims[1],
@@ -59,7 +62,8 @@ __global__ void __launch_bounds__(256) k_esdf_gather(MapParams P, DeviceBuffers 
     const int x = c0[0] + t % len[0], y = c0[1] + (t / len[0]) % len[1], z = c0[2] + t / (len[0] * len[1]);
     const int sub = ((z - g[2] * n) * n + (y - g[1] * n)) * n + (x - g[0] * n);
     char st;
-    blk[esdf_index(G, x - G.lo[0], y - G.lo[1], z - G.lo[2])] = view_blocks<kInflated>(v, sub, st) ? 1 : 0;
+    const bool b = view_blocks<kInflated>(v, sub, st);
+    cls[esdf_index(G, x - G.lo[0], y - G.lo[1], z - G.lo[2])] = b ? kCellBlocking : (st == 'f' ? kCellFree : kCellUnknown);
   }
 }
 
@@ -72,7 +76,7 @@ __global__ void __launch_bounds__(256) k_esdf_x(EsdfGrid G, const uint8_t *blk, 
   __shared__ int s_scan[4][256];
   const int nx = G.dims[0], t = threadIdx.x;
   const size_t row = (size_t)blockIdx.x * nx;
-  for (int x = t; x < nx; x += 256) s_blk[x] = blk[row + x];
+  for (int x = t; x < nx; x += 256) s_blk[x] = blk[row + x] == kCellBlocking;
   __syncthreads();
   const int per = (nx + 255) / 256, x0 = t * per, x1 = min(x0 + per, nx);
   const int kNone = 1 << 30;

@@ -28,6 +28,7 @@
 #include "esdf_kernels.cuh"
 #include "frontier_kernels.cuh"
 #include "view_kernels.cuh"
+#include "reach_kernels.cuh"
 
 using namespace mlm;
 
@@ -280,6 +281,13 @@ struct mlm_map {
   ViewSetup *view_setup = nullptr;
   unsigned long long *view_tiles = nullptr;
   size_t view_cap = 0;
+  // reachability field (mlm_reach_*): class bytes and costs of reach_cap_cells cells, worklists of reach_cap_tiles tiles,
+  // grown by a larger box; reach_grid is the box of the last build
+  uint8_t *reach_cls = nullptr;
+  int *reach_cost = nullptr, *reach_mark = nullptr, *reach_list = nullptr, *reach_ctl = nullptr;
+  size_t reach_cap_cells = 0, reach_cap_tiles = 0;
+  bool reach_built = false;
+  ReachGrid reach_grid = {};
 };
 
 namespace {
@@ -1388,6 +1396,7 @@ int mlm_create(const mlm_config *cfg, int device, mlm_handle *out) {
 static void esdf_free(mlm_handle h);
 static void frontier_free(mlm_handle h);
 static void view_free(mlm_handle h);
+static void reach_free(mlm_handle h);
 
 int mlm_destroy(mlm_handle h) {
   if (!h) return MLM_ERR_INVALID_ARG;
@@ -1405,6 +1414,7 @@ int mlm_destroy(mlm_handle h) {
   esdf_free(h);
   frontier_free(h);
   view_free(h);
+  reach_free(h);
   if (h->d_input) cudaFree(h->d_input);
   if (h->h_stage) cudaFreeHost(h->h_stage);
   if (h->l2_buf) cudaFree(h->l2_buf);
@@ -1864,24 +1874,19 @@ static void esdf_free(mlm_handle h) {
   h->esdf_built = false;
 }
 
-int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3], double max_dist, int flags) {
-  if (!h) return MLM_ERR_INVALID_ARG;
-  if (!box_min || !box_max || (flags != 0 && flags != MLM_ESDF_INFLATED) || !std::isfinite(max_dist) || !(max_dist > 0)) {
-    g_last_error = "mlm_esdf_build: null box, flags other than 0 / MLM_ESDF_INFLATED, or max_dist not finite and > 0";
-    return MLM_ERR_INVALID_ARG;
-  }
-  int rc = refuse_sharded(h, "mlm_esdf_build");
-  if (rc != MLM_OK) return rc;
-  EsdfGrid G = {};
+// rule 1 of the distance-field spec and its limits (the reachability field shares them): the box's cells, the subboxes
+// meeting it and d_sub into G, the number of cells into `cells`
+static int esdf_box(mlm_handle h, const double box_min[3], const double box_max[3], const char *fn, EsdfGrid &G,
+                    long long &cells) {
   const int n = h->P.n;
-  long long cells = 1;
+  cells = 1;
   for (int k = 0; k < 3; k++) {
     int lo, hi;
-    rc = box_axis_cells(h, box_min[k], box_max[k], "mlm_esdf_build", &lo, &hi);
+    const int rc = box_axis_cells(h, box_min[k], box_max[k], fn, &lo, &hi);
     if (rc != MLM_OK) return rc;
     const long long nk = (long long)hi - lo + 1;
     if (nk > kEsdfMaxAxis) {
-      g_last_error = "mlm_esdf_build: more than 4096 cells along an axis";
+      g_last_error = std::string(fn) + ": more than 4096 cells along an axis";
       return MLM_ERR_CAPACITY;
     }
     cells *= nk;
@@ -1891,10 +1896,25 @@ int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3
     G.gdims[k] = host_floor_div(hi, n) - G.glo[k] + 1;
   }
   if (cells > kEsdfMaxCells) {
-    g_last_error = "mlm_esdf_build: more than 2^28 cells in the box";
+    g_last_error = std::string(fn) + ": more than 2^28 cells in the box";
     return MLM_ERR_CAPACITY;
   }
   G.d = h->P.d_sub;
+  return MLM_OK;
+}
+
+int mlm_esdf_build(mlm_handle h, const double box_min[3], const double box_max[3], double max_dist, int flags) {
+  if (!h) return MLM_ERR_INVALID_ARG;
+  if (!box_min || !box_max || (flags != 0 && flags != MLM_ESDF_INFLATED) || !std::isfinite(max_dist) || !(max_dist > 0)) {
+    g_last_error = "mlm_esdf_build: null box, flags other than 0 / MLM_ESDF_INFLATED, or max_dist not finite and > 0";
+    return MLM_ERR_INVALID_ARG;
+  }
+  int rc = refuse_sharded(h, "mlm_esdf_build");
+  if (rc != MLM_OK) return rc;
+  EsdfGrid G = {};
+  long long cells = 0;
+  rc = esdf_box(h, box_min, box_max, "mlm_esdf_build", G, cells);
+  if (rc != MLM_OK) return rc;
   G.max_dist = max_dist;
   CUDA_TRY(cudaSetDevice(h->device));
   if ((size_t)cells > h->esdf_cap) {
@@ -1996,6 +2016,242 @@ int mlm_esdf_export(mlm_handle h, float *out, size_t cap, int32_t lo3[3], int32_
     CUDA_TRY(d_out.alloc(cells));
     esdf_export_launch(h, cells, d_out);
     CUDA_TRY(cudaMemcpyAsync(out, d_out, cells * sizeof(float), cudaMemcpyDeviceToHost, h->stream));
+  }
+  CUDA_TRY(cudaStreamSynchronize(h->stream));
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+// ---- reachability field (reach_kernels.cuh) ------------------------------------------------------------------
+// a field is there to query / export
+static int reach_ready(mlm_handle h, const char *fn) {
+  const int rc = refuse_sharded(h, fn);
+  if (rc != MLM_OK) return rc;
+  if (!h->reach_built) {
+    g_last_error = std::string(fn) + ": no reachability field has been built (mlm_reach_build first)";
+    return MLM_ERR_INVALID_ARG;
+  }
+  return MLM_OK;
+}
+// class bytes and costs per cell; per tile the queue marks and two worklists; the three queue counts and the barrier
+static ScratchList reach_scratch(mlm_handle h, size_t cells, size_t tiles) {
+  return {{(void **)&h->reach_cls, cells}, {(void **)&h->reach_cost, cells * sizeof(int)},
+          {(void **)&h->reach_mark, tiles * sizeof(int)}, {(void **)&h->reach_list, 2 * tiles * sizeof(int)},
+          {(void **)&h->reach_ctl, 4 * sizeof(int)}};
+}
+static void reach_free(mlm_handle h) {
+  scratch_free(reach_scratch(h, 0, 0));
+  h->reach_cap_cells = h->reach_cap_tiles = 0;
+  h->reach_built = false;
+}
+
+int mlm_reach_build(mlm_handle h, const double box_min[3], const double box_max[3], const double *starts,
+                    size_t n_starts, double max_dist, int flags, int32_t *n_sources) {
+  if (!h) return MLM_ERR_INVALID_ARG;
+  if (!box_min || !box_max || !starts || n_starts == 0 || (flags & ~(MLM_REACH_INFLATED | MLM_REACH_UNKNOWN)) ||
+      !std::isfinite(max_dist) || !(max_dist > 0)) {
+    g_last_error = "mlm_reach_build: null box or starts, n_starts == 0, flags other than MLM_REACH_INFLATED | "
+                   "MLM_REACH_UNKNOWN, or max_dist not finite and > 0";
+    return MLM_ERR_INVALID_ARG;
+  }
+  int rc = refuse_sharded(h, "mlm_reach_build");
+  if (rc != MLM_OK) return rc;
+  ReachGrid R = {};
+  long long cells = 0;
+  rc = esdf_box(h, box_min, box_max, "mlm_reach_build", R.box, cells);
+  if (rc != MLM_OK) return rc;
+  const double d = h->P.d_sub;
+  const double K = std::floor((max_dist / d) * 1000.0);  // rule 5's budget
+  if (!(K <= (double)kReachMaxBudget)) {
+    g_last_error = "mlm_reach_build: the cost budget floor(max_dist / d_sub * 1000) exceeds 2^30";
+    return MLM_ERR_CAPACITY;
+  }
+  R.budget = (int)K;
+  R.flags = flags;
+  for (int k = 0; k < 3; k++) R.tiles[k] = (R.box.dims[k] + kReachTile - 1) / kReachTile;
+  const size_t tiles = (size_t)R.tiles[0] * R.tiles[1] * R.tiles[2];
+  // rule 3: the distinct source cells, as box-linear indices, found on the host
+  std::vector<int> src;
+  src.reserve(n_starts);
+  for (size_t i = 0; i < n_starts; i++) {
+    bool in = true;
+    int c[3] = {0, 0, 0};
+    for (int k = 0; k < 3 && in; k++) {
+      const double q = starts[3 * i + k] / d;
+      in = std::fabs(q) < 1073741824.0;
+      if (in) c[k] = (int)std::floor(q) - R.box.lo[k];
+      in = in && c[k] >= 0 && c[k] < R.box.dims[k];
+    }
+    if (in) src.push_back((c[2] * R.box.dims[1] + c[1]) * R.box.dims[0] + c[0]);
+  }
+  std::sort(src.begin(), src.end());
+  src.erase(std::unique(src.begin(), src.end()), src.end());
+  CUDA_TRY(cudaSetDevice(h->device));
+  // from here on the buffers change: a build that fails part way leaves no field rather than a mix of two builds
+  h->reach_built = false;
+  if ((size_t)cells > h->reach_cap_cells || tiles > h->reach_cap_tiles) {
+    const size_t cc = std::max((size_t)cells, h->reach_cap_cells), ct = std::max(tiles, h->reach_cap_tiles);
+    reach_free(h);
+    rc = scratch_alloc(reach_scratch(h, cc, ct), "mlm_reach_build: field buffers");
+    if (rc != MLM_OK) return rc;
+    h->reach_cap_cells = cc;
+    h->reach_cap_tiles = ct;
+  }
+  cudaStream_t s = h->stream;
+  const int subs = R.box.gdims[0] * R.box.gdims[1] * R.box.gdims[2];
+  if (flags & MLM_REACH_INFLATED) k_esdf_gather<true><<<subs, 256, 0, s>>>(h->P, h->D, R.box, h->reach_cls);
+  else k_esdf_gather<false><<<subs, 256, 0, s>>>(h->P, h->D, R.box, h->reach_cls);
+  h->launches++;
+  CUDA_TRY(cudaMemsetAsync(h->reach_cost, 0x7f, (size_t)cells * sizeof(int), s));  // kReachInf
+  CUDA_TRY(cudaMemsetAsync(h->reach_mark, 0, tiles * sizeof(int), s));
+  CUDA_TRY(cudaMemsetAsync(h->reach_ctl, 0, 4 * sizeof(int), s));
+  ReachWork W = {h->reach_mark, h->reach_list, h->reach_list + tiles, h->reach_ctl,
+                 reinterpret_cast<unsigned *>(h->reach_ctl + 3)};
+  if (!src.empty()) {
+    {
+      StreamTemp<int> d_src(s);
+      CUDA_TRY(d_src.alloc(src.size()));
+      CUDA_TRY(cudaMemcpyAsync(d_src, src.data(), src.size() * sizeof(int), cudaMemcpyHostToDevice, s));
+      k_reach_seed<<<grid_for(src.size(), 256), 256, 0, s>>>(R, d_src, (int)src.size(), h->reach_cls, h->reach_cost, W);
+    }
+    // as many CTAs as are resident at once, at most one per tile
+    int per_sm = 0;
+    CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_reach_solve, kReachThreads, 0));
+    const int G = (int)std::min<size_t>((size_t)h->sm_count * std::max(per_sm, 1), tiles);
+    const uint8_t *cls = h->reach_cls;
+    int *cost = h->reach_cost;
+    void *args[] = {&R, &cls, &cost, &W};
+    CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_reach_solve, dim3(G), dim3(kReachThreads), args, 0, s));
+    h->launches += 2;
+  }
+  CUDA_TRY(cudaGetLastError());
+  h->reach_grid = R;
+  h->reach_built = true;
+  if (n_sources) *n_sources = (int32_t)src.size();
+  return MLM_OK;
+}
+
+static void reach_cost_launch(mlm_handle h, const double *d_pos, size_t n, double *d_out) {
+  k_reach_cost<<<grid_for(n, 256), 256, 0, h->stream>>>(h->reach_grid, h->reach_cost, d_pos, n, d_out);
+  h->launches++;
+}
+int mlm_reach_cost_device(mlm_handle h, const double *d_pos, size_t n, double *d_out) {
+  if (!h || ((!d_pos || !d_out) && n)) return MLM_ERR_INVALID_ARG;
+  const int rc = reach_ready(h, "mlm_reach_cost");
+  if (rc != MLM_OK) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (n == 0) return MLM_OK;
+  reach_cost_launch(h, d_pos, n, d_out);
+  return MLM_OK;
+}
+// the host variant stages the points and costs through the handle's stream (like mlm_esdf_distance)
+int mlm_reach_cost(mlm_handle h, const double *pos, size_t n, double *out) {
+  if (!h || ((!pos || !out) && n)) return MLM_ERR_INVALID_ARG;
+  const int rc = reach_ready(h, "mlm_reach_cost");
+  if (rc != MLM_OK) return rc;
+  if (n == 0) return MLM_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  {
+    StreamTemp<double> d_buf(s);  // points, costs
+    CUDA_TRY(d_buf.alloc(n * 4));
+    CUDA_TRY(cudaMemcpyAsync(d_buf, pos, n * 24, cudaMemcpyHostToDevice, s));
+    reach_cost_launch(h, d_buf, n, d_buf + 3 * n);
+    CUDA_TRY(cudaMemcpyAsync(out, d_buf + 3 * n, n * 8, cudaMemcpyDeviceToHost, s));
+  }
+  CUDA_TRY(cudaStreamSynchronize(s));
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+static int reach_paths_check(mlm_handle h, const void *goals, size_t n, size_t max_cells, const void *cells3,
+                             const void *len) {
+  if (!h || ((!goals || !len) && n) || (!cells3 && n && max_cells)) return MLM_ERR_INVALID_ARG;
+  if (n && max_cells > ((size_t)1 << 62) / 12 / n) {
+    g_last_error = "mlm_reach_paths: n * max_cells * 3 cells overflow";
+    return MLM_ERR_INVALID_ARG;
+  }
+  return reach_ready(h, "mlm_reach_paths");
+}
+static void reach_paths_launch(mlm_handle h, const double *d_goals, size_t n, size_t max_cells, int32_t *d_cells3,
+                               int32_t *d_len) {
+  k_reach_paths<<<grid_for(n * 32, 256), 256, 0, h->stream>>>(h->reach_grid, h->reach_cls, h->reach_cost, d_goals, n,
+                                                             max_cells, d_cells3, d_len);
+  h->launches++;
+}
+int mlm_reach_paths_device(mlm_handle h, const double *d_goals, size_t n, size_t max_cells, int32_t *d_cells3,
+                           int32_t *d_len) {
+  const int rc = reach_paths_check(h, d_goals, n, max_cells, d_cells3, d_len);
+  if (rc != MLM_OK) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  if (n == 0) return MLM_OK;
+  reach_paths_launch(h, d_goals, n, max_cells, d_cells3, d_len);
+  return MLM_OK;
+}
+int mlm_reach_paths(mlm_handle h, const double *goals, size_t n, size_t max_cells, int32_t *cells3, int32_t *len) {
+  const int rc = reach_paths_check(h, goals, n, max_cells, cells3, len);
+  if (rc != MLM_OK) return rc;
+  if (n == 0) return MLM_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  {
+    StreamTemp<double> d_g(s);
+    StreamTemp<int32_t> d_o(s);  // lengths, cells
+    CUDA_TRY(d_g.alloc(n * 3));
+    CUDA_TRY(d_o.alloc(n + n * max_cells * 3));
+    CUDA_TRY(cudaMemcpyAsync(d_g, goals, n * 24, cudaMemcpyHostToDevice, s));
+    reach_paths_launch(h, d_g, n, max_cells, d_o + n, d_o);
+    CUDA_TRY(cudaMemcpyAsync(len, d_o, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (max_cells)
+      CUDA_TRY(cudaMemcpyAsync(cells3, d_o + n, n * max_cells * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+  }
+  CUDA_TRY(cudaStreamSynchronize(s));
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+// lo3 / dims3 always; the field when out has room for it (out == NULL with cap 0 asks for the size only)
+static int reach_export_check(mlm_handle h, const int32_t *out, size_t cap, int32_t lo3[3], int32_t dims3[3],
+                              size_t &cells) {
+  if (!h || !lo3 || !dims3) return MLM_ERR_INVALID_ARG;
+  const int rc = reach_ready(h, "mlm_reach_export");
+  if (rc != MLM_OK) return rc;
+  const EsdfGrid &G = h->reach_grid.box;
+  for (int k = 0; k < 3; k++) {
+    lo3[k] = G.lo[k];
+    dims3[k] = G.dims[k];
+  }
+  cells = (size_t)G.dims[0] * G.dims[1] * G.dims[2];
+  if (!out && cap == 0) return MLM_OK;
+  if (!out) return MLM_ERR_INVALID_ARG;
+  if (cap < cells) {
+    g_last_error = "mlm_reach_export: cap is smaller than N_x * N_y * N_z";
+    return MLM_ERR_CAPACITY;
+  }
+  return MLM_OK;
+}
+static void reach_export_launch(mlm_handle h, size_t cells, int32_t *d_out) {
+  k_reach_export<<<grid_for(cells, 256), 256, 0, h->stream>>>(h->reach_cost, cells, d_out);
+  h->launches++;
+}
+int mlm_reach_export_device(mlm_handle h, int32_t *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]) {
+  size_t cells = 0;
+  const int rc = reach_export_check(h, d_out, cap, lo3, dims3, cells);
+  if (rc != MLM_OK || !d_out) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  reach_export_launch(h, cells, d_out);
+  return MLM_OK;
+}
+int mlm_reach_export(mlm_handle h, int32_t *out, size_t cap, int32_t lo3[3], int32_t dims3[3]) {
+  size_t cells = 0;
+  const int rc = reach_export_check(h, out, cap, lo3, dims3, cells);
+  if (rc != MLM_OK || !out) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  {
+    StreamTemp<int32_t> d_out(h->stream);
+    CUDA_TRY(d_out.alloc(cells));
+    reach_export_launch(h, cells, d_out);
+    CUDA_TRY(cudaMemcpyAsync(out, d_out, cells * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
   }
   CUDA_TRY(cudaStreamSynchronize(h->stream));
   CUDA_TRY(cudaGetLastError());

@@ -9,6 +9,7 @@
 #include <cstddef>
 #include <cstdint>
 #include <algorithm>
+#include <array>
 #include <stdexcept>
 #include <string>
 #include <vector>
@@ -202,6 +203,38 @@ class mlmap {
   }
   void getEsdfs(const Vec3 *pos, size_t n, double *dist, Vec3 *grad = nullptr) {
     check(mlm_esdf_distance(h_, n ? pos->v : nullptr, n, dist, grad ? grad->v : nullptr), "mlm_esdf_distance");
+  }
+  // reachability field over a box (no reference counterpart; spec at mlm_reach_build): exact 26-connected path costs
+  // from the start cells, a snapshot of the map until the next build; returns the number of distinct source cells.
+  // getReachCost is +inf where unreachable, NaN outside the box; getReachPath returns the whole path, its cells goal first
+  // (empty when there is none); getReachPaths writes at most max_cells cells per goal with the full length in len
+  // (-1 / -2 as the spec), so len[i] > max_cells tells a truncated path
+  int buildReach(const Vec3 &min, const Vec3 &max, const Vec3 *starts, size_t n, double max_dist, bool inflated = false,
+                 bool unknown = false) {
+    int32_t ns = 0;
+    check(mlm_reach_build(h_, min.v, max.v, n ? starts->v : nullptr, n, max_dist,
+                          (inflated ? MLM_REACH_INFLATED : 0) | (unknown ? MLM_REACH_UNKNOWN : 0), &ns),
+          "mlm_reach_build");
+    return ns;
+  }
+  double getReachCost(const Vec3 &pos) {
+    double c;
+    check(mlm_reach_cost(h_, pos.v, 1, &c), "mlm_reach_cost");
+    return c;
+  }
+  void getReachCosts(const Vec3 *pos, size_t n, double *cost) {
+    check(mlm_reach_cost(h_, n ? pos->v : nullptr, n, cost), "mlm_reach_cost");
+  }
+  std::vector<std::array<int32_t, 3>> getReachPath(const Vec3 &goal) {
+    // the length first (no cells), then exactly that many cells
+    int32_t len = 0;
+    check(mlm_reach_paths(h_, goal.v, 1, 0, nullptr, &len), "mlm_reach_paths");
+    std::vector<std::array<int32_t, 3>> cells(len > 0 ? (size_t)len : 0);
+    if (!cells.empty()) check(mlm_reach_paths(h_, goal.v, 1, cells.size(), cells[0].data(), &len), "mlm_reach_paths");
+    return cells;
+  }
+  void getReachPaths(const Vec3 *goals, size_t n, size_t max_cells, int32_t *cells3, int32_t *len) {
+    check(mlm_reach_paths(h_, n ? goals->v : nullptr, n, max_cells, cells3, len), "mlm_reach_paths");
   }
 
   // frontier clustering (no reference counterpart; spec at mlm_frontier_clusters): the clusters with >= min_cells cells
