@@ -421,6 +421,33 @@ int mlm_reach_paths_device(mlm_handle h, const double *d_goals, size_t n, size_t
 int mlm_reach_export(mlm_handle h, int32_t *out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
 int mlm_reach_export_device(mlm_handle h, int32_t *d_out, size_t cap, int32_t lo3[3], int32_t dims3[3]);
 
+/* Path-cost matrix over a box of the map: the cost from each of n_starts starts to each of n_goals goals, the input of a
+ * tour over viewpoints (an asymmetric TSP over the current pose and one viewpoint per frontier cluster).
+ *  Definition: out[i * n_goals + j] is, bit for bit, what mlm_reach_cost returns at goals[j] after
+ *  mlm_reach_build(h, box_min, box_max, starts + 3 * i, 1, max_dist, flags).  Box, traversable set, moves, weights,
+ *  budget, NaN and +inf are rules 1-6 of the reachability field.  So:
+ *   - the matrix is not symmetric in general: a start cell is a source and traversable in its own row whatever its
+ *     state, but as a goal of another row it is reached only if it is in T;
+ *   - a row whose start fails rule 1 or lies outside the box has no source: +inf at the goals in the box, NaN elsewhere.
+ *  The call leaves the field of mlm_reach_build as it is (mlm_reach_cost, mlm_reach_paths and mlm_reach_export answer
+ *  from the last build as before) and needs no earlier build.  The rows are solved in batches of at most 2^28 field
+ *  cells (at least one row); the results do not depend on the batching.
+ * mlm_reach_matrix_device only enqueues on the handle's stream and finds each row's source cell on the device; the host
+ * variant stages through the stream and returns when out is filled.  The arguments are checked first; then
+ * n_starts == 0 or n_goals == 0 returns MLM_OK and does nothing.  MLM_ERR_INVALID_ARG: null handle; null box; a null
+ * pointer with a non-zero count (out when n_starts * n_goals > 0); n_starts * n_goals doubles overflowing size_t; and the
+ * argument errors of mlm_reach_build (flags, max_dist, box corners, box_min > box_max).  MLM_ERR_CAPACITY: the box
+ * limits of rule 1 and K > 2^30.  A rank of a sharded map with world > 1 returns MLM_ERR_UNSUPPORTED.  The scratch
+ * belongs to the handle, apart from the field's buffers: allocated by the first call, grown for larger needs, freed by
+ * mlm_destroy. */
+int mlm_reach_matrix(mlm_handle h, const double box_min[3], const double box_max[3],
+                     const double *starts /* n_starts x 3 */, size_t n_starts, const double *goals /* n_goals x 3 */,
+                     size_t n_goals, double max_dist, int flags /* MLM_REACH_INFLATED | MLM_REACH_UNKNOWN */,
+                     double *out /* n_starts x n_goals, row-major */);
+int mlm_reach_matrix_device(mlm_handle h, const double box_min[3], const double box_max[3], const double *d_starts,
+                            size_t n_starts, const double *d_goals, size_t n_goals, double max_dist, int flags,
+                            double *d_out);
+
 /* ---- stream control / timing (CUDA events on the handle's own stream) ------------------------- */
 
 int mlm_sync(mlm_handle h);

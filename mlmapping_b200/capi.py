@@ -166,7 +166,7 @@ ABI_SYMBOLS = [
     "mlm_frontier_clusters", "mlm_frontier_clusters_device", "mlm_sizeof_frontier_cluster",
     "mlm_view_gain", "mlm_view_gain_device", "mlm_sizeof_view_gain",
     "mlm_reach_build", "mlm_reach_cost", "mlm_reach_cost_device", "mlm_reach_paths", "mlm_reach_paths_device",
-    "mlm_reach_export", "mlm_reach_export_device",
+    "mlm_reach_export", "mlm_reach_export_device", "mlm_reach_matrix", "mlm_reach_matrix_device",
 ]
 FRAME_KERNELS = ["k_project", "k_column", "k_fuse"]
 
@@ -243,6 +243,8 @@ def load_library() -> C.CDLL:
         "mlm_reach_paths_device": ([vp, vp, sz, sz, vp, vp], C.c_int),
         "mlm_reach_export": ([vp, vp, sz, ip, ip], C.c_int),
         "mlm_reach_export_device": ([vp, vp, sz, ip, ip], C.c_int),
+        "mlm_reach_matrix": ([vp, dp, dp, vp, sz, vp, sz, C.c_double, C.c_int, vp], C.c_int),
+        "mlm_reach_matrix_device": ([vp, dp, dp, vp, sz, vp, sz, C.c_double, C.c_int, vp], C.c_int),
         "mlm_sync": ([vp], C.c_int),
         "mlm_timer_start": ([vp], C.c_int),
         "mlm_timer_stop_ms": ([vp, fp], C.c_int),
@@ -734,6 +736,34 @@ class MLMap:
         lo, dims = (C.c_int32 * 3)(), (C.c_int32 * 3)()
         self._check(self._lib.mlm_reach_export_device(self._h, d_out or None, cap, lo, dims))
         return np.array(lo[:], dtype=np.int32), np.array(dims[:], dtype=np.int32)
+
+    # ---- path-cost matrix over a box (no reference counterpart; spec in include/mlmap_b200.h) --------------------
+    @staticmethod
+    def _box3(box_min, box_max):
+        return tuple((C.c_double * 3)(*[float(v) for v in np.asarray(b, dtype=np.float64).reshape(3)])
+                     for b in (box_min, box_max))
+
+    def reach_matrix(self, box_min, box_max, starts, goals, max_dist: float, inflated: bool = False,
+                     unknown: bool = False) -> np.ndarray:
+        """(n_starts, n_goals) path costs in metres: row i is reach_cost(goals) after build_reach(box_min, box_max,
+        [starts[i]], max_dist, inflated, unknown) (+inf unreachable, NaN outside the box); the last build_reach field
+        is left as it is"""
+        a, b = self._box3(box_min, box_max)
+        s, g = self._pos(starts), self._pos(goals)
+        out = np.empty((s.shape[0], g.shape[0]), dtype=np.float64)
+        flags = (REACH_INFLATED if inflated else 0) | (REACH_UNKNOWN if unknown else 0)
+        self._check(self._lib.mlm_reach_matrix(self._h, a, b, s.ctypes.data, s.shape[0], g.ctypes.data, g.shape[0],
+                                               float(max_dist), flags, out.ctypes.data))
+        return out
+
+    def reach_matrix_device(self, box_min, box_max, d_starts: int, n_starts: int, d_goals: int, n_goals: int,
+                            max_dist: float, d_out: int, inflated: bool = False, unknown: bool = False):
+        """the same on device memory (n_starts x 3 and n_goals x 3 doubles in, n_starts x n_goals doubles out); only
+        enqueues"""
+        a, b = self._box3(box_min, box_max)
+        flags = (REACH_INFLATED if inflated else 0) | (REACH_UNKNOWN if unknown else 0)
+        self._check(self._lib.mlm_reach_matrix_device(self._h, a, b, d_starts or None, n_starts, d_goals or None,
+                                                      n_goals, float(max_dist), flags, d_out or None))
 
     # ---- stream / timing -------------------------------------------------------------------------
     def sync(self):

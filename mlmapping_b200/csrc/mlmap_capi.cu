@@ -288,6 +288,12 @@ struct mlm_map {
   size_t reach_cap_cells = 0, reach_cap_tiles = 0;
   bool reach_built = false;
   ReachGrid reach_grid = {};
+  // path-cost matrix (mlm_reach_matrix), apart from the field above: class bytes of mat_cap_cells cells; per field of a
+  // batch the costs (mat_cap_fcells cells in all), the queue marks and two worklists (mat_cap_items items in all) and the
+  // source cell (mat_cap_rows); the three queue counts and the barrier
+  uint8_t *mat_cls = nullptr;
+  int *mat_cost = nullptr, *mat_mark = nullptr, *mat_list = nullptr, *mat_src = nullptr, *mat_ctl = nullptr;
+  size_t mat_cap_cells = 0, mat_cap_fcells = 0, mat_cap_items = 0, mat_cap_rows = 0;
 };
 
 namespace {
@@ -1397,6 +1403,7 @@ static void esdf_free(mlm_handle h);
 static void frontier_free(mlm_handle h);
 static void view_free(mlm_handle h);
 static void reach_free(mlm_handle h);
+static void reach_matrix_free(mlm_handle h);
 
 int mlm_destroy(mlm_handle h) {
   if (!h) return MLM_ERR_INVALID_ARG;
@@ -1415,6 +1422,7 @@ int mlm_destroy(mlm_handle h) {
   frontier_free(h);
   view_free(h);
   reach_free(h);
+  reach_matrix_free(h);
   if (h->d_input) cudaFree(h->d_input);
   if (h->h_stage) cudaFreeHost(h->h_stage);
   if (h->l2_buf) cudaFree(h->l2_buf);
@@ -2045,6 +2053,23 @@ static void reach_free(mlm_handle h) {
   h->reach_built = false;
 }
 
+// rules 1 and 5 for a build or a matrix: the box, its tiles, the budget and the flags into R, the box's cells into `cells`
+static int reach_grid_of(mlm_handle h, const double box_min[3], const double box_max[3], double max_dist, int flags,
+                         const char *fn, ReachGrid &R, long long &cells) {
+  R = {};
+  const int rc = esdf_box(h, box_min, box_max, fn, R.box, cells);
+  if (rc != MLM_OK) return rc;
+  const double K = std::floor((max_dist / h->P.d_sub) * 1000.0);  // rule 5's budget
+  if (!(K <= (double)kReachMaxBudget)) {
+    g_last_error = std::string(fn) + ": the cost budget floor(max_dist / d_sub * 1000) exceeds 2^30";
+    return MLM_ERR_CAPACITY;
+  }
+  R.budget = (int)K;
+  R.flags = flags;
+  for (int k = 0; k < 3; k++) R.tiles[k] = (R.box.dims[k] + kReachTile - 1) / kReachTile;
+  return MLM_OK;
+}
+
 int mlm_reach_build(mlm_handle h, const double box_min[3], const double box_max[3], const double *starts,
                     size_t n_starts, double max_dist, int flags, int32_t *n_sources) {
   if (!h) return MLM_ERR_INVALID_ARG;
@@ -2056,19 +2081,11 @@ int mlm_reach_build(mlm_handle h, const double box_min[3], const double box_max[
   }
   int rc = refuse_sharded(h, "mlm_reach_build");
   if (rc != MLM_OK) return rc;
-  ReachGrid R = {};
+  ReachGrid R;
   long long cells = 0;
-  rc = esdf_box(h, box_min, box_max, "mlm_reach_build", R.box, cells);
+  rc = reach_grid_of(h, box_min, box_max, max_dist, flags, "mlm_reach_build", R, cells);
   if (rc != MLM_OK) return rc;
   const double d = h->P.d_sub;
-  const double K = std::floor((max_dist / d) * 1000.0);  // rule 5's budget
-  if (!(K <= (double)kReachMaxBudget)) {
-    g_last_error = "mlm_reach_build: the cost budget floor(max_dist / d_sub * 1000) exceeds 2^30";
-    return MLM_ERR_CAPACITY;
-  }
-  R.budget = (int)K;
-  R.flags = flags;
-  for (int k = 0; k < 3; k++) R.tiles[k] = (R.box.dims[k] + kReachTile - 1) / kReachTile;
   const size_t tiles = (size_t)R.tiles[0] * R.tiles[1] * R.tiles[2];
   // rule 3: the distinct source cells, as box-linear indices, found on the host
   std::vector<int> src;
@@ -2254,6 +2271,126 @@ int mlm_reach_export(mlm_handle h, int32_t *out, size_t cap, int32_t lo3[3], int
     CUDA_TRY(cudaMemcpyAsync(out, d_out, cells * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
   }
   CUDA_TRY(cudaStreamSynchronize(h->stream));
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+// ---- path-cost matrix (reach_kernels.cuh) --------------------------------------------------------------------------
+// at most this many field cells per solve launch (1 GiB of int32 costs), and at least one field
+constexpr long long kReachMatrixCells = 1ll << 28;
+
+static ScratchList reach_matrix_scratch(mlm_handle h, size_t cells, size_t fcells, size_t items, size_t rows) {
+  return {{(void **)&h->mat_cls, cells}, {(void **)&h->mat_cost, fcells * sizeof(int)},
+          {(void **)&h->mat_mark, items * sizeof(int)}, {(void **)&h->mat_list, 2 * items * sizeof(int)},
+          {(void **)&h->mat_src, rows * sizeof(int)}, {(void **)&h->mat_ctl, 4 * sizeof(int)}};
+}
+static void reach_matrix_free(mlm_handle h) {
+  scratch_free(reach_matrix_scratch(h, 0, 0, 0, 0));
+  h->mat_cap_cells = h->mat_cap_fcells = h->mat_cap_items = h->mat_cap_rows = 0;
+}
+
+// the arguments of both variants; R and cells describe the box when the call has work to do
+static int reach_matrix_check(mlm_handle h, const double box_min[3], const double box_max[3], const void *starts,
+                              size_t n_starts, const void *goals, size_t n_goals, double max_dist, int flags,
+                              const void *out, ReachGrid &R, long long &cells) {
+  if (!h) return MLM_ERR_INVALID_ARG;
+  if (!box_min || !box_max || (!starts && n_starts) || (!goals && n_goals) || (!out && n_starts && n_goals) ||
+      (flags & ~(MLM_REACH_INFLATED | MLM_REACH_UNKNOWN)) || !std::isfinite(max_dist) || !(max_dist > 0)) {
+    g_last_error = "mlm_reach_matrix: null box, a null pointer with a non-zero count, flags other than "
+                   "MLM_REACH_INFLATED | MLM_REACH_UNKNOWN, or max_dist not finite and > 0";
+    return MLM_ERR_INVALID_ARG;
+  }
+  if (n_starts && n_goals > SIZE_MAX / sizeof(double) / n_starts) {
+    g_last_error = "mlm_reach_matrix: n_starts * n_goals entries overflow";
+    return MLM_ERR_INVALID_ARG;
+  }
+  const int rc = refuse_sharded(h, "mlm_reach_matrix");
+  if (rc != MLM_OK) return rc;
+  return reach_grid_of(h, box_min, box_max, max_dist, flags, "mlm_reach_matrix", R, cells);
+}
+
+// one class gather, then per batch of fields: reset, seed, one cooperative solve, the batch's rows of the matrix
+static int reach_matrix_enqueue(mlm_handle h, const ReachGrid &R, long long cells, const double *d_starts,
+                                size_t n_starts, const double *d_goals, size_t n_goals, double *d_out) {
+  const size_t tiles = (size_t)R.tiles[0] * R.tiles[1] * R.tiles[2];
+  const size_t batch = std::min<size_t>(n_starts, (size_t)std::max<long long>(1, kReachMatrixCells / cells));
+  CUDA_TRY(cudaSetDevice(h->device));
+  const size_t need[4] = {(size_t)cells, batch * cells, batch * tiles, batch};
+  size_t *cap[4] = {&h->mat_cap_cells, &h->mat_cap_fcells, &h->mat_cap_items, &h->mat_cap_rows};
+  if (need[0] > *cap[0] || need[1] > *cap[1] || need[2] > *cap[2] || need[3] > *cap[3]) {
+    size_t grown[4];
+    for (int k = 0; k < 4; k++) grown[k] = std::max(need[k], *cap[k]);
+    reach_matrix_free(h);
+    const int rc = scratch_alloc(reach_matrix_scratch(h, grown[0], grown[1], grown[2], grown[3]),
+                                 "mlm_reach_matrix: scratch buffers");
+    if (rc != MLM_OK) return rc;
+    for (int k = 0; k < 4; k++) *cap[k] = grown[k];
+  }
+  cudaStream_t s = h->stream;
+  const int subs = R.box.gdims[0] * R.box.gdims[1] * R.box.gdims[2];
+  if (R.flags & MLM_REACH_INFLATED) k_esdf_gather<true><<<subs, 256, 0, s>>>(h->P, h->D, R.box, h->mat_cls);
+  else k_esdf_gather<false><<<subs, 256, 0, s>>>(h->P, h->D, R.box, h->mat_cls);
+  h->launches++;
+  int per_sm = 0;
+  CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_reach_matrix_solve, kReachThreads, 0));
+  for (size_t row0 = 0; row0 < n_starts; row0 += batch) {
+    const size_t nb = std::min(batch, n_starts - row0);
+    CUDA_TRY(cudaMemsetAsync(h->mat_cost, 0x7f, nb * cells * sizeof(int), s));  // kReachInf
+    CUDA_TRY(cudaMemsetAsync(h->mat_mark, 0, nb * tiles * sizeof(int), s));
+    CUDA_TRY(cudaMemsetAsync(h->mat_ctl, 0, 4 * sizeof(int), s));
+    ReachWork W = {h->mat_mark, h->mat_list, h->mat_list + nb * tiles, h->mat_ctl,
+                   reinterpret_cast<unsigned *>(h->mat_ctl + 3)};
+    k_reach_matrix_seed<<<grid_for(nb, 256), 256, 0, s>>>(R, d_starts + 3 * row0, (int)nb, (size_t)cells, (int)tiles,
+                                                          h->mat_src, h->mat_cost, W);
+    // as many CTAs as are resident at once, at most one per work item
+    const int G = (int)std::min<size_t>((size_t)h->sm_count * std::max(per_sm, 1), nb * tiles);
+    ReachGrid Rs = R;
+    const uint8_t *cls = h->mat_cls;
+    int *cost = h->mat_cost;
+    const int *src = h->mat_src;
+    size_t fc = (size_t)cells;
+    int nt = (int)tiles;
+    void *args[] = {&Rs, &cls, &cost, &W, &src, &fc, &nt};
+    CUDA_TRY(cudaLaunchCooperativeKernel((const void *)k_reach_matrix_solve, dim3(G), dim3(kReachThreads), args, 0, s));
+    k_reach_matrix_gather<<<grid_for(nb * n_goals, 256), 256, 0, s>>>(R, h->mat_cost, (size_t)cells, d_goals, n_goals,
+                                                                      nb * n_goals, d_out + row0 * n_goals);
+    h->launches += 3;
+  }
+  CUDA_TRY(cudaGetLastError());
+  return MLM_OK;
+}
+
+int mlm_reach_matrix_device(mlm_handle h, const double box_min[3], const double box_max[3], const double *d_starts,
+                            size_t n_starts, const double *d_goals, size_t n_goals, double max_dist, int flags,
+                            double *d_out) {
+  ReachGrid R;
+  long long cells = 0;
+  const int rc = reach_matrix_check(h, box_min, box_max, d_starts, n_starts, d_goals, n_goals, max_dist, flags, d_out,
+                                    R, cells);
+  if (rc != MLM_OK || n_starts == 0 || n_goals == 0) return rc;
+  return reach_matrix_enqueue(h, R, cells, d_starts, n_starts, d_goals, n_goals, d_out);
+}
+// the host variant stages the starts, goals and matrix through the handle's stream
+int mlm_reach_matrix(mlm_handle h, const double box_min[3], const double box_max[3], const double *starts,
+                     size_t n_starts, const double *goals, size_t n_goals, double max_dist, int flags, double *out) {
+  ReachGrid R;
+  long long cells = 0;
+  int rc = reach_matrix_check(h, box_min, box_max, starts, n_starts, goals, n_goals, max_dist, flags, out, R, cells);
+  if (rc != MLM_OK || n_starts == 0 || n_goals == 0) return rc;
+  CUDA_TRY(cudaSetDevice(h->device));
+  cudaStream_t s = h->stream;
+  const size_t n = n_starts * n_goals;
+  {
+    StreamTemp<double> d_buf(s);  // starts, goals, matrix
+    CUDA_TRY(d_buf.alloc(3 * n_starts + 3 * n_goals + n));
+    double *d_s = d_buf, *d_g = d_s + 3 * n_starts, *d_o = d_g + 3 * n_goals;
+    CUDA_TRY(cudaMemcpyAsync(d_s, starts, n_starts * 24, cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(d_g, goals, n_goals * 24, cudaMemcpyHostToDevice, s));
+    rc = reach_matrix_enqueue(h, R, cells, d_s, n_starts, d_g, n_goals, d_o);
+    if (rc != MLM_OK) return rc;
+    CUDA_TRY(cudaMemcpyAsync(out, d_o, n * sizeof(double), cudaMemcpyDeviceToHost, s));
+  }
+  CUDA_TRY(cudaStreamSynchronize(s));
   CUDA_TRY(cudaGetLastError());
   return MLM_OK;
 }

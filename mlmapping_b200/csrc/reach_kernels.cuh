@@ -19,6 +19,8 @@
 // cell its halo holds improves after it was read (or holds a source); so the launch ends at the unique fixpoint, which is
 // the exact minimum.  Every round after the first follows an improvement of some cell, which bounds the round count far
 // below the int range of the round numbers; the barrier between rounds is wrap-safe (reach_barrier).
+// The path-cost matrix (mlm_reach_matrix) solves one field per start with the same tile pass, the fields of a batch in
+// one cooperative launch over (field, tile) work items (k_reach_matrix_seed / _solve / _gather, below).
 // Queries are one thread per point; paths one warp per goal, the 26 candidate predecessors on 26 lanes and a ballot for
 // the first in the spec's order.
 #pragma once
@@ -102,12 +104,28 @@ __device__ __forceinline__ uint32_t reach_halo_tiles(const int l[3]) {
       for (int dx = lo[0]; dx <= hi[0]; dx++) m |= 1u << ((dz + 1) * 9 + (dy + 1) * 3 + dx + 1);
   return m;
 }
-// queue for round r the tile at offset j (a bit of reach_halo_tiles) from tile t3, when the box has one there
-__device__ __forceinline__ void reach_queue_near(const ReachGrid &R, const ReachWork &W, const int t3[3], int j, int r) {
+// queue for round r the tile at offset j (a bit of reach_halo_tiles) from tile t3, when the box has one there; the work
+// item is base + the tile (base = f * tiles for field f of a matrix batch)
+__device__ __forceinline__ void reach_queue_near(const ReachGrid &R, const ReachWork &W, const int t3[3], int j, int r,
+                                                 int base = 0) {
   const int n3[3] = {t3[0] + j % 3 - 1, t3[1] + j / 3 % 3 - 1, t3[2] + j / 9 - 1};
   if (n3[0] >= 0 && n3[0] < R.tiles[0] && n3[1] >= 0 && n3[1] < R.tiles[1] && n3[2] >= 0 && n3[2] < R.tiles[2])
-    reach_queue(W, (n3[2] * R.tiles[1] + n3[1]) * R.tiles[0] + n3[0], r);
+    reach_queue(W, base + (n3[2] * R.tiles[1] + n3[1]) * R.tiles[0] + n3[0], r);
 }
+
+// What a tile pass needs to know of its field beyond the shared class bytes.  The single build marks its sources in the
+// class bytes (kCellSource) and its work items are the tiles.  Field f of a matrix batch has its own source cell, which
+// is passable in that field only (so the class bytes stay shared), and its work items are f * tiles + t.
+struct ReachSingle {
+  __device__ __forceinline__ bool source(size_t) const { return false; }
+  __device__ __forceinline__ int base() const { return 0; }
+};
+struct ReachRow {
+  int src;    // the box-linear source cell, -1 when the row has none
+  int item0;  // f * tiles
+  __device__ __forceinline__ bool source(size_t gi) const { return (long long)gi == src; }
+  __device__ __forceinline__ int base() const { return item0; }
+};
 
 // idx[i]: the box-linear index of a distinct source cell
 __global__ void __launch_bounds__(256) k_reach_seed(ReachGrid R, const int *idx, int n, uint8_t *cls, int *cost,
@@ -127,9 +145,10 @@ __global__ void __launch_bounds__(256) k_reach_seed(ReachGrid R, const int *idx,
 }
 
 // one tile of round r: stage it with its halo, relax to a local fixpoint, store the improved cells, queue the
-// neighbours that share an improved boundary cell for round r + 1
+// neighbours that share an improved boundary cell for round r + 1; cost is the field's own grid
+template <class Field>
 __device__ __forceinline__ void reach_tile(const ReachGrid &R, const uint8_t *cls, int *cost, const ReachWork &W, int t,
-                                           int r, int *s_cost, uint8_t *s_pass, uint32_t &s_touch) {
+                                           int r, int *s_cost, uint8_t *s_pass, uint32_t &s_touch, const Field &F) {
   const int tid = threadIdx.x;
   const int t3[3] = {t % R.tiles[0], (t / R.tiles[0]) % R.tiles[1], t / (R.tiles[0] * R.tiles[1])};
   const int nx = R.box.dims[0], ny = R.box.dims[1];
@@ -145,7 +164,7 @@ __device__ __forceinline__ void reach_tile(const ReachGrid &R, const uint8_t *cl
     const size_t gi = ((size_t)g[2] * ny + g[1]) * nx + g[0];
     // costs other CTAs store in this launch: read through L2 (ld.cg), never a stale L1 line
     s_cost[i] = in ? __ldcg(cost + gi) : kReachInf;
-    s_pass[i] = in && reach_passable(cls[gi], R.flags);
+    s_pass[i] = in && (reach_passable(cls[gi], R.flags) || F.source(gi));
   }
   if (tid == 0) s_touch = 0;
   __syncthreads();
@@ -191,7 +210,7 @@ __device__ __forceinline__ void reach_tile(const ReachGrid &R, const uint8_t *cl
     if (m) atomicOr(&s_touch, m);
   }
   __syncthreads();
-  if (tid < 27 && ((s_touch >> tid) & 1)) reach_queue_near(R, W, t3, tid, r + 1);
+  if (tid < 27 && ((s_touch >> tid) & 1)) reach_queue_near(R, W, t3, tid, r + 1, F.base());
   __syncthreads();  // shared memory is reused by the next tile
 }
 
@@ -212,35 +231,93 @@ __device__ __forceinline__ void reach_barrier(unsigned *counter, unsigned target
   __syncthreads();
 }
 
+// the rounds of a solve: work(item, r) for every item of round r's worklist, a device-wide barrier, until a round queues
+// nothing
+template <class Work>
+__device__ __forceinline__ void reach_rounds(const ReachWork &W, Work &&work) {
+  const int G = (int)gridDim.x;
+  int n_cur = __ldcg(W.count + 1);
+  for (int r = 1; n_cur > 0; r++) {
+    if (blockIdx.x == 0 && threadIdx.x == 0) W.count[(r + 2) % 3] = 0;  // round r + 1's queue; read in round r - 1
+    const int *list = (r & 1) ? W.list1 : W.list0;
+    for (int i = blockIdx.x; i < n_cur; i += G) work(__ldcg(list + i), r);
+    reach_barrier(W.bar, (unsigned)r * (unsigned)G);
+    n_cur = __ldcg(W.count + (r + 1) % 3);  // nobody changes it before the next barrier: every CTA sees the same value
+  }
+}
+
 // the whole solve as one cooperative launch (every CTA resident, so the barrier cannot deadlock)
 __global__ void __launch_bounds__(kReachThreads, 2) k_reach_solve(ReachGrid R, const uint8_t *cls, int *cost,
                                                                   ReachWork W) {
   __shared__ int s_cost[kReachHalo * kReachHalo * kReachHalo];
   __shared__ uint8_t s_pass[kReachHalo * kReachHalo * kReachHalo];
   __shared__ uint32_t s_touch;
-  const int G = (int)gridDim.x;
-  int n_cur = __ldcg(W.count + 1);
-  for (int r = 1; n_cur > 0; r++) {
-    if (blockIdx.x == 0 && threadIdx.x == 0) W.count[(r + 2) % 3] = 0;  // round r + 1's queue; read in round r - 1
-    const int *list = (r & 1) ? W.list1 : W.list0;
-    for (int i = blockIdx.x; i < n_cur; i += G) reach_tile(R, cls, cost, W, __ldcg(list + i), r, s_cost, s_pass, s_touch);
-    reach_barrier(W.bar, (unsigned)r * (unsigned)G);
-    n_cur = __ldcg(W.count + (r + 1) % 3);  // nobody changes it before the next barrier: every CTA sees the same value
-  }
+  reach_rounds(W, [&](int t, int r) { reach_tile(R, cls, cost, W, t, r, s_cost, s_pass, s_touch, ReachSingle{}); });
+}
+
+// rule 6 at point p of the field `cost`
+__device__ __forceinline__ double reach_cost_at(const ReachGrid &R, const int *cost, const double *p) {
+  int c[3];
+  if (!reach_cell(R, p, c)) return __longlong_as_double(0x7ff8000000000000ll);
+  const int v = __ldg(cost + esdf_index(R.box, c[0] - R.box.lo[0], c[1] - R.box.lo[1], c[2] - R.box.lo[2]));
+  return v == kReachInf ? __longlong_as_double(0x7ff0000000000000ll) : ((double)v / 1000.0) * R.box.d;
 }
 
 // rule 6, one thread per point
 __global__ void __launch_bounds__(256) k_reach_cost(ReachGrid R, const int *cost, const double *pos, size_t n,
                                                     double *out) {
   const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
+  if (i < n) out[i] = reach_cost_at(R, cost, pos + 3 * i);
+}
+
+// ---- path-cost matrix (mlm_reach_matrix): one field per start, the fields of a batch solved in one launch ----------
+// Field f of a batch owns cost[f * cells ...] and the work items f * tiles + t (marks and worklists sized for all of
+// them); the class bytes are gathered once per call and never hold a source.  Each field is exactly the single build's
+// field from that one start: the same tile pass (reach_tile), with the field's source passable in its own field only.
+
+// one thread per field: row f's source cell by rule 1 (the host rule of mlm_reach_build, through ray_cell), cost 0, and
+// its tile and every tile whose halo holds it on round 1's worklist; src[f] = -1 for a row without a source
+__global__ void __launch_bounds__(256) k_reach_matrix_seed(ReachGrid R, const double *starts, int n, size_t cells,
+                                                           int tiles, int *src, int *cost, ReachWork W) {
+  const int f = blockIdx.x * blockDim.x + threadIdx.x;
+  if (f >= n) return;
   int c[3];
-  if (!reach_cell(R, pos + 3 * i, c)) {
-    out[i] = __longlong_as_double(0x7ff8000000000000ll);
+  if (!reach_cell(R, starts + 3 * (size_t)f, c)) {
+    src[f] = -1;
     return;
   }
-  const int v = __ldg(cost + esdf_index(R.box, c[0] - R.box.lo[0], c[1] - R.box.lo[1], c[2] - R.box.lo[2]));
-  out[i] = v == kReachInf ? __longlong_as_double(0x7ff0000000000000ll) : ((double)v / 1000.0) * R.box.d;
+  const int x = c[0] - R.box.lo[0], y = c[1] - R.box.lo[1], z = c[2] - R.box.lo[2];
+  const int i = (int)esdf_index(R.box, x, y, z);
+  src[f] = i;
+  cost[(size_t)f * cells + i] = 0;
+  const int l[3] = {x % kReachTile, y % kReachTile, z % kReachTile};
+  const int t3[3] = {x / kReachTile, y / kReachTile, z / kReachTile};
+  const uint32_t m = reach_halo_tiles(l);
+  for (int j = 0; j < 27; j++)
+    if ((m >> j) & 1) reach_queue_near(R, W, t3, j, 1, f * tiles);
+}
+
+// the solve of every field of a batch as one cooperative launch: the rounds of k_reach_solve over (field, tile) items
+__global__ void __launch_bounds__(kReachThreads, 2) k_reach_matrix_solve(ReachGrid R, const uint8_t *cls, int *cost,
+                                                                         ReachWork W, const int *src, size_t cells,
+                                                                         int tiles) {
+  __shared__ int s_cost[kReachHalo * kReachHalo * kReachHalo];
+  __shared__ uint8_t s_pass[kReachHalo * kReachHalo * kReachHalo];
+  __shared__ uint32_t s_touch;
+  reach_rounds(W, [&](int item, int r) {
+    const int f = item / tiles;
+    reach_tile(R, cls, cost + (size_t)f * cells, W, item - f * tiles, r, s_cost, s_pass, s_touch,
+               ReachRow{__ldg(src + f), f * tiles});
+  });
+}
+
+// rule 6 for every (row, goal) of a batch, one thread each: out[f * n_goals + j] from field f at goals[j]
+__global__ void __launch_bounds__(256) k_reach_matrix_gather(ReachGrid R, const int *cost, size_t cells,
+                                                             const double *goals, size_t n_goals, size_t n, double *out) {
+  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const size_t f = i / n_goals;
+  out[i] = reach_cost_at(R, cost + f * cells, goals + 3 * (i - f * n_goals));
 }
 
 // rule 7, one warp per goal: lane j < 26 tests the j-th offset of the spec's order, the ballot's lowest lane wins

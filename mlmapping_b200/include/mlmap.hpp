@@ -236,6 +236,15 @@ class mlmap {
   void getReachPaths(const Vec3 *goals, size_t n, size_t max_cells, int32_t *cells3, int32_t *len) {
     check(mlm_reach_paths(h_, n ? goals->v : nullptr, n, max_cells, cells3, len), "mlm_reach_paths");
   }
+  // path-cost matrix (spec at mlm_reach_matrix): out[i * n_goals + j] = getReachCost(goals[j]) after buildReach from
+  // starts[i] alone; the field of the last buildReach is left as it is
+  void getReachMatrix(const Vec3 &min, const Vec3 &max, const Vec3 *starts, size_t n_starts, const Vec3 *goals,
+                      size_t n_goals, double max_dist, double *out, bool inflated = false, bool unknown = false) {
+    check(mlm_reach_matrix(h_, min.v, max.v, n_starts ? starts->v : nullptr, n_starts, n_goals ? goals->v : nullptr,
+                           n_goals, max_dist, (inflated ? MLM_REACH_INFLATED : 0) | (unknown ? MLM_REACH_UNKNOWN : 0),
+                           out),
+          "mlm_reach_matrix");
+  }
 
   // frontier clustering (no reference counterpart; spec at mlm_frontier_clusters): the clusters with >= min_cells cells
   // sorted by key (z, y, x); box_min / box_max both null for the whole map; cells3 / cluster_of (optional) receive every
